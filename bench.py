@@ -8,6 +8,7 @@ the measured bf16 tensor-core peak reached by the implicit-GEMM kernel.
 
     python bench.py --gpus N --steps K --warmup W           (N>1: launched by torch.distributed.run, one rank per GPU)
     python bench.py --impl reference ...                    (the reference's CPU path = fp32 torch oracle, host cores)
+    python bench.py --dump-outputs DIR ...                  (also writes what the last timed step computed, DIR/*.npy)
 
 Prints ONE JSON line on rank 0 (schema in the task contract; extra keys: roofline, cpu_baseline, e2e, gpu_launches,
 clocks, kernels).
@@ -268,6 +269,38 @@ def predict_section(dev, rank, world, side, batch, max_over_ranks, barrier, peak
                     "d2h_bytes": host_mask.numel() * world, "part_mask_equals_sharded_mask": same}}
 
 
+DUMP_SAMPLE = 1 << 20        # elements kept of each parameter-sized vector (4 MB as float32)
+DUMP_LOGITS_MAX = 8 << 20    # logits kept whole up to 32 MB (batch 64 x 2 x 256 x 256), sampled beyond
+
+
+def _seeded_sample(t: torch.Tensor, k: int, seed: int) -> torch.Tensor:
+    """t flattened, or k of its elements at indices drawn from a fixed seed: the same indices on every run and build"""
+    flat = t.reshape(-1)
+    if flat.numel() <= k:
+        return flat
+    idx = torch.randint(0, flat.numel(), (k,), generator=torch.Generator().manual_seed(seed))
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(path: str, net) -> None:
+    """What a caller of the timed training step holds after its last step, as float32 .npy files (about 40 MB in all):
+    the loss the step returns, the logits of its forward pass, and a fixed sample of the parameters after its update
+    and of its gradients.  Parameters and gradients are taken in the oracle's parameter order, not the plan's flat
+    layout, so that two builds of the project can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    logits = net.logits_nchw()
+    names = [e.name for e in net.layout.entries]
+    params = torch.cat([net.param(n).reshape(-1) for n in names])
+    grads = torch.cat([net.grad(n).reshape(-1) for n in names])
+    arrays = {"loss": net.loss,
+              "logits": logits if logits.numel() <= DUMP_LOGITS_MAX else _seeded_sample(logits, DUMP_LOGITS_MAX, 1),
+              "params_sample": _seeded_sample(params, DUMP_SAMPLE, 2),
+              "grads_sample": _seeded_sample(grads, DUMP_SAMPLE, 3)}
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def plan_bytes(plan) -> int:
     """algorithmic bytes of one implicit-GEMM launch: activations in (every view once), weights, residual / mask
     operands, output - all bf16 at their unpadded channel counts (fp32 for the head's logits)"""
@@ -417,7 +450,11 @@ def main():
                     "(BASELINE configs[2]: 20000)")
     ap.add_argument("--no-extra", action="store_true", help="skip the BASELINE configs[3] / configs[4] sub-records")
     ap.add_argument("--r50-batch", type=int, default=16, help="tiles per GPU per step of the xresnet50 / 512-px line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the loss, logits and a fixed "
+                    "sample of the parameters and gradients of the last timed training step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b2u":
+        ap.error("--dump-outputs writes the outputs of the CUDA training step (--impl b2u)")
     args.warmup = max(args.warmup, 3) if args.impl == "b2u" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -490,6 +527,8 @@ def main():
     dev_ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     loss_val = float(net.loss.item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net)     # before the e2e steps below overwrite the plan's buffers
 
     # ---- e2e: public API with HOST buffers, H2D of the tiles and D2H of the loss every step inside the timed region
     # (every step copies its own batch from pinned host memory; the copy of batch i+1 is enqueued on a copy stream
