@@ -324,6 +324,24 @@ int b2u_ce_fwd_bwd(const float* logits, int32_t ld, const uint8_t* labels, int64
 int b2u_ce_finalize(const float* loss_partial, int32_t rows, const float* wsum_partial, int32_t wsum_rows, float* loss,
                     void* stream);
 
+/* ---- loss: fastai FocalLossFlat(axis=1, gamma, weight) -------------------------------------------------------- */
+/* logits / labels / dlogits as for CE.  Per pixel l = w[y]*nll, f = (1-exp(-l))^gamma * l; `rows` block partials of
+ * sum f, reduced by b2u_mse_finalize(P) for mean (mean != 0) or b2u_mse_finalize(1) for sum.  dlogits (NULL: loss only)
+ * = df/dlogits * grad_scale (/ P for mean).  gamma >= 0. */
+int b2u_focal_fwd_bwd(const float* logits, int32_t ld, const uint8_t* labels, int64_t P, int32_t C, const float* weight,
+                      float gamma, int32_t mean, void* dlogits, int32_t ldg, float* loss_partial, int32_t rows,
+                      float grad_scale, void* stream);
+/* ---- loss: fastai DiceLoss(axis=1, smooth, reduction, square_in_union), two phases ---------------------------- */
+/* Samples are N runs of HW pixels.  b2u_dice_stats writes fp32 partial[N][blocks_per_sample][3][C] = per block
+ * {sum p*t, sum p (sum p^2 with square_in_union), sum t}.  b2u_dice_bwd folds them per (n, c) in block order,
+ * writes loss_partial[n] = sum_c (1 - (2I+s)/(U+s)) and dlogits (NULL: loss only) = d(loss)/d(logits) * grad_scale
+ * (/ (N*C) for mean); the loss is b2u_mse_finalize(loss_partial, N, mean ? N*C : 1).  Deterministic, no atomics. */
+int b2u_dice_stats(const float* logits, int32_t ld, const uint8_t* labels, int32_t N, int64_t HW, int32_t C,
+                   int32_t square_in_union, float* partial, int32_t blocks_per_sample, void* stream);
+int b2u_dice_bwd(const float* logits, int32_t ld, const uint8_t* labels, int32_t N, int64_t HW, int32_t C,
+                 int32_t square_in_union, const float* partial, int32_t blocks_per_sample, float smooth, int32_t mean,
+                 void* dlogits, int32_t ldg, float* loss_partial, float grad_scale, void* stream);
+
 /* ---- regression variant: MSELossFlat(axis=1) (train.py:189-192) + the sums behind fastai's rmse / R2Score metrics -- */
 /* pred = lane 0 of the fp32 head output [P][ld]; target fp32 [P]; loss = mean (pred - target)^2; dpred bf16 [P][ldg]
  * (NULL: loss only) lane 0 = grad_scale * 2 (pred - target) / P, other lanes 0.  `rows` block partials, then finalize. */

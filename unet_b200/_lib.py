@@ -157,6 +157,9 @@ def _declare(lib):
         "b2u_ce_weight_sum": [u8p, i64, vp, i32, vp, i32, vp],
         "b2u_ce_fwd_bwd": [vp, i32, u8p, i64, i32, vp, vp, i32, vp, i32, vp, i32, f32, vp],
         "b2u_ce_finalize": [vp, i32, vp, i32, vp, vp],
+        "b2u_focal_fwd_bwd": [vp, i32, u8p, i64, i32, vp, f32, i32, vp, i32, vp, i32, f32, vp],
+        "b2u_dice_stats": [vp, i32, u8p, i32, i64, i32, i32, vp, i32, vp],
+        "b2u_dice_bwd": [vp, i32, u8p, i32, i64, i32, i32, vp, i32, f32, i32, vp, i32, vp, f32, vp],
         "b2u_mse_fwd_bwd": [vp, i32, vp, i64, vp, i32, vp, i32, f32, vp],
         "b2u_mse_finalize": [vp, i32, i64, vp, vp],
         "b2u_regression_sums": [vp, i32, vp, i64, vp, i32, vp, vp, vp],

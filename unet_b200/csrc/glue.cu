@@ -695,6 +695,222 @@ __global__ void mse_finalize_kernel(const float* loss_partial, int rows, long lo
   }
 }
 
+// ------------------------------------------------------------------------------------------------ focal / dice losses
+// fastai FocalLossFlat(axis=1, gamma, weight=w): per pixel l = w[y] * (-log p_y), pt = exp(-l), f = (1 - pt)^gamma * l.
+// Block partials of sum f; b2u_mse_finalize divides by P ('mean') or by 1 ('sum').  dlogits = gs * f'(l) * w[y] *
+// (softmax - onehot) with f'(l) = (1 - pt)^gamma * (1 + gamma * pt * l / (1 - pt)).  The second term is the
+// gamma * (1-pt)^(gamma-1) * pt * l of the chain rule written so that it stays finite: where 1 - pt == 0 it is 0 (its
+// limit for every gamma > 0), so a saturated correct pixel gives 0 and never 0^negative * 0.  Accurate expf / logf: the
+// loss is compared with a float64 evaluation at 1e-5.
+template <int MAXC>
+__global__ void focal_fwd_bwd_kernel(const float* __restrict__ logits, int ld, const uint8_t* __restrict__ labels,
+                                     long long P, int C, const float* __restrict__ weight, float gamma,
+                                     __nv_bfloat16* __restrict__ dlogits, int ldg, float* __restrict__ loss_partial,
+                                     float gs) {
+  pdl_enter();
+  __shared__ float sh[32];
+  float acc = 0.f;
+  const long long per = (P + gridDim.x - 1) / gridDim.x;
+  const long long p0 = (long long)blockIdx.x * per, p1 = min(P, p0 + per);
+  for (long long p = p0 + threadIdx.x; p < p1; p += blockDim.x) {
+    float z[MAXC];
+    float m = -INFINITY;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      z[c] = (c < C) ? logits[p * ld + c] : -INFINITY;
+      m = fmaxf(m, z[c]);
+    }
+    const int y = labels[p];
+    const bool ok = y < C;
+    float zy = m, se = 0.f;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      zy = (c == y) ? z[c] : zy;
+      z[c] = (c < C) ? expf(z[c] - m) : 0.f;
+      se += z[c];
+    }
+    const float wy = ok ? (weight ? __ldg(weight + y) : 1.f) : 0.f;
+    const float l = wy * ((m - zy) + logf(se));          // se >= 1: the log is >= 0
+    const float omp = -expm1f(-l);                         // 1 - pt
+    const float q = powf(omp, gamma);                      // powf(0, 0) = 1: gamma = 0 is plain weighted CE
+    acc += q * l;
+    if (dlogits) {
+      const float dfdl = q * (omp > 0.f ? 1.f + gamma * expf(-l) * (l / omp) : 1.f);
+      const float g = gs * dfdl * wy;
+      const float inv = 1.f / se;
+      for (int c0 = 0; c0 < ldg; c0 += 8) {
+        float gv[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+          const int c = c0 + k;
+          float zc = 0.f;
+#pragma unroll
+          for (int q2 = 0; q2 < MAXC; ++q2) zc = (q2 == c) ? z[q2] : zc;
+          gv[k] = (c < C) ? g * (zc * inv - (c == y ? 1.f : 0.f)) : 0.f;
+        }
+        uint4 u;
+        u.x = pack_bf16x2(gv[0], gv[1]); u.y = pack_bf16x2(gv[2], gv[3]);
+        u.z = pack_bf16x2(gv[4], gv[5]); u.w = pack_bf16x2(gv[6], gv[7]);
+        *reinterpret_cast<uint4*>(dlogits + p * ldg + c0) = u;
+      }
+    }
+  }
+  const float r = block_sum(acc, sh);
+  if (threadIdx.x == 0) loss_partial[blockIdx.x] = r;
+}
+
+// fastai DiceLoss(axis=1, smooth, square_in_union), phase 1.  Grid (bps, N): block (b, n) covers the b-th of bps equal
+// pixel ranges of sample n and writes partial[(n*bps + b)*3C + {0, C, 2C} + c] = {sum p_c t_c, sum p_c (or p_c^2),
+// sum t_c} over its pixels (t = one-hot label; a label >= C is all zeros).  256 threads; per-thread registers, then
+// warp shuffles and the 8 warp sums in warp order: no atomics, the same bits every run.
+template <int MAXC>
+__global__ void __launch_bounds__(256) dice_stats_kernel(const float* __restrict__ logits, int ld,
+                                                         const uint8_t* __restrict__ labels, long long HW, int C,
+                                                         int square, float* __restrict__ partial) {
+  pdl_enter();
+  __shared__ float sh[3 * MAXC][8];
+  const int n = blockIdx.y, bps = gridDim.x;
+  const long long per = (HW + bps - 1) / bps;
+  const long long p0 = (long long)blockIdx.x * per, p1 = min(HW, p0 + per);
+  const long long base = (long long)n * HW;
+  float si[MAXC], su[MAXC], st[MAXC];
+#pragma unroll
+  for (int c = 0; c < MAXC; ++c) si[c] = su[c] = st[c] = 0.f;
+  for (long long p = base + p0 + threadIdx.x; p < base + p1; p += blockDim.x) {
+    float z[MAXC];
+    float m = -INFINITY;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      z[c] = (c < C) ? logits[p * ld + c] : -INFINITY;
+      m = fmaxf(m, z[c]);
+    }
+    float se = 0.f;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      z[c] = (c < C) ? expf(z[c] - m) : 0.f;
+      se += z[c];
+    }
+    const float inv = 1.f / se;
+    const int y = labels[p];
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      const float pc = z[c] * inv;
+      si[c] += (c == y) ? pc : 0.f;
+      su[c] += square ? pc * pc : pc;
+      st[c] += (c == y) ? 1.f : 0.f;
+    }
+  }
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+#pragma unroll
+  for (int c = 0; c < MAXC; ++c) {
+    if (c < C) {
+      float a = si[c], b = su[c], t = st[c];
+      for (int o = 16; o > 0; o >>= 1) {
+        a += __shfl_xor_sync(0xffffffffu, a, o);
+        b += __shfl_xor_sync(0xffffffffu, b, o);
+        t += __shfl_xor_sync(0xffffffffu, t, o);
+      }
+      if (lane == 0) { sh[c][w] = a; sh[MAXC + c][w] = b; sh[2 * MAXC + c][w] = t; }
+    }
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 3 * C; i += blockDim.x) {
+    const int k = i / C, c = i - k * C;
+    float r = 0.f;
+    for (int j = 0; j < 8; ++j) r += sh[k * MAXC + c][j];
+    partial[((long long)n * bps + blockIdx.x) * 3 * C + i] = r;
+  }
+}
+
+// DiceLoss phase 2.  Every block of sample n folds that sample's bps partials in block order (double), so all blocks
+// derive the same I_c, U_c = sum p (or p^2) + sum t.  Block 0 of the sample writes loss_partial[n] = sum_c (1 - d_c),
+// d_c = (2 I_c + s) / (U_c + s).  With dlogits: g_c = -r (2 t_c (U_c+s) - (2 I_c+s) u'_c) / (U_c+s)^2 (u' = 1, or 2 p_c
+// with square_in_union) is pulled back through the softmax: dz_j = p_j (g_j - sum_c p_c g_c).  The grid's x extent
+// (blocks per sample of this pass) need not equal bps.
+template <int MAXC>
+__global__ void __launch_bounds__(256) dice_bwd_kernel(const float* __restrict__ logits, int ld,
+                                                       const uint8_t* __restrict__ labels, long long HW, int C,
+                                                       int square, const float* __restrict__ partial, int bps,
+                                                       float smooth, float r, __nv_bfloat16* __restrict__ dlogits,
+                                                       int ldg, float* __restrict__ loss_partial) {
+  pdl_enter();
+  __shared__ double s_stat[3 * MAXC];
+  __shared__ float s_a[MAXC], s_b[MAXC];
+  const int n = blockIdx.y;
+  if (threadIdx.x < 3 * C) {
+    double t = 0.0;
+    for (int b = 0; b < bps; ++b) t += partial[((long long)n * bps + b) * 3 * C + threadIdx.x];
+    s_stat[threadIdx.x] = t;
+  }
+  __syncthreads();
+  if (threadIdx.x < C) {
+    const int c = threadIdx.x;
+    const double den = s_stat[C + c] + s_stat[2 * C + c] + (double)smooth;
+    s_a[c] = (float)(2.0 * (double)r / den);
+    s_b[c] = (float)((double)r * (2.0 * s_stat[c] + (double)smooth) / (den * den));
+  }
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    double l = 0.0;
+    for (int c = 0; c < C; ++c)
+      l += 1.0 - (2.0 * s_stat[c] + (double)smooth) / (s_stat[C + c] + s_stat[2 * C + c] + (double)smooth);
+    loss_partial[n] = (float)l;
+  }
+  __syncthreads();
+  if (!dlogits) return;
+  float a[MAXC], bb[MAXC];
+#pragma unroll
+  for (int c = 0; c < MAXC; ++c) {
+    a[c] = (c < C) ? s_a[c] : 0.f;
+    bb[c] = (c < C) ? s_b[c] : 0.f;
+  }
+  const long long per = (HW + gridDim.x - 1) / gridDim.x;
+  const long long p0 = (long long)blockIdx.x * per, p1 = min(HW, p0 + per);
+  const long long base = (long long)n * HW;
+  for (long long p = base + p0 + threadIdx.x; p < base + p1; p += blockDim.x) {
+    float z[MAXC];
+    float m = -INFINITY;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      z[c] = (c < C) ? logits[p * ld + c] : -INFINITY;
+      m = fmaxf(m, z[c]);
+    }
+    float se = 0.f;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      z[c] = (c < C) ? expf(z[c] - m) : 0.f;
+      se += z[c];
+    }
+    const float inv = 1.f / se;
+    const int y = labels[p];
+    float g[MAXC];
+    float dot = 0.f;
+#pragma unroll
+    for (int c = 0; c < MAXC; ++c) {
+      z[c] *= inv;                                                        // p_c (0 beyond C)
+      g[c] = bb[c] * (square ? 2.f * z[c] : 1.f) - ((c == y) ? a[c] : 0.f);
+      dot += z[c] * g[c];
+    }
+    for (int c0 = 0; c0 < ldg; c0 += 8) {
+      float gv[8];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        const int c = c0 + k;
+        float pc = 0.f, gc = 0.f;
+#pragma unroll
+        for (int q = 0; q < MAXC; ++q) {
+          pc = (q == c) ? z[q] : pc;
+          gc = (q == c) ? g[q] : gc;
+        }
+        gv[k] = pc * (gc - dot);                                          // 0 beyond C: p_c = 0 there
+      }
+      uint4 u;
+      u.x = pack_bf16x2(gv[0], gv[1]); u.y = pack_bf16x2(gv[2], gv[3]);
+      u.z = pack_bf16x2(gv[4], gv[5]); u.w = pack_bf16x2(gv[6], gv[7]);
+      *reinterpret_cast<uint4*>(dlogits + p * ldg + c0) = u;
+    }
+  }
+}
+
 // validation sums of the regression metrics (fastai rmse, R2Score; train.py:190): sums[0..3] += {sum (p-t)^2, sum t,
 // sum t^2, n} in double.  Block partials are combined by the last block in block order (fixed order: deterministic).
 __global__ void regression_sums_kernel(const float* __restrict__ pred, int ld, const float* __restrict__ target,
@@ -1176,6 +1392,61 @@ extern "C" int b2u_mse_fwd_bwd(const float* pred, int32_t ld, const float* targe
 extern "C" int b2u_mse_finalize(const float* loss_partial, int32_t rows, int64_t P, float* loss, void* stream) {
   B2U_CHECK_ARG(loss_partial && loss && rows > 0 && P > 0, "mse_finalize: bad argument");
   launch_k(mse_finalize_kernel, dim3(1), dim3(32), 0, (cudaStream_t)stream, loss_partial, rows, (long long)P, loss);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_focal_fwd_bwd(const float* logits, int32_t ld, const uint8_t* labels, int64_t P, int32_t C,
+                                 const float* weight, float gamma, int32_t mean, void* dlogits, int32_t ldg,
+                                 float* loss_partial, int32_t rows, float grad_scale, void* stream) {
+  B2U_CHECK_ARG(logits && labels && loss_partial && rows > 0 && P > 0 && gamma >= 0.f, "focal_fwd_bwd: bad argument");
+  B2U_CHECK_ARG(C >= 1 && C <= 32 && C <= ld && (!dlogits || (ldg >= C && ldg % 8 == 0)),
+                "focal_fwd_bwd: C=%d ld=%d ldg=%d unsupported (ldg must be a multiple of 8)", C, ld, ldg);
+  cudaStream_t st = (cudaStream_t)stream;
+  const float gs = mean ? (float)((double)grad_scale / (double)P) : grad_scale;
+  if (C <= 8)
+    launch_k(focal_fwd_bwd_kernel<8>, dim3(rows), dim3(256), 0, st, logits, ld, labels, (long long)P, C, weight, gamma,
+             (bf)dlogits, ldg, loss_partial, gs);
+  else
+    launch_k(focal_fwd_bwd_kernel<32>, dim3(rows), dim3(256), 0, st, logits, ld, labels, (long long)P, C, weight, gamma,
+             (bf)dlogits, ldg, loss_partial, gs);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_dice_stats(const float* logits, int32_t ld, const uint8_t* labels, int32_t N, int64_t HW, int32_t C,
+                              int32_t square_in_union, float* partial, int32_t blocks_per_sample, void* stream) {
+  B2U_CHECK_ARG(logits && labels && partial && N > 0 && N <= 65535 && HW > 0 && blocks_per_sample > 0,
+                "dice_stats: bad argument");
+  B2U_CHECK_ARG(C >= 1 && C <= 32 && C <= ld, "dice_stats: C=%d ld=%d unsupported", C, ld);
+  cudaStream_t st = (cudaStream_t)stream;
+  const dim3 grid(blocks_per_sample, N);
+  if (C <= 8)
+    launch_k(dice_stats_kernel<8>, grid, dim3(256), 0, st, logits, ld, labels, (long long)HW, C, square_in_union, partial);
+  else
+    launch_k(dice_stats_kernel<32>, grid, dim3(256), 0, st, logits, ld, labels, (long long)HW, C, square_in_union, partial);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_dice_bwd(const float* logits, int32_t ld, const uint8_t* labels, int32_t N, int64_t HW, int32_t C,
+                            int32_t square_in_union, const float* partial, int32_t blocks_per_sample, float smooth,
+                            int32_t mean, void* dlogits, int32_t ldg, float* loss_partial, float grad_scale,
+                            void* stream) {
+  B2U_CHECK_ARG(logits && labels && partial && loss_partial && N > 0 && N <= 65535 && HW > 0 && blocks_per_sample > 0,
+                "dice_bwd: bad argument");
+  B2U_CHECK_ARG(C >= 1 && C <= 32 && C <= ld && (!dlogits || (ldg >= C && ldg % 8 == 0)),
+                "dice_bwd: C=%d ld=%d ldg=%d unsupported (ldg must be a multiple of 8)", C, ld, ldg);
+  cudaStream_t st = (cudaStream_t)stream;
+  const float r = mean ? (float)((double)grad_scale / ((double)N * C)) : grad_scale;
+  // loss only (validation): one block per sample folds the statistics
+  const dim3 grid(dlogits ? blocks_per_sample : 1, N);
+  if (C <= 8)
+    launch_k(dice_bwd_kernel<8>, grid, dim3(256), 0, st, logits, ld, labels, (long long)HW, C, square_in_union, partial,
+             blocks_per_sample, smooth, r, (bf)dlogits, ldg, loss_partial);
+  else
+    launch_k(dice_bwd_kernel<32>, grid, dim3(256), 0, st, logits, ld, labels, (long long)HW, C, square_in_union, partial,
+             blocks_per_sample, smooth, r, (bf)dlogits, ldg, loss_partial);
   B2U_LAUNCH_CHECK();
   return B2U_OK;
 }

@@ -20,6 +20,7 @@ from typing import Callable, Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import _lib, ops
+from .losses import LossSpec, dice_blocks_per_sample, launch_loss
 from .layout import ConvSpec, NetSpec, ParamLayout, build_spec, conv_flops, shuffle_row_of_co
 from .ops import ConvPlan, WgradPlan, padc, view_nhwc
 
@@ -105,7 +106,8 @@ class UNetB200:
     def __init__(self, arch: str = "xresnet34", n_in: int = 4, n_out: int = 2, size: Tuple[int, int] = (256, 256),
                  batch: int = 8, training: bool = True, device: Optional[torch.device] = None,
                  class_weights: Optional[Sequence[float]] = None, self_attention: bool = False,
-                 input_div: Tuple[float, float] = (255.0, 1.0), regression: bool = False):
+                 input_div: Tuple[float, float] = (255.0, 1.0), regression: bool = False,
+                 loss_spec: Optional[LossSpec] = None):
         if not torch.cuda.is_available():
             raise _lib.B2UError("UNetB200 needs a CUDA device (sm_100a); there is no CPU path")
         self.lib = _lib.load()
@@ -116,6 +118,10 @@ class UNetB200:
         self.regression = bool(regression)
         if self.regression and n_out != 1:
             raise ValueError("the regression variant has n_out = 1 (train.py:137-138)")
+        # the training loss (losses.LossSpec): cross-entropy by default, MSE for regression, focal or Dice on request
+        self.loss_spec = loss_spec or LossSpec()
+        if self.regression and self.loss_spec.name != "ce":
+            raise ValueError(f"the regression variant trains with MSELossFlat only, not the {self.loss_spec.name} loss")
         self.spec: NetSpec = build_spec(arch, n_in, n_out, self.self_attention)
         self.layout = ParamLayout(self.spec)
         self.N, (self.H, self.W) = batch, size
@@ -929,7 +935,11 @@ class UNetB200:
             self.loss = torch.zeros(1, dtype=torch.float32, device=dev)
             self._ce_rows = 592
             self._wsum_part = torch.zeros(self._ce_rows, dtype=torch.float32, device=dev)
-            self._loss_part = torch.zeros(self._ce_rows, dtype=torch.float32, device=dev)
+            self._loss_part = torch.zeros(max(self._ce_rows, N), dtype=torch.float32, device=dev)   # Dice: one per sample
+            # DiceLoss: per-block statistics of every (sample, class), folded by its backward kernel
+            self._dice_bps = dice_blocks_per_sample(N, H * W) if self.loss_spec.name == "dice" else 0
+            self._dice_part = torch.zeros(N * self._dice_bps * 3 * spec.n_out, dtype=torch.float32, device=dev) \
+                if self._dice_bps else None
 
             def tail_bwd():
                 dL = self.dlogits
@@ -1024,6 +1034,12 @@ class UNetB200:
             _lib.check(lib.b2u_mse_finalize(self._loss_part.data_ptr(), self._ce_rows, P_, self.loss.data_ptr(), s),
                        "b2u_mse_finalize")
             return self.loss
+        if self.loss_spec.name != "ce":
+            # FocalLossFlat / DiceLoss (losses.py): one fused pass, or Dice statistics + backward
+            launch_loss(lib, self.loss_spec, self.logits, self.labels, self.N, self.H * self.W, self.n_out,
+                        _p(self.class_weights), self.dlogits.data_ptr(), self.dlogits.shape[-1], self._loss_part,
+                        self._ce_rows, self._dice_part, self._dice_bps, self.loss, grad_scale, s)
+            return self.loss
         _lib.check(lib.b2u_ce_weight_sum(self.labels.data_ptr(), P_, _p(self.class_weights), self.n_out,
                                          self._wsum_part.data_ptr(), self._ce_rows, s), "b2u_ce_weight_sum")
         _lib.check(lib.b2u_ce_fwd_bwd(self.logits.data_ptr(), ld, self.labels.data_ptr(), P_, self.n_out,
@@ -1087,5 +1103,5 @@ class UNetB200:
 
     @property
     def launches_per_train_step(self) -> int:
-        # forward + CE (3) + backward + optimizer (1) + weight staging (1)
-        return self.launches_fwd + 3 + self.launches_bwd + 2
+        # forward + loss (CE and Dice 3, focal 2) + backward + optimizer (1) + weight staging (1)
+        return self.launches_fwd + (2 if self.loss_spec.name == "focal" else 3) + self.launches_bwd + 2

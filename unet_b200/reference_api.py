@@ -36,6 +36,7 @@ from . import _lib, ops
 from .engine import Trainer, one_cycle
 from .network import UNetB200, input_divisors
 from .predict_engine import TiledPredictor, gather_mask_strips
+from .losses import LossSpec, dice_blocks_per_sample, launch_loss, parse_loss_func, warn_dice_weights
 from .geotiff import GeoInfo, geotiff_info, open_mask, open_tile, read_geotiff, write_geotiff
 from .tiling import colour_classes, compute_windows, placement_from_geotransform, shard_windows_by_columns
 
@@ -58,7 +59,7 @@ class Learner:
                  class_weights: Optional[Sequence[float]] = None, opt_func: str = "adam", lr: float = 1e-3,
                  wd: float = 0.01, encoder_factor: float = 10.0, moms: Sequence[float] = (0.95, 0.85, 0.95),
                  self_attention: bool = False, regression: bool = False, input_dtype: torch.dtype = torch.uint8,
-                 sixteen_bit: bool = False):
+                 sixteen_bit: bool = False, loss_spec: Optional[LossSpec] = None):
         self.arch, self.n_in, self.n_classes, self.size, self.bs = arch, n_in, n_classes, tuple(size), batch_size
         self.class_weights = list(class_weights) if class_weights is not None else None
         self.self_attention, self.regression = bool(self_attention), bool(regression)
@@ -67,9 +68,11 @@ class Learner:
         self.input_dtype, self.sixteen_bit = input_dtype, bool(sixteen_bit)
         self.input_div = input_divisors(self.sixteen_bit, self.regression)
         self.n_out = 1 if self.regression else n_classes                    # train.py:137-140
+        self.loss_spec = loss_spec or LossSpec()
         self.net = UNetB200(arch, n_in, self.n_out, self.size, batch_size, training=True,
                             class_weights=None if self.regression else self.class_weights,
-                            self_attention=self.self_attention, input_div=self.input_div, regression=self.regression)
+                            self_attention=self.self_attention, input_div=self.input_div, regression=self.regression,
+                            loss_spec=self.loss_spec)
         # fastai's own start: BatchNorm gamma 1 / beta 1e-3, gamma 0 on the last BatchNorm of every ResBlock (BatchZero),
         # decoder biases N(0, 0.01) (network.init_parameters)
         self.net.init_parameters(seed=0, randomize_bn=False)
@@ -174,7 +177,9 @@ class Learner:
         if self._val is None:
             dev, rows = net.device, 592
             f = lambda n, dt=torch.float32: torch.zeros(n, dtype=dt, device=dev)
-            self._val = dict(rows=rows, wsum=f(rows), part=f(rows), loss=f(1), losses=f(4096),
+            bps = dice_blocks_per_sample(net.N, net.H * net.W) if self.loss_spec.name == "dice" else 0
+            self._val = dict(rows=rows, wsum=f(rows), part=f(max(rows, net.N)), loss=f(1), losses=f(4096),
+                             dice_bps=bps, dice_part=f(max(1, net.N * bps * 3 * self.n_out)),
                              labels=torch.zeros((net.N, net.H, net.W), device=dev,
                                                 dtype=torch.float32 if self.regression else torch.uint8),
                              counts=f(3 * max(1, self.n_classes), torch.int64), sums=f(4, torch.float64),
@@ -183,7 +188,8 @@ class Learner:
 
     def validate(self, batches: Iterable) -> Dict[str, float]:
         """One pass over the validation batches on the eval plan, reduced on the device: valid_loss as fastai's AvgLoss
-        (per-batch loss weighted by the number of REAL samples: a padded last batch does not count its padding) and
+        (per-batch loss weighted by the number of REAL samples: a padded last batch does not count its padding; the loss
+        is the one the model trains with, and a Dice loss sums its statistics over the real samples only) and
         DiceMulti (macro Dice over the classes present; regression: rmse and R2Score).  One device-to-host read at the end."""
         net = self._eval_net()
         lib, v = net.lib, self._val_buffers(net)
@@ -209,6 +215,12 @@ class Learner:
                 _lib.check(lib.b2u_regression_sums(net.logits.data_ptr(), ld, v["labels"].data_ptr(), P_,
                                                    v["partial"].data_ptr(), v["rows"], v["sums"].data_ptr(),
                                                    v["ticket"].data_ptr(), s), "b2u_regression_sums")
+            elif self.loss_spec.name != "ce":
+                # the loss the model trains with (FocalLossFlat / DiceLoss), over the n real samples
+                launch_loss(lib, self.loss_spec, net.logits, v["labels"], n, HW, net.n_out, net.class_weights.data_ptr(),
+                            None, 0, v["part"], v["rows"], v["dice_part"], v["dice_bps"], v["loss"], 1.0, s)
+                _lib.check(lib.b2u_dice_counts(net.logits.data_ptr(), ld, v["labels"].data_ptr(), P_, net.n_out,
+                                               v["counts"].data_ptr(), s), "b2u_dice_counts")
             else:
                 w = net.class_weights.data_ptr()
                 _lib.check(lib.b2u_ce_weight_sum(v["labels"].data_ptr(), P_, w, net.n_out, v["wsum"].data_ptr(),
@@ -270,7 +282,7 @@ class Learner:
         torch.save({"arch": self.arch, "n_in": self.n_in, "n_classes": self.n_classes, "size": list(self.size),
                     "batch_size": self.bs, "class_weights": self.class_weights, "self_attention": self.self_attention,
                     "regression": self.regression, "sixteen_bit": self.sixteen_bit,
-                    "input_dtype": str(self.input_dtype).replace("torch.", ""),
+                    "input_dtype": str(self.input_dtype).replace("torch.", ""), "loss_func": self.loss_spec.as_dict(),
                     "state_dict": {k: v.cpu() for k, v in self.state_dict().items()}}, path)
 
 
@@ -298,13 +310,21 @@ def unet_learner_MS(n_in: int, n_classes: int, arch="xresnet34", size: Tuple[int
     """train.py:98-160.  `n_in` / `size` replace what the reference probes from `dls.train_ds` (:124-125) and
     `n_classes` replaces `len(dls.vocab)` (:140); `pretrained` may be a state_dict with fastai keys.  `regression`:
     n_out = 1 (:137-138), MSELossFlat (:189-192), rmse / R2Score metrics (:190).  `input_dtype` / `sixteen_bit`: the
-    element type of the raw tiles and whether the dataset is the reference's 'int16' kind (utils.py:72-89)."""
-    if loss_func is not None and not isinstance(loss_func, str):
-        warnings.warn("loss_func objects are ignored: the plan implements CrossEntropyLossFlat(axis=1) with class weights "
-                      "(MSELossFlat(axis=1) for regression)")
+    element type of the raw tiles and whether the dataset is the reference's 'int16' kind (utils.py:72-89).
+    `loss_func`: None (CrossEntropyLossFlat(axis=1) with `class_weights`), a string in fastai call syntax such as
+    "FocalLossFlat(axis=1, gamma=3)" or "DiceLoss(square_in_union=True)", or a CrossEntropyLossFlat / FocalLossFlat /
+    DiceLoss object (see `losses.parse_loss_func`).  FocalLossFlat takes `class_weights` as its weight; DiceLoss has
+    none.  The regression variant trains with MSELossFlat only."""
+    spec = parse_loss_func(loss_func)
+    if spec is None:
+        warnings.warn(f"loss_func {type(loss_func).__name__} is not supported: the plan trains with "
+                      "CrossEntropyLossFlat(axis=1) with class weights (MSELossFlat(axis=1) for regression)")
+        spec = LossSpec()
+    if not regression:
+        warn_dice_weights(spec, class_weights)
     learn = Learner(_arch_name(arch), n_in, n_classes, size, batch_size, class_weights, opt_func, lr, wd,
                     encoder_factor, moms, self_attention=self_attention, regression=regression,
-                    input_dtype=input_dtype, sixteen_bit=sixteen_bit)
+                    input_dtype=input_dtype, sixteen_bit=sixteen_bit, loss_spec=spec)
     if isinstance(pretrained, dict):
         learn.load_state_dict(pretrained)
     return learn
@@ -322,7 +342,8 @@ def load_learner(path, batch_size: Optional[int] = None) -> Learner:
     learn = Learner(ck["arch"], ck["n_in"], ck["n_classes"], tuple(ck["size"]), batch_size or ck["batch_size"],
                     ck.get("class_weights"), self_attention=ck.get("self_attention", False),
                     regression=ck.get("regression", False), sixteen_bit=ck.get("sixteen_bit", False),
-                    input_dtype=_DTYPES[ck.get("input_dtype", "uint8")])
+                    input_dtype=_DTYPES[ck.get("input_dtype", "uint8")],
+                    loss_spec=LossSpec.from_dict(ck.get("loss_func")))
     learn.load_state_dict(ck["state_dict"])
     return learn
 
@@ -641,7 +662,8 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
     `data_path/{trai,vali}/{img_tiles,mask_tiles}/*.tif` (utils.py:25-36, data.py:102-105); trains with fastai's recipe
     (Adam, wd 0.01, discriminative lrs `slice(lr/ENCODER_FACTOR, lr)`, one-cycle) and writes
     `<model_Path>/<description>/<description>.pkl`, `.json` and `_history.csv` (train.py:314-320, 234, 255).
-    `enable_regression`: n_out 1, MSELossFlat, rmse / R2Score, monitor r2_score (train.py:189-201).  8- and 16-bit tiles
+    `enable_regression`: n_out 1, MSELossFlat, rmse / R2Score, monitor r2_score (train.py:189-201).  `loss_func` picks
+    the classification loss as `unet_learner_MS` describes; it is recorded in `<description>.json`.  8- and 16-bit tiles
     follow the reference's input contract (`get_datatype`).  `transforms=True` applies the geometric part of the reference's
     augmentation (flips / 90-degree rotations of image and mask together, on the device-bound batch) to the share
     `n_transform_imgs` of every batch; albumentations pipeline objects (`aug_pipe`), the LR finder, plots and the model
@@ -691,7 +713,8 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
         cw = list(CLASS_WEIGHTS)
     learn = unet_learner_MS(nb, n_classes, ARCHITECTURE, (h, w), BATCH_SIZE, class_weights=cw, lr=LEARNING_RATE,
                             encoder_factor=ENCODER_FACTOR, self_attention=self_attention, regression=regression,
-                            input_dtype=torch.from_numpy(np.zeros(0, dtype=np_dt)).dtype, sixteen_bit=sixteen_bit)
+                            input_dtype=torch.from_numpy(np.zeros(0, dtype=np_dt)).dtype, sixteen_bit=sixteen_bit,
+                            loss_func=loss_func)
     if existing_model:
         if not os.path.exists(existing_model):
             raise FileNotFoundError(existing_model)
@@ -720,7 +743,7 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
                        "class_weights": cw, "batch_size": BATCH_SIZE, "epochs": EPOCHS, "learning_rate": LEARNING_RATE,
                        "encoder_factor": ENCODER_FACTOR, "train_tiles": len(train_files), "valid_tiles": len(valid_files),
                        "class_zero": bool(class_zero), "enable_regression": regression, "datatype": "int16" if sixteen_bit else "int8",
-                       "n_gpus": world, "history": learn.history}, f, indent=1)
+                       "n_gpus": world, "loss_func": learn.loss_spec.as_dict(), "history": learn.history}, f, indent=1)
     _barrier()
     return learn
 
