@@ -308,6 +308,16 @@ int b2u_im2col(const void* x, int32_t ldx, int32_t C, int32_t N, int32_t H, int3
  * the device */
 int b2u_crop_tiles(const void* raster, int32_t r_dtype, float div, float div2, int32_t C, int64_t Y, int64_t X,
                    const int32_t* y0, const int32_t* x0, int32_t T, int32_t P, void* out, int32_t ld, void* stream);
+/* Training batch cut out of a device-resident raster and its label raster, with the dihedral augmentation in the same
+ * pass: the crop of create_tiles_unet.py:410 (the image and mask tiles split_raster writes) and the flips / 90-degree
+ * rotations of utils.py:196-295 (SegmentationAlbumentationsTransform on image and mask together).
+ *   x[t][c] = D_op[t](raster[c, y0[t]:y0[t]+P, x0[t]:x0[t]+P])      raw band values of r_dtype (B2U_DT_U8/U16/I16)
+ *   y[t]    = D_op[t](labels[y0[t]:y0[t]+P, x0[t]:x0[t]+P])          l_dtype B2U_DT_U8 (class ids) or B2U_DT_F32
+ * raster [C][Y][X], labels [Y][X]; y0 / x0 / op are device int32 [T].  D_op flips the last axis when op & 4, then turns
+ * op & 3 quarter turns as torch.rot90(., k, (-2, -1)); op 0 is the identity.  Pixels outside the raster are zero. */
+int b2u_crop_train_batch(const void* raster, int32_t r_dtype, int32_t C, int64_t Y, int64_t X, const void* labels,
+                         int32_t l_dtype, const int32_t* y0, const int32_t* x0, const int32_t* op, int32_t T, int32_t P,
+                         void* x, void* y, void* stream);
 /* bf16/f32 NHWC -> fp32 NCHW */
 int b2u_nhwc_to_nchw_f32(const void* x, int32_t x_is_f32, int32_t ld, float* y, int32_t N, int32_t C, int32_t H,
                          int32_t W, void* stream);

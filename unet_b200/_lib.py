@@ -153,6 +153,7 @@ def _declare(lib):
         "b2u_pointwise_smallk": [vp, i32, i32, vp, i32, vp, i32, vp, i32, i64, i32, vp],
         "b2u_im2col": [vp, i32, i32, i32, i32, i32, i32, i32, i32, vp, i32, vp],
         "b2u_crop_tiles": [vp, i32, f32, f32, i32, i64, i64, vp, vp, i32, i32, vp, i32, vp],
+        "b2u_crop_train_batch": [vp, i32, i32, i64, i64, vp, i32, vp, vp, vp, i32, i32, vp, vp, vp],
         "b2u_nhwc_to_nchw_f32": [vp, i32, i32, vp, i32, i32, i32, i32, vp],
         "b2u_ce_weight_sum": [u8p, i64, vp, i32, vp, i32, vp],
         "b2u_ce_fwd_bwd": [vp, i32, u8p, i64, i32, vp, vp, i32, vp, i32, vp, i32, f32, vp],

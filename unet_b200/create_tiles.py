@@ -14,7 +14,7 @@ from __future__ import annotations
 import os
 import warnings
 from pathlib import Path
-from typing import List, Optional, Sequence
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -34,16 +34,15 @@ def _keep(crop: np.ndarray, max_empty: float) -> bool:
     return crop.size != 0 and not (np.sum(crop != 0) < np.prod(crop.shape) * (1 - max_empty))
 
 
-def create_train_test_split(path, split: Optional[Sequence[float]] = None, seed: int = 0) -> dict:
-    """create_tiles_unet.py:70-176: moves `path/img_tiles/*.tif` + `path/mask_tiles/*.tif` into `trai/`, `vali/` (and
-    `test/` when the third ratio is non-zero); returns the file names per subset."""
+def split_names(names: Sequence[str], split: Optional[Sequence[float]] = None, seed: int = 0) -> Dict[str, List[str]]:
+    """The subset decision of create_tiles_unet.py:70-176: tile names -> {"trai": [...], "vali": [...] (, "test": [...])}
+    by a seeded shuffle of the sorted names; a third subset only when the third ratio is non-zero."""
     if split is None:
         split = [0.7, 0.2, 0.1]
     if np.round(np.sum(split), decimals=3) != 1.0:
         split = [0.7, 0.2, 0.1]
         warnings.warn("Train/Vali/Test-Split percentage does not sum to 1, reseting to 70%/20%/10%.")
-    src = Path(path)
-    files = sorted(p.name for p in (src / "img_tiles").glob("*.tif"))
+    files = sorted(names)
     np.random.default_rng(seed).shuffle(files)
     n = len(files)
     three = len(split) == 3 and split[-1] != 0
@@ -52,6 +51,14 @@ def create_train_test_split(path, split: Optional[Sequence[float]] = None, seed:
     parts = {"trai": files[:a], "vali": files[a:b]}
     if three:
         parts["test"] = files[b:]
+    return parts
+
+
+def create_train_test_split(path, split: Optional[Sequence[float]] = None, seed: int = 0) -> dict:
+    """create_tiles_unet.py:70-176: moves `path/img_tiles/*.tif` + `path/mask_tiles/*.tif` into `trai/`, `vali/` (and
+    `test/` when the third ratio is non-zero) as `split_names` decides; returns the file names per subset."""
+    src = Path(path)
+    parts = split_names([p.name for p in (src / "img_tiles").glob("*.tif")], split, seed)
     for name, fs in parts.items():
         for sub in ("img_tiles", "mask_tiles"):
             (src / name / sub).mkdir(parents=True, exist_ok=True)
@@ -66,13 +73,20 @@ def create_train_test_split(path, split: Optional[Sequence[float]] = None, seed:
     return parts
 
 
-def split_raster(path_to_raster=None, path_to_mask=None, base_dir=".", patch_size: int = 400, patch_overlap: float = 0.20,
-                 split: Optional[Sequence[float]] = None, max_empty: float = 0.9, class_zero: bool = False,
-                 seed: int = 0) -> List[Path]:
-    """create_tiles_unet.py:252-431 with the reference's argument order.  Cuts the raster (and its mask) into
-    `patch_size` windows with `patch_overlap`, zeroes no-data pixels in both, drops tiles that are more than `max_empty`
-    zeros, writes `<base_dir>/img_tiles/<raster>_<index>.tif` (+ `mask_tiles/`) with the window's georeferencing and -
-    when a mask is given - distributes them into trai / vali / test.  Returns the image-tile paths written."""
+class PreparedRaster(NamedTuple):
+    """What `split_raster` cuts its tiles from: the raster `[C, H, W]` and its mask `[bands, H, W]` (None without one)
+    after the class_zero shift and the no-data zeroing, and the kept tiles as (file name, window (x, y, w, h))."""
+    image: np.ndarray
+    mask: Optional[np.ndarray]
+    geo: GeoInfo
+    tiles: List[Tuple[str, Window]]
+
+
+def prepare_raster(path_to_raster, path_to_mask=None, patch_size: int = 400, patch_overlap: float = 0.20,
+                   max_empty: float = 0.9, class_zero: bool = False) -> PreparedRaster:
+    """The decisions of create_tiles_unet.py:252-431 before any file is written: class_zero shift of the mask, no-data
+    pixels of image and mask zeroed in both, the grid check, the windows, the empty-tile filter (:414/:422) and the
+    tile names `<raster stem>_<window index>.tif`."""
     if path_to_raster is None:
         raise ValueError("path_to_raster is required")
     image, geo = read_geotiff(path_to_raster)
@@ -107,30 +121,46 @@ def split_raster(path_to_raster=None, path_to_mask=None, base_dir=".", patch_siz
     if H < patch_size or W < patch_size:
         raise ValueError("Patch size of {} is larger than the image dimensions {}".format(patch_size, [H, W]))   # :398-400
     windows = compute_windows(img_hwc, patch_size, patch_overlap)
+    stem = os.path.splitext(os.path.basename(str(path_to_raster)))[0]
+    tiles = []
+    for index, (x, y, w, h) in enumerate(windows):
+        if not _keep(image[:, y:y + h, x:x + w], max_empty):
+            continue
+        if include_mask and not _keep(mask[:1, y:y + h, x:x + w], max_empty):
+            continue
+        tiles.append((f"{stem}_{index}.tif", (x, y, w, h)))
+    return PreparedRaster(image, mask, geo, tiles)
+
+
+def split_raster(path_to_raster=None, path_to_mask=None, base_dir=".", patch_size: int = 400, patch_overlap: float = 0.20,
+                 split: Optional[Sequence[float]] = None, max_empty: float = 0.9, class_zero: bool = False,
+                 seed: int = 0) -> List[Path]:
+    """create_tiles_unet.py:252-431 with the reference's argument order.  Cuts the raster (and its mask) into
+    `patch_size` windows with `patch_overlap`, zeroes no-data pixels in both, drops tiles that are more than `max_empty`
+    zeros, writes `<base_dir>/img_tiles/<raster>_<index>.tif` (+ `mask_tiles/`) with the window's georeferencing and -
+    when a mask is given - distributes them into trai / vali / test.  Returns the image-tile paths written."""
+    prep = prepare_raster(path_to_raster, path_to_mask, patch_size, patch_overlap, max_empty, class_zero)
+    image, mask, geo = prep.image, prep.mask, prep.geo
+    include_mask = mask is not None
     base = Path(base_dir)
     (base / "img_tiles").mkdir(parents=True, exist_ok=True)
     if include_mask:
         (base / "mask_tiles").mkdir(parents=True, exist_ok=True)
-    stem = os.path.splitext(os.path.basename(str(path_to_raster)))[0]
     written = []
-    for index, (x, y, w, h) in enumerate(windows):
-        crop = image[:, y:y + h, x:x + w]
-        if not _keep(crop, max_empty):
-            continue
-        if include_mask:
-            crop_mask = mask[:1, y:y + h, x:x + w]
-            if not _keep(crop_mask, max_empty):
-                continue
+    for name, (x, y, w, h) in prep.tiles:
         g = geo.window(x, y)
         g = GeoInfo(g.geotransform, g.geokeys, g.geodoubles, g.geoascii, None, g.georeferenced)
-        name = f"{stem}_{index}.tif"
-        write_geotiff(base / "img_tiles" / name, crop, g)
+        write_geotiff(base / "img_tiles" / name, image[:, y:y + h, x:x + w], g)
         if include_mask:
-            cm = crop_mask if crop_mask.dtype.kind == "f" else crop_mask.astype(np.uint8)      # :236-241 Float32 or Byte
-            write_geotiff(base / "mask_tiles" / name, cm, g)
+            write_geotiff(base / "mask_tiles" / name, mask_tile_values(mask[:1, y:y + h, x:x + w]), g)
         written.append(base / "img_tiles" / name)
     if include_mask:
         parts = create_train_test_split(base, split=split, seed=seed)
         where = {f: k for k, fs in parts.items() for f in fs}
         written = [base / where[p.name] / "img_tiles" / p.name for p in written]
     return written
+
+
+def mask_tile_values(mask: np.ndarray) -> np.ndarray:
+    """The values a mask tile is stored with (:236-241): a floating-point mask keeps its type, any other becomes Byte."""
+    return mask if mask.dtype.kind == "f" else mask.astype(np.uint8)

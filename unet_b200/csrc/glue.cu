@@ -538,6 +538,77 @@ __global__ void crop_tiles_kernel(const void* __restrict__ raster, int dtype, fl
   }
 }
 
+// Source pixel (si, sj) of output pixel (i, j) of a dihedrally transformed P x P tile: bit 2 of `op` flips the last axis
+// first, then op & 3 quarter turns of torch.rot90(., k, (-2, -1)).
+__device__ __forceinline__ void dihedral_src(int op, int P, int i, int j, int& si, int& sj) {
+  int u, v;
+  switch (op & 3) {
+    case 0: u = i; v = j; break;
+    case 1: u = j; v = P - 1 - i; break;
+    case 2: u = P - 1 - i; v = P - 1 - j; break;
+    default: u = P - 1 - j; v = i; break;
+  }
+  si = u;
+  sj = (op & 4) ? P - 1 - v : v;
+}
+
+// One 32 x 32 block of one output plane.  The map is a signed permutation of the two axes, so the source pixels of an
+// output block form one axis-aligned 32 x 32 block (hanging over the tile edge when P is not a multiple of 32): it is
+// read row by row into shared memory and written back row by row, so that both sides stay coalesced when a quarter
+// turn transposes.  Pixels outside the raster read as zero, as in crop_tiles_kernel.
+template <typename T>
+__device__ __forceinline__ void crop_dihedral_block(const T* __restrict__ src, long long Y, long long X, int y0, int x0,
+                                                    int op, int P, int a, int b, T* __restrict__ dst, T* tile) {
+  int s0i, s0j, s1i, s1j;
+  dihedral_src(op, P, a, b, s0i, s0j);
+  dihedral_src(op, P, a + 31, b + 31, s1i, s1j);
+  const int ri = min(s0i, s1i), rj = min(s0j, s1j);
+  for (int r = threadIdx.y; r < 32; r += blockDim.y) {
+    const int si = ri + r, sj = rj + (int)threadIdx.x;
+    if (si >= 0 && si < P && sj >= 0 && sj < P) {
+      const long long gy = (long long)y0 + si, gx = (long long)x0 + sj;
+      tile[r * 33 + threadIdx.x] = (gy >= 0 && gy < Y && gx >= 0 && gx < X) ? src[gy * X + gx] : T(0);
+    }
+  }
+  __syncthreads();
+  for (int r = threadIdx.y; r < 32; r += blockDim.y) {
+    const int i = a + r, j = b + (int)threadIdx.x;
+    if (i < P && j < P) {
+      int si, sj;
+      dihedral_src(op, P, i, j, si, sj);
+      dst[(long long)i * P + j] = tile[(si - ri) * 33 + (sj - rj)];
+    }
+  }
+}
+
+// grid (tile blocks, C + 1, T): plane c < C of tile t is image band c, plane C its label
+template <typename TI, typename TL>
+__global__ void __launch_bounds__(256) crop_train_batch_kernel(const TI* __restrict__ raster, const TL* __restrict__ labels,
+                                                               int C, long long Y, long long X, const int* __restrict__ ty0,
+                                                               const int* __restrict__ tx0, const int* __restrict__ top,
+                                                               int P, int nb, TI* __restrict__ x, TL* __restrict__ y) {
+  __shared__ __align__(16) unsigned char smem[32 * 33 * 4];
+  pdl_enter();
+  const int t = blockIdx.z, c = blockIdx.y;
+  const int a = (blockIdx.x / nb) * 32, b = (blockIdx.x % nb) * 32;
+  const int y0 = ty0[t], x0 = tx0[t], op = top[t];
+  const long long PP = (long long)P * P;
+  if (c < C)
+    crop_dihedral_block(raster + (long long)c * Y * X, Y, X, y0, x0, op, P, a, b, x + ((long long)t * C + c) * PP,
+                        reinterpret_cast<TI*>(smem));
+  else
+    crop_dihedral_block(labels, Y, X, y0, x0, op, P, a, b, y + (long long)t * PP, reinterpret_cast<TL*>(smem));
+}
+
+template <typename TI, typename TL>
+static cudaError_t launch_crop_train_batch(const void* raster, const void* labels, int C, long long Y, long long X,
+                                           const int* y0, const int* x0, const int* op, int T, int P, void* x, void* y,
+                                           cudaStream_t st) {
+  const int nb = (P + 31) / 32;
+  return launch_k(crop_train_batch_kernel<TI, TL>, dim3(nb * nb, C + 1, T), dim3(32, 8), 0, st, (const TI*)raster,
+                  (const TL*)labels, C, Y, X, y0, x0, op, P, nb, (TI*)x, (TL*)y);
+}
+
 __global__ void nhwc_to_nchw_f32_kernel(const void* __restrict__ x, int is_f32, int ld, float* __restrict__ y, int N,
                                         int C, int H, int W) {
   pdl_enter();
@@ -1333,6 +1404,34 @@ extern "C" int b2u_crop_tiles(const void* raster, int32_t r_dtype, float div, fl
   const long long items = (long long)T * P * P;
   launch_k(crop_tiles_kernel, dim3(grid_for(items, 256)), dim3(256), 0, (cudaStream_t)stream, raster, r_dtype, div, div2, C, Y, X, y0,
            x0, T, P, (bf)out, ld);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_crop_train_batch(const void* raster, int32_t r_dtype, int32_t C, int64_t Y, int64_t X, const void* labels,
+                                    int32_t l_dtype, const int32_t* y0, const int32_t* x0, const int32_t* op, int32_t T,
+                                    int32_t P, void* x, void* y, void* stream) {
+  B2U_CHECK_ARG(raster && labels && y0 && x0 && op && x && y, "crop_train_batch: null argument");
+  B2U_CHECK_ARG(C > 0 && C < 65535 && T > 0 && T <= 65535 && P > 0 && P <= Y && P <= X && (long long)P * P < (1ll << 31),
+                "crop_train_batch: C=%d T=%d P=%d Y=%lld X=%lld out of range", C, T, P, (long long)Y, (long long)X);
+  B2U_CHECK_ARG(r_dtype >= B2U_DT_U8 && r_dtype <= B2U_DT_I16,
+                "crop_train_batch: r_dtype=%d (1 u8, 2 u16, 3 i16)", r_dtype);
+  B2U_CHECK_ARG(l_dtype == B2U_DT_U8 || l_dtype == B2U_DT_F32, "crop_train_batch: l_dtype=%d (0 f32, 1 u8)", l_dtype);
+  const cudaStream_t st = (cudaStream_t)stream;
+  const bool f = l_dtype == B2U_DT_F32;
+  switch (r_dtype) {
+    case B2U_DT_U8:
+      f ? launch_crop_train_batch<uint8_t, float>(raster, labels, C, Y, X, y0, x0, op, T, P, x, y, st)
+        : launch_crop_train_batch<uint8_t, uint8_t>(raster, labels, C, Y, X, y0, x0, op, T, P, x, y, st);
+      break;
+    case B2U_DT_U16:
+      f ? launch_crop_train_batch<uint16_t, float>(raster, labels, C, Y, X, y0, x0, op, T, P, x, y, st)
+        : launch_crop_train_batch<uint16_t, uint8_t>(raster, labels, C, Y, X, y0, x0, op, T, P, x, y, st);
+      break;
+    default:
+      f ? launch_crop_train_batch<int16_t, float>(raster, labels, C, Y, X, y0, x0, op, T, P, x, y, st)
+        : launch_crop_train_batch<int16_t, uint8_t>(raster, labels, C, Y, X, y0, x0, op, T, P, x, y, st);
+  }
   B2U_LAUNCH_CHECK();
   return B2U_OK;
 }

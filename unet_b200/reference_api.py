@@ -123,8 +123,9 @@ class Learner:
                     self.trainer.set_adam_hyper(lr, mom)
                 else:
                     self.trainer.lr = lr
-                # the next batch's H2D copy runs behind this step; the loss stays on the device (no host sync per step)
-                loss = self.trainer.step(x, y, prefetch=None if nxt is None else (nxt[0], nxt[1]))
+                # the next batch's H2D copy runs behind this step; the loss stays on the device (no host sync per step).
+                # Device batches are not prefetched: the side copy stream would not wait for the kernel producing them.
+                loss = self.trainer.step(x, y, prefetch=None if nxt is None or nxt[0].is_cuda else (nxt[0], nxt[1]))
                 if n < losses.numel():
                     losses[n:n + 1].copy_(loss, non_blocking=True)
                 n += 1
@@ -608,49 +609,97 @@ def get_datatype(files: Sequence[Path]) -> str:
     """utils.py:72-89: the dataset kind is read off the FIRST training tile - 'int8' when its largest value (ignoring
     nodata pixels of band 1) is below 257, else 'int16' - and decides whether the batch transform divides by 255."""
     arr, geo = read_geotiff(files[0])
-    keep = np.ones(arr.shape[1:], dtype=bool) if getattr(geo, "nodata", None) is None else arr[0] != geo.nodata
-    vals = arr[:, keep]
+    return _dataset_kind(arr, getattr(geo, "nodata", None))
+
+
+def _dataset_kind(tile: np.ndarray, nodata) -> str:
+    """`get_datatype` on the values of a `[bands, H, W]` tile"""
+    keep = np.ones(tile.shape[1:], dtype=bool) if nodata is None else tile[0] != nodata
+    vals = tile[:, keep]
     return "int8" if (vals.size == 0 or vals.max() < 257) else "int16"
+
+
+class _BatchDeal:
+    """The batch sequence of one epoch over `n_items` samples (data.py:100-105 DataLoader semantics): a shuffle seeded
+    with `shuffle_seed + epoch` (None: file order), `drop_last`, and with `drop_last=False` a last partial batch padded
+    by repeating its first sample (`n_real` tells how many samples count).  Data parallel: the global batch sequence is
+    dealt round-robin, rank r takes batches r, r + world, ... and every rank sees the same number of batches (the
+    gradient all-reduce needs equal step counts)."""
+
+    def __init__(self, n_items: int, batch_size: int, shuffle_seed: Optional[int], drop_last: bool, rank: int = 0,
+                 world: int = 1):
+        self.n_items, self.batch_size, self.shuffle_seed, self.rank, self.world = n_items, batch_size, shuffle_seed, rank, world
+        n_global = n_items // batch_size if drop_last else -(-n_items // batch_size)
+        self.n_batches = n_global // world if world > 1 else n_global
+
+    def __call__(self, epoch: int) -> List[Tuple[List[int], int]]:
+        """[(sample indices of the batch, n_real)] of this rank in `epoch`"""
+        order = list(range(self.n_items))
+        if self.shuffle_seed is not None:
+            np.random.default_rng(self.shuffle_seed + epoch).shuffle(order)      # the same order on every rank
+        out = []
+        for k in range(self.n_batches):
+            b0 = (k * self.world + self.rank) * self.batch_size
+            idx = order[b0:b0 + self.batch_size]
+            n_real = len(idx)
+            if n_real < self.batch_size:
+                idx = idx + [idx[0]] * (self.batch_size - n_real)
+            out.append((idx, n_real))
+        return out
 
 
 def _tile_batches(files: Sequence[Path], batch_size: int, n_classes: int, class_zero: bool, shuffle_seed: Optional[int],
                   drop_last: bool, regression: bool = False, rank: int = 0, world: int = 1):
     """Batches of (raw tiles [B,n_in,H,W], labels [B,H,W], n_real) from `img_tiles/*.tif` + `mask_tiles/*.tif`
-    (data.py:100-105, utils.py:40-55): labels are uint8 class ids, or the float32 mask band for the regression variant
-    (RegressionBlock).  With `drop_last=False` the last partial batch is padded by repetition and `n_real` tells how
-    many samples count.  Data parallel: the global batch sequence is dealt round-robin, rank r takes batches r, r + world,
-    ... and every rank sees the same number of batches (the gradient all-reduce needs equal step counts)."""
-    n_global = len(files) // batch_size if drop_last else -(-len(files) // batch_size)
-    n_batches = n_global // world if world > 1 else n_global
+    (data.py:100-105, utils.py:40-55) in the order `_BatchDeal` deals them: labels are uint8 class ids, or the float32
+    mask band for the regression variant (RegressionBlock)."""
+    deal = _BatchDeal(len(files), batch_size, shuffle_seed, drop_last, rank, world)
 
     def gen():
-        order = list(range(len(files)))
+        epoch = gen.epoch
         if shuffle_seed is not None:
-            np.random.default_rng(shuffle_seed + gen.epoch).shuffle(order)      # the same order on every rank
             gen.epoch += 1
-        for k in range(n_batches):
-            b0 = (k * world + rank) * batch_size
-            idx = order[b0:b0 + batch_size]
-            n_real = len(idx)
-            if n_real < batch_size:
-                idx = idx + [idx[0]] * (batch_size - n_real)
+        for idx, n_real in deal(epoch):
             xs, ys = [], []
             for i in idx:
                 x = open_tile(files[i])
                 if x.dtype not in _NP_OK:
                     raise ValueError(f"{files[i]}: {x.dtype} tiles are not supported (uint8, uint16 or int16 band values)")
-                y = open_mask(files[i])
-                if regression:
-                    ys.append(y.astype(np.float32))
-                else:
-                    if y.max() >= n_classes:
-                        raise ValueError(f"{files[i]}: mask label {int(y.max())} >= number of classes {n_classes}")
-                    ys.append(y.astype(np.uint8))
                 xs.append(x)
+                ys.append(_label_values(open_mask(files[i]), n_classes, regression, files[i]))
             yield torch.from_numpy(np.stack(xs)), torch.from_numpy(np.stack(ys)), n_real
     gen.epoch = 0
-    gen.n_batches = n_batches        # known without touching the files (fit_one_cycle sizes its schedule with it)
+    gen.n_batches = deal.n_batches   # known without touching the files (fit_one_cycle sizes its schedule with it)
     return gen
+
+
+def _label_values(y: np.ndarray, n_classes: int, regression: bool, where) -> np.ndarray:
+    """mask tile values -> training labels: float32 targets (regression) or uint8 class ids below `n_classes`"""
+    if regression:
+        return y.astype(np.float32)
+    if y.max() >= n_classes:
+        raise ValueError(f"{where}: mask label {int(y.max())} >= number of classes {n_classes}")
+    return y.astype(np.uint8)
+
+
+def _class_weights(CLASS_WEIGHTS, n_classes: int, regression: bool, train_masks: Iterable[np.ndarray]) -> List[float]:
+    """train.py:330-339: the loss weights.  `train_masks` (the mask tiles of the first 1200 training samples, read only
+    for "weighted") feed utils.py:105-117 get_class_weights: total / count per class.  The reference takes the counts
+    from `unique()`, which silently drops absent classes; here an absent class keeps its slot (count clamped to 1).  The
+    weighted-mean CE is invariant to the common scale."""
+    if regression:
+        return [1.0]                                                               # train.py:330-331
+    if isinstance(CLASS_WEIGHTS, str):
+        if CLASS_WEIGHTS == "even":
+            return [1.0 / n_classes] * n_classes                                   # train.py:338-339
+        if CLASS_WEIGHTS == "weighted":
+            counts = np.zeros(n_classes, dtype=np.float64)
+            for m in train_masks:
+                counts += np.bincount(m.ravel(), minlength=n_classes)[:n_classes]
+            # plain floats: the exported checkpoint must load with weights_only=True (no numpy scalars)
+            return [float(v) for v in counts.sum() / np.maximum(counts, 1.0)]
+        raise ValueError(f"CLASS_WEIGHTS {CLASS_WEIGHTS!r} not understood")
+    return list(CLASS_WEIGHTS)
 
 
 def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, visualize_data_example=False,
@@ -670,7 +719,6 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
     summary are outside the built path and are skipped with a warning.
     Data parallel: launched under `torch.distributed.run` (params_and_main `N_GPUS`), every rank trains on its share of
     the batches, gradients are all-reduced by the trainer, and only rank 0 writes files.  Returns the trained Learner."""
-    import json
     from .engine import init_distributed
     rank, _, world = init_distributed() if int(os.environ.get("WORLD_SIZE", "1")) > 1 else (0, 0, 1)
     if LR_FINDER:
@@ -690,27 +738,36 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
     nb, h, w, np_dt, _ = geotiff_info(train_files[0])                              # train.py:124-125 probes the first item
     if np_dt not in _NP_OK:
         raise ValueError(f"{train_files[0]}: {np_dt} tiles are not supported (uint8, uint16 or int16 band values)")
-    sixteen_bit = get_datatype(train_files) == "int16"                             # train.py:298
+    n_classes = len(CODES)
+    regression = bool(enable_regression)
+    tb = _tile_batches(train_files, BATCH_SIZE, n_classes, class_zero, shuffle_seed=0,
+                       drop_last=len(train_files) >= BATCH_SIZE * world, regression=regression, rank=rank, world=world)
+    if transforms:
+        tb = augmented(tb, float(n_transform_imgs), seed=0 if split_idx is None else int(split_idx))
+    # every rank validates the whole validation set (identical metrics on every rank: no collective, same best epoch)
+    vb = _tile_batches(valid_files, BATCH_SIZE, n_classes, class_zero, None, False, regression=regression) if valid_files else None
+    return _train_and_export(
+        tb, vb, len(train_files), len(valid_files), rank, world, nb, (h, w), np_dt,
+        sixteen_bit=get_datatype(train_files) == "int16",                                                    # train.py:298
+        class_weights=_class_weights(CLASS_WEIGHTS, n_classes, regression, (open_mask(f) for f in train_files[:1200])),
+        model_Path=model_Path, description=description, BATCH_SIZE=BATCH_SIZE, existing_model=existing_model,
+        enable_regression=regression, ARCHITECTURE=ARCHITECTURE, EPOCHS=EPOCHS, LEARNING_RATE=LEARNING_RATE,
+        ENCODER_FACTOR=ENCODER_FACTOR, loss_func=loss_func, monitor=monitor, self_attention=self_attention, CODES=CODES,
+        class_zero=class_zero)
+
+
+def _train_and_export(tb, vb, n_train: int, n_valid: int, rank: int, world: int, nb: int, tile_hw: Tuple[int, int], np_dt,
+                      sixteen_bit: bool, class_weights: List[float], *, model_Path, description, BATCH_SIZE,
+                      existing_model, enable_regression, ARCHITECTURE, EPOCHS, LEARNING_RATE, ENCODER_FACTOR, loss_func,
+                      monitor, self_attention, CODES, class_zero, extra_json: Optional[dict] = None):
+    """train.py:287-375 after the data is found: learner, monitor rules, fit, export and the description JSON, over the
+    training / validation batch sources `tb` / `vb` (callables as `fit_one_cycle` takes them; `vb` may be None)."""
+    import json
     codes = list(CODES)
     n_classes = len(codes)
     regression = bool(enable_regression)
-    if regression:
-        cw = [1.0]                                                                 # train.py:330-331
-    elif isinstance(CLASS_WEIGHTS, str):
-        if CLASS_WEIGHTS == "even":
-            cw = [1.0 / n_classes] * n_classes                                     # train.py:338-339
-        elif CLASS_WEIGHTS == "weighted":
-            # utils.py:105-117 get_class_weights: total / count per class over (up to 1200) training masks.  The
-            # reference takes the counts from `unique()`, which silently drops absent classes; here an absent class
-            # keeps its slot (count clamped to 1).  The weighted-mean CE is invariant to the common scale.
-            counts = np.zeros(n_classes, dtype=np.float64)
-            for f in train_files[:1200]:
-                counts += np.bincount(open_mask(f).ravel(), minlength=n_classes)[:n_classes]
-            cw = list(counts.sum() / np.maximum(counts, 1.0))
-        else:
-            raise ValueError(f"CLASS_WEIGHTS {CLASS_WEIGHTS!r} not understood")
-    else:
-        cw = list(CLASS_WEIGHTS)
+    cw = class_weights
+    h, w = tile_hw
     learn = unet_learner_MS(nb, n_classes, ARCHITECTURE, (h, w), BATCH_SIZE, class_weights=cw, lr=LEARNING_RATE,
                             encoder_factor=ENCODER_FACTOR, self_attention=self_attention, regression=regression,
                             input_dtype=torch.from_numpy(np.zeros(0, dtype=np_dt)).dtype, sixteen_bit=sixteen_bit,
@@ -722,12 +779,6 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
     out_dir = Path(model_Path) / description
     if rank == 0:
         out_dir.mkdir(parents=True, exist_ok=True)
-    tb = _tile_batches(train_files, BATCH_SIZE, n_classes, class_zero, shuffle_seed=0,
-                       drop_last=len(train_files) >= BATCH_SIZE * world, regression=regression, rank=rank, world=world)
-    if transforms:
-        tb = augmented(tb, float(n_transform_imgs), seed=0 if split_idx is None else int(split_idx))
-    # every rank validates the whole validation set (identical metrics on every rank: no collective, same best epoch)
-    vb = _tile_batches(valid_files, BATCH_SIZE, n_classes, class_zero, None, False, regression=regression) if valid_files else None
     if monitor not in (None, "train_loss", "valid_loss", "r2_score", "dice_multi"):
         raise ValueError("Monitor must be one of ['train_loss', 'valid_loss', 'r2_score', 'dice_multi']")    # train.py:207-208
     mon = monitor or ("r2_score" if regression else "dice_multi")                                             # train.py:198-201
@@ -741,38 +792,205 @@ def train_func(data_path, existing_model, model_Path, description, BATCH_SIZE, v
         with open(out_dir / f"{description}.json", "w") as f:
             json.dump({"description": description, "architecture": learn.arch, "bands": nb, "tile": [h, w], "codes": codes,
                        "class_weights": cw, "batch_size": BATCH_SIZE, "epochs": EPOCHS, "learning_rate": LEARNING_RATE,
-                       "encoder_factor": ENCODER_FACTOR, "train_tiles": len(train_files), "valid_tiles": len(valid_files),
+                       "encoder_factor": ENCODER_FACTOR, "train_tiles": n_train, "valid_tiles": n_valid,
                        "class_zero": bool(class_zero), "enable_regression": regression, "datatype": "int16" if sixteen_bit else "int8",
-                       "n_gpus": world, "loss_func": learn.loss_spec.as_dict(), "history": learn.history}, f, indent=1)
+                       "n_gpus": world, "loss_func": learn.loss_spec.as_dict(), **(extra_json or {}),
+                       "history": learn.history}, f, indent=1)
     _barrier()
     return learn
+
+
+def train_geotiff(pairs, patch_size: int = 400, patch_overlap: float = 0.20, split: Optional[Sequence[float]] = None,
+                  max_empty: float = 0.9, class_zero: bool = False, seed: int = 0, *, model_Path, description,
+                  BATCH_SIZE, existing_model=None, enable_regression=False, CLASS_WEIGHTS="even",
+                  ARCHITECTURE="xresnet34", EPOCHS=1, LEARNING_RATE=1e-3, ENCODER_FACTOR=10, loss_func=None,
+                  monitor=None, self_attention=False, VALID_SCENES=("vali",), CODES=("background", "class1"),
+                  transforms=False, split_idx=None, n_transform_imgs=0):
+    """Tile-free variant of the training path: what `split_raster(raster, mask, base_dir, patch_size, patch_overlap,
+    split, max_empty, class_zero, seed)` for every pair into one `base_dir`, then `train_func(base_dir, ...)` with the
+    same training arguments produce - the same weights, history, metrics and exported model - without writing a tile.
+    `pairs` is one (raster, mask) pair of GeoTIFF paths or a list of them.  The prepared rasters and labels are uploaded
+    once; every batch is cut out of them on the device by `b2u_crop_train_batch`, with the dihedral augmentation of
+    `transforms` in the same pass, so no host work on pixels remains per step.  The windows are listed, split and
+    ordered exactly as `train_func` would find the tile files (`_raster_windows`).  Rasters must fit in host memory and
+    in HBM.  Data parallel under `torch.distributed.run`: every rank uploads the rasters and takes its share of the
+    batches; only rank 0 writes.  Returns the trained Learner."""
+    from .engine import init_distributed
+    share = _aug_share(n_transform_imgs) if transforms else None
+    regression = bool(enable_regression)
+    n_classes = len(CODES)
+    images, labels, train, valid = _raster_windows(pairs, patch_size, patch_overlap, split, max_empty, class_zero, seed,
+                                                   VALID_SCENES)
+    crop = lambda a, e: a[..., e[2][1]:e[2][1] + patch_size, e[2][0]:e[2][0] + patch_size]
+    for e in train + valid:
+        _label_values(crop(labels[e[1]], e), n_classes, regression, e[0])       # _tile_batches' check, before training
+    rank, _, world = init_distributed() if int(os.environ.get("WORLD_SIZE", "1")) > 1 else (0, 0, 1)
+    nb, np_dt = images[0].shape[0], images[0].dtype
+    # one device raster for all pairs: pair k occupies rows [yoff[k], yoff[k] + Y_k) and its own columns
+    yoff = np.cumsum([0] + [a.shape[1] for a in images])
+    Y, X = int(yoff[-1]), max(a.shape[2] for a in images)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    bits = lambda a: torch.from_numpy(a.view(np.int16) if a.dtype == np.uint16 else a)     # uint16 moved as its bits
+    pad = any(a.shape[2] != X for a in images)
+    alloc = torch.zeros if pad else torch.empty
+    img_d = alloc((nb, Y, X), dtype=bits(np.zeros(0, np_dt)).dtype, device=dev)
+    lab_d = alloc((Y, X), dtype=torch.float32 if regression else torch.uint8, device=dev)
+    for k, (a, lab) in enumerate(zip(images, labels)):
+        img_d[:, yoff[k]:yoff[k + 1], :a.shape[2]].copy_(bits(a))
+        lab_d[yoff[k]:yoff[k + 1], :a.shape[2]].copy_(torch.from_numpy(lab.astype(np.float32 if regression else np.uint8)))
+    yx = lambda es: np.array([(yoff[e[1]] + e[2][1], e[2][0]) for e in es], dtype=np.int32).reshape(-1, 2)
+    x_dtype = torch.from_numpy(np.zeros(0, dtype=np_dt)).dtype
+    tb = _raster_batches(img_d, lab_d, x_dtype, yx(train), patch_size, BATCH_SIZE,
+                         _BatchDeal(len(train), BATCH_SIZE, 0, len(train) >= BATCH_SIZE * world, rank, world),
+                         share, 0 if split_idx is None else int(split_idx))
+    # every rank validates the whole validation set, as train_func does
+    vb = _raster_batches(img_d, lab_d, x_dtype, yx(valid), patch_size, BATCH_SIZE,
+                         _BatchDeal(len(valid), BATCH_SIZE, None, False), None, 0) if valid else None
+    return _train_and_export(
+        tb, vb, len(train), len(valid), rank, world, nb, (patch_size, patch_size), np_dt,
+        sixteen_bit=_dataset_kind(crop(images[train[0][1]], train[0]), None) == "int16",
+        class_weights=_class_weights(CLASS_WEIGHTS, n_classes, regression, (crop(labels[e[1]], e) for e in train[:1200])),
+        model_Path=model_Path, description=description, BATCH_SIZE=BATCH_SIZE, existing_model=existing_model,
+        enable_regression=regression, ARCHITECTURE=ARCHITECTURE, EPOCHS=EPOCHS, LEARNING_RATE=LEARNING_RATE,
+        ENCODER_FACTOR=ENCODER_FACTOR, loss_func=loss_func, monitor=monitor, self_attention=self_attention, CODES=CODES,
+        class_zero=class_zero,
+        extra_json={"rasters": [str(r) for r, _ in _as_pairs(pairs)], "masks": [str(m) for _, m in _as_pairs(pairs)],
+                    "patch_size": patch_size, "patch_overlap": patch_overlap,
+                    "split": None if split is None else list(split), "max_empty": max_empty, "split_seed": seed})
+
+
+def _as_pairs(pairs) -> List[Tuple]:
+    """one (raster, mask) pair or a list of them -> a list of pairs"""
+    if isinstance(pairs, (tuple, list)) and len(pairs) == 2 and all(isinstance(q, (str, os.PathLike)) for q in pairs):
+        pairs = [pairs]
+    return [tuple(q) for q in pairs]
+
+
+def _raster_windows(pairs, patch_size: int, patch_overlap: float, split, max_empty: float, class_zero: bool, seed: int,
+                    VALID_SCENES):
+    """The tiles `split_raster` would write for every pair into one directory, in the order `train_func` would read
+    them: scenes in sorted order, names sorted inside a scene, every scene not in VALID_SCENES training (`test` of a
+    three-way split included).  Returns (prepared images, mask-tile values per pair, training entries, validation
+    entries); an entry is (tile name, pair index, window (x, y, w, h))."""
+    from .create_tiles import mask_tile_values, prepare_raster, split_names
+    pairs = _as_pairs(pairs)
+    if not pairs or any(len(q) != 2 or q[1] is None for q in pairs):
+        raise ValueError("train_geotiff needs one or more (raster, mask) pairs")
+    stems = [os.path.splitext(os.path.basename(str(r)))[0] for r, _ in pairs]
+    if len(set(stems)) != len(stems):
+        raise ValueError(f"raster names {stems} collide: split_raster would write their tiles over each other")
+    valid_scenes = [VALID_SCENES] if isinstance(VALID_SCENES, str) else list(VALID_SCENES)
+    images, labels, scenes = [], [], {}
+    for k, (raster, mask) in enumerate(pairs):
+        prep = prepare_raster(raster, mask, patch_size, patch_overlap, max_empty, class_zero)
+        if prep.image.dtype not in _NP_OK:
+            raise ValueError(f"{raster}: {prep.image.dtype} rasters are not supported (uint8, uint16 or int16 band values)")
+        wins = dict(prep.tiles)
+        for scene, names in split_names(list(wins), split, seed).items():
+            scenes.setdefault(scene, []).extend((name, k, wins[name]) for name in names)
+        images.append(prep.image)
+        labels.append(mask_tile_values(prep.mask[0]))
+    if len({(a.shape[0], a.dtype) for a in images}) != 1:
+        raise ValueError("the rasters differ in band count or sample type")
+    train, valid = [], []
+    for scene in sorted(scenes):
+        (valid if scene in valid_scenes else train).extend(sorted(scenes[scene], key=lambda e: e[0]))
+    if not train:
+        raise ValueError("no training windows: none was kept, or all of them went to validation scenes")
+    return images, labels, train, valid
+
+
+def _epoch_table(deal: _BatchDeal, epoch: int, yx: np.ndarray, share: Optional[float], aug_seed: int):
+    """The crop table of one epoch, int32 [n_batches, (y0, x0, op), B], and the n_real of every batch: the windows of
+    `deal(epoch)` and, when `share` is not None, the dihedral ops `augmented` would draw for them, in its order."""
+    batches = deal(epoch)
+    B = deal.batch_size
+    table = np.zeros((max(1, len(batches)), 3, B), dtype=np.int32)
+    rng = np.random.default_rng(aug_seed + epoch) if share is not None else None
+    for k, (idx, _) in enumerate(batches):
+        table[k, :2] = yx[idx].T
+        for i, op in (_aug_ops(rng, B, share) if rng is not None else ()):
+            table[k, 2, i] = op
+    return table, [n for _, n in batches]
+
+
+_RASTER_DT = {torch.uint8: _lib.DT_U8, torch.uint16: _lib.DT_U16, torch.int16: _lib.DT_I16}
+
+
+def _raster_batches(img_d: torch.Tensor, lab_d: torch.Tensor, x_dtype: torch.dtype, yx: np.ndarray, P: int, B: int,
+                    deal: _BatchDeal, share: Optional[float], aug_seed: int):
+    """Device batches of (raw tiles [B,C,P,P], labels [B,P,P], n_real) cut out of the device raster `img_d` [C,Y,X] and
+    labels `lab_d` [Y,X] at the window origins `yx` [N, (y0, x0)]: the batches `_tile_batches` (wrapped in `augmented`
+    when `share` is not None) yields over the same windows.  An epoch's `_epoch_table` goes to the device in one copy
+    and each batch's crop reads its slice of it: no per-step host-to-device copy, no per-step synchronisation.  Batches
+    are cut into a ring of two buffers: `fit_one_cycle` takes batch k+1 before it enqueues step k, and stream order
+    keeps the buffer of step k intact until the step's input copy has run."""
+    lib, dev = _lib.load(), img_d.device
+    C, Y, X = img_d.shape
+    ring = [(torch.empty((B, C, P, P), dtype=x_dtype, device=dev), torch.empty((B, P, P), dtype=lab_d.dtype, device=dev))
+            for _ in range(2)]
+    r_dt = _RASTER_DT[x_dtype]
+    l_dt = _lib.DT_F32 if lab_d.dtype == torch.float32 else _lib.DT_U8
+
+    def gen():
+        epoch = gen.epoch
+        gen.epoch += 1
+        table, n_real = _epoch_table(deal, epoch, yx, share, aug_seed)
+        tab = torch.from_numpy(table).to(dev)
+        s = ops.stream_ptr()
+        for k, n in enumerate(n_real):
+            xb, yb = ring[k % 2]
+            t0 = tab.data_ptr() + k * 3 * B * 4
+            _lib.check(lib.b2u_crop_train_batch(img_d.data_ptr(), r_dt, C, Y, X, lab_d.data_ptr(), l_dt, t0, t0 + 4 * B,
+                                                t0 + 8 * B, B, P, xb.data_ptr(), yb.data_ptr(), s), "b2u_crop_train_batch")
+            yield xb, yb, n
+    gen.epoch = 0
+    gen.n_batches = deal.n_batches
+    return gen
 
 
 def augmented(batches: Callable[[], Iterable], share: float, seed: int = 0):
     """The geometric core of the reference's augmentation (utils.py:196-295 SegmentationAlbumentationsTransform applied to
     `ceil(B * n_transform_imgs)` images of every batch, image and mask together; the reference's default pipelines are
-    flips and 90-degree rotations): each selected sample gets one of the eight dihedral transforms.  Pure index
-    permutations of the raw integer tiles - no resampling, no value change - executed on the batch before it is copied to
-    the device; square tiles only (a 90-degree rotation must keep the shape)."""
-    if not (0.0 <= share <= 1.0):
-        raise ValueError(f"The n_transform_imgs parameter ({share}) must be between 1 and 0.")      # utils.py:236
+    flips and 90-degree rotations): each selected sample gets one of the eight dihedral transforms (`_aug_ops`).  Pure
+    index permutations of the raw integer tiles - no resampling, no value change - executed on the batch before it is
+    copied to the device; square tiles only (a 90-degree rotation must keep the shape)."""
+    share = _aug_share(share)
 
     def gen():
         rng = np.random.default_rng(seed + gen.epoch)
         gen.epoch += 1
         for x, y, n in batches():
-            B = x.shape[0]
-            k_aug = math.ceil(B * share)
-            if k_aug and x.shape[-1] == x.shape[-2]:
-                x, y = x.clone(), y.clone()
-                for i in rng.choice(B, size=k_aug, replace=False):
-                    op = int(rng.integers(0, 8))
-                    xi, yi = x[i], y[i]
-                    if op & 4:
-                        xi, yi = xi.flip(-1), yi.flip(-1)
-                    xi, yi = torch.rot90(xi, op & 3, (-2, -1)), torch.rot90(yi, op & 3, (-2, -1))
-                    x[i], y[i] = xi, yi
+            if x.shape[-1] == x.shape[-2]:
+                ops = _aug_ops(rng, x.shape[0], share)
+                if ops:
+                    # uint16 tiles are permuted as their int16 bits: torch has no CPU flip / rot90 for uint16
+                    dt = x.dtype
+                    x, y = (x.view(torch.int16) if dt == torch.uint16 else x).clone(), y.clone()
+                    for i, op in ops:
+                        xi, yi = x[i], y[i]
+                        if op & 4:
+                            xi, yi = xi.flip(-1), yi.flip(-1)
+                        xi, yi = torch.rot90(xi, op & 3, (-2, -1)), torch.rot90(yi, op & 3, (-2, -1))
+                        x[i], y[i] = xi, yi
+                    x = x.view(dt)
             yield x, y, n
     gen.epoch = 0
     gen.n_batches = getattr(batches, "n_batches", None)
     return gen
+
+
+def _aug_share(share) -> float:
+    share = float(share)
+    if not (0.0 <= share <= 1.0):
+        raise ValueError(f"The n_transform_imgs parameter ({share}) must be between 1 and 0.")      # utils.py:236
+    return share
+
+
+def _aug_ops(rng: np.random.Generator, B: int, share: float) -> List[Tuple[int, int]]:
+    """The random draws of one augmented batch, in the order they are made: `ceil(B * share)` distinct samples, then one
+    dihedral op in [0, 8) for each - bit 2 flips the last axis, then op & 3 quarter turns of torch.rot90(., k, (-2, -1))."""
+    k_aug = math.ceil(B * share)
+    if not k_aug:
+        return []
+    return [(int(i), int(rng.integers(0, 8))) for i in rng.choice(B, size=k_aug, replace=False)]
