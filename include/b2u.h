@@ -419,6 +419,17 @@ int b2u_stitch_finalize_mean(const float* acc, const uint8_t* cnt, int32_t C, in
 int b2u_softmax_nchw(const float* logits, int32_t ld, int32_t C, int64_t tiles, int32_t H, int32_t W, float* probs,
                      uint8_t* argmax, void* stream);
 
+/* ---- assessment: confusion counts of predicted class maps against truth maps (predict.py:56-143 validation_vision,
+ * sklearn.metrics.confusion_matrix / classification_report) -------------------------------------------------------
+ * T images of H x W uint8 class ids; pixel (t, y, x) of a map is at base + t * stride + y * pitch + x (the stride is
+ * unused when T == 1; pitch and base need no alignment, rows are read with 16-byte loads where both maps allow).
+ * Accumulates (device):  joint[truth * C + pred] += 1 (uint64 [C][C]) for pixels with both values < C, skipped += 1
+ * (uint64) for the others; tile_hist (nullable, uint32 [T][2][C]) += per image the truth histogram ([t][0]) and the
+ * prediction histogram ([t][1]) of the counted pixels.  1 <= C <= 32.  Integer counts: bit-identical on every run. */
+int b2u_confusion_counts(const uint8_t* pred, int64_t pred_pitch, int64_t pred_stride, const uint8_t* truth,
+                         int64_t truth_pitch, int64_t truth_stride, int32_t T, int32_t H, int32_t W, int32_t C,
+                         uint64_t* joint, uint32_t* tile_hist, uint64_t* skipped, void* stream);
+
 /* ---- SelfAttention (fastai layers.SelfAttention on UnetBlock.conv2 when self_attention=True, train.py:142) --------
  * The 1x1 query / key / value convolutions run through b2u_conv_*, the two batched attention products are plain
  * library GEMMs issued by the host layer; these entry points are the rest of the block. */

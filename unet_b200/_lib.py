@@ -177,6 +177,7 @@ def _declare(lib):
         "b2u_stitch_accumulate_raw": [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, u8p, i64, i64, i64, i64, vp],
         "b2u_stitch_finalize_mean": [vp, u8p, i32, i64, i64, f32, vp, vp],
         "b2u_softmax_nchw": [vp, i32, i32, i64, i32, i32, vp, u8p, vp],
+        "b2u_confusion_counts": [u8p, i64, i64, u8p, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp],
     }
     for name, args in sigs.items():
         fn = getattr(lib, name, None)

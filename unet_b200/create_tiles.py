@@ -95,24 +95,10 @@ def prepare_raster(path_to_raster, path_to_mask=None, patch_size: int = 400, pat
     mask = None
     if include_mask:
         mask, mgeo = read_geotiff(path_to_mask)
-        mask = mask.copy()
-        if class_zero:                                                   # :282-283 shift labels, keep no-data
-            sel = np.ones(mask.shape, bool) if mgeo.nodata is None else mask != mgeo.nodata
-            mask[sel] += 1
-        same_grid = (np.round(geo.geotransform[0], 3) == np.round(mgeo.geotransform[0], 3)
-                     and np.round(geo.geotransform[3], 3) == np.round(mgeo.geotransform[3], 3)
-                     and image.shape[1:] == mask.shape[1:])
-        if not same_grid:
-            raise ValueError("image and mask grids differ; re-aligning them (create_tiles_unet.py:287-352) is outside "
-                             "the built path - resample the mask onto the image grid first")
-        bad = np.zeros(image.shape[1:], bool)                             # :366-369
-        if nodata is not None:
-            bad |= (image == nodata).any(axis=0)
-        if mgeo.nodata is not None:
-            bad |= (mask == mgeo.nodata).any(axis=0)
+        check_same_grid(geo, mgeo, image.shape[1:], mask.shape[1:])
+        mask, bad = mask_labels(image, nodata, mask, mgeo.nodata, class_zero)
         image = image.copy()
         image[:, bad] = 0
-        mask[:, bad] = 0
     elif nodata is not None:
         image = image.copy()
         image[:, (image == nodata).any(axis=0)] = 0
@@ -130,6 +116,35 @@ def prepare_raster(path_to_raster, path_to_mask=None, patch_size: int = 400, pat
             continue
         tiles.append((f"{stem}_{index}.tif", (x, y, w, h)))
     return PreparedRaster(image, mask, geo, tiles)
+
+
+def check_same_grid(geo: GeoInfo, mgeo: GeoInfo, image_hw, mask_hw) -> None:
+    """The grid check of create_tiles_unet.py:287-352: the mask must share the raster's origin (to 3 decimals) and its
+    height and width; re-aligning them is refused with a ValueError."""
+    same_grid = (np.round(geo.geotransform[0], 3) == np.round(mgeo.geotransform[0], 3)
+                 and np.round(geo.geotransform[3], 3) == np.round(mgeo.geotransform[3], 3)
+                 and tuple(image_hw) == tuple(mask_hw))
+    if not same_grid:
+        raise ValueError("image and mask grids differ; re-aligning them (create_tiles_unet.py:287-352) is outside "
+                         "the built path - resample the mask onto the image grid first")
+
+
+def mask_labels(image: np.ndarray, nodata, mask: np.ndarray, mask_nodata, class_zero: bool):
+    """The label conversion of create_tiles_unet.py:282-283, 366-369 on a raster `[C, H, W]` and its mask `[bands, H, W]`
+    (whole or the same window of both): with `class_zero` every label that is not the mask's no-data value is shifted
+    by one, then pixels that are no-data in the image or in the mask are zeroed.  Returns (the converted mask, a copy;
+    the no-data pixels [H, W], which `prepare_raster` also zeroes in the image)."""
+    mask = mask.copy()
+    if class_zero:                                                       # :282-283 shift labels, keep no-data
+        sel = np.ones(mask.shape, bool) if mask_nodata is None else mask != mask_nodata
+        mask[sel] += 1
+    bad = np.zeros(image.shape[1:], bool)                                 # :366-369
+    if nodata is not None:
+        bad |= (image == nodata).any(axis=0)
+    if mask_nodata is not None:
+        bad |= (mask == mask_nodata).any(axis=0)
+    mask[:, bad] = 0
+    return mask, bad
 
 
 def split_raster(path_to_raster=None, path_to_mask=None, base_dir=".", patch_size: int = 400, patch_overlap: float = 0.20,

@@ -6,6 +6,9 @@
 // (train.py:218), softmax + numpy sum/count/argmax merge (predict.py:193-203, 284-334).
 #include <stdlib.h>
 
+#include <algorithm>
+#include <type_traits>
+
 #include "host_util.h"
 #include "ptx.cuh"
 #include "stream.cuh"
@@ -1229,6 +1232,134 @@ __global__ void softmax_nchw_kernel(const float* __restrict__ logits, int ld, in
   }
 }
 
+// Confusion counts of a predicted class map against a truth class map (sklearn.metrics.confusion_matrix orientation:
+// bin truth * C + pred).  Block (x, t) owns rows [x * rows, (x + 1) * rows) of image t and a warp one row at a time, so
+// a block's joint counts are also the histograms of its image.  Land-cover maps put almost every pixel into two or
+// three bins, which serialises per-pixel shared-memory atomics; so the counts of a block are privatised twice:
+//   C <= 4 (<= 16 bins): in registers, as 8-bit fields of two 64-bit words (one shift and one add per pixel), spilled
+//     to 32-bit register totals every <= 255 pixels and reduced over the warp with redux.sync at the end;
+//   C > 4: warp-aggregated shared-memory increments, one atomic per distinct bin of a warp (__match_any_sync + __popc).
+// Integer counts throughout: the result is the same bits for any grid and any schedule.
+struct RegBins {
+  unsigned long long lo = 0, hi = 0;   // bins 0..7 and 8..15, one byte each
+  unsigned tot[16] = {};
+  unsigned skip = 0;
+  int pend = 0;                        // pixels in the byte fields since the last spill (<= 255)
+  __device__ __forceinline__ void px(unsigned t, unsigned p, unsigned C) {
+    if (t < C && p < C) {
+      const unsigned b = t * C + p;
+      const unsigned long long s = 1ull << ((b & 7) << 3);
+      lo += b < 8 ? s : 0ull;
+      hi += b < 8 ? 0ull : s;
+    } else {
+      ++skip;
+    }
+  }
+  __device__ __forceinline__ void spill() {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      tot[k] += (unsigned)(lo >> (8 * k)) & 255u;
+      tot[8 + k] += (unsigned)(hi >> (8 * k)) & 255u;
+    }
+    lo = hi = 0;
+    pend = 0;
+  }
+  __device__ __forceinline__ void done(int n) {
+    pend += n;
+    if (pend > 255 - 16) spill();
+  }
+};
+
+struct SharedBins {
+  unsigned* bins;
+  unsigned skip = 0;
+  __device__ __forceinline__ void px(unsigned t, unsigned p, unsigned C) {
+    const unsigned key = (t < C && p < C) ? t * C + p : 0xffffu;
+    const unsigned peers = __match_any_sync(__activemask(), key);
+    if ((threadIdx.x & 31) == (unsigned)(__ffs(peers) - 1)) {
+      if (key != 0xffffu) atomicAdd(&bins[key], (unsigned)__popc(peers));
+      else skip += __popc(peers);
+    }
+  }
+  __device__ __forceinline__ void done(int) {}
+};
+
+template <class Bins>
+__device__ __forceinline__ void bins_add16(Bins& c, uint4 t, uint4 p, unsigned C) {
+  const unsigned tw[4] = {t.x, t.y, t.z, t.w}, pw[4] = {p.x, p.y, p.z, p.w};
+#pragma unroll
+  for (int w = 0; w < 4; ++w)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) c.px((tw[w] >> (8 * k)) & 255u, (pw[w] >> (8 * k)) & 255u, C);
+  c.done(16);
+}
+
+template <bool SMALL>
+__global__ void __launch_bounds__(256) confusion_counts_kernel(const uint8_t* __restrict__ pred, long long pp, long long ps,
+                                                               const uint8_t* __restrict__ truth, long long tp, long long ts,
+                                                               int H, int W, int C, int rows,
+                                                               unsigned long long* __restrict__ joint,
+                                                               unsigned* __restrict__ tile_hist,
+                                                               unsigned long long* __restrict__ skipped) {
+  __shared__ unsigned sj[32 * 32];
+  __shared__ unsigned sskip;
+  pdl_enter();
+  const int NB = C * C;
+  for (int i = threadIdx.x; i < NB; i += blockDim.x) sj[i] = 0u;
+  if (threadIdx.x == 0) sskip = 0u;
+  __syncthreads();
+  typename std::conditional<SMALL, RegBins, SharedBins>::type c;
+  if constexpr (!SMALL) c.bins = sj;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const int t = blockIdx.y;
+  const int y1 = min(H, (blockIdx.x + 1) * rows);
+  for (int y = blockIdx.x * rows + warp; y < y1; y += nw) {
+    const uint8_t* p = pred + t * ps + y * pp;
+    const uint8_t* q = truth + t * ts + y * tp;
+    // 16-byte loads from the first 16-byte boundary of the row when both rows sit at the same offset from it
+    int head = (int)((16 - (reinterpret_cast<uintptr_t>(p) & 15)) & 15);
+    if ((reinterpret_cast<uintptr_t>(p) ^ reinterpret_cast<uintptr_t>(q)) & 15) head = W;
+    head = min(head, W);
+    const int nv = (W - head) >> 4;
+    for (int x = lane; x < head; x += 32) { c.px(__ldg(q + x), __ldg(p + x), C); c.done(1); }
+    const uint4* pv = reinterpret_cast<const uint4*>(p + head);
+    const uint4* qv = reinterpret_cast<const uint4*>(q + head);
+    int v = lane;
+    for (; v + 96 < nv; v += 128) {     // four chunk pairs in flight per lane
+      uint4 a[4], b[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) { a[u] = __ldg(qv + v + 32 * u); b[u] = __ldg(pv + v + 32 * u); }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) bins_add16(c, a[u], b[u], C);
+    }
+    for (; v < nv; v += 32) bins_add16(c, __ldg(qv + v), __ldg(pv + v), C);
+    for (int x = head + 16 * nv + lane; x < W; x += 32) { c.px(__ldg(q + x), __ldg(p + x), C); c.done(1); }
+  }
+  if constexpr (SMALL) {
+    c.spill();
+#pragma unroll
+    for (int k = 0; k < 16; ++k) {
+      const unsigned s = __reduce_add_sync(0xffffffffu, c.tot[k]);
+      if (lane == 0 && k < NB && s) atomicAdd(&sj[k], s);
+    }
+  }
+  const unsigned sk = __reduce_add_sync(0xffffffffu, c.skip);
+  if (lane == 0 && sk) atomicAdd(&sskip, sk);
+  __syncthreads();
+  for (int i = threadIdx.x; i < NB; i += blockDim.x)
+    if (sj[i]) atomicAdd(&joint[i], (unsigned long long)sj[i]);
+  if (tile_hist) {
+    // [t][0][c]: truth histogram (row sums), [t][1][c]: prediction histogram (column sums)
+    for (int i = threadIdx.x; i < 2 * C; i += blockDim.x) {
+      const int k = i / C, cl = i - k * C;
+      unsigned s = 0;
+      for (int j = 0; j < C; ++j) s += k == 0 ? sj[cl * C + j] : sj[j * C + cl];
+      if (s) atomicAdd(&tile_hist[((long long)t * 2 + k) * C + cl], s);
+    }
+  }
+  if (threadIdx.x == 0 && sskip) atomicAdd(skipped, (unsigned long long)sskip);
+}
+
 }  // namespace b2u
 
 using namespace b2u;
@@ -1691,6 +1822,36 @@ extern "C" int b2u_softmax_nchw(const float* logits, int32_t ld, int32_t C, int6
     launch_k(softmax_nchw_kernel<8>, dim3(grid_for(items, 256)), dim3(256), 0, st, logits, ld, C, tiles, H, W, probs, argmax);
   else
     launch_k(softmax_nchw_kernel<32>, dim3(grid_for(items, 256)), dim3(256), 0, st, logits, ld, C, tiles, H, W, probs, argmax);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_confusion_counts(const uint8_t* pred, int64_t pred_pitch, int64_t pred_stride, const uint8_t* truth,
+                                    int64_t truth_pitch, int64_t truth_stride, int32_t T, int32_t H, int32_t W, int32_t C,
+                                    uint64_t* joint, uint32_t* tile_hist, uint64_t* skipped, void* stream) {
+  B2U_CHECK_ARG(pred && truth && joint && skipped, "confusion_counts: null argument");
+  B2U_CHECK_ARG(T >= 1 && T <= 65535 && H >= 1 && W >= 1 && C >= 1 && C <= 32,
+                "confusion_counts: T=%d H=%d W=%d C=%d out of range", T, H, W, C);
+  B2U_CHECK_ARG(pred_pitch >= W && truth_pitch >= W &&
+                (T == 1 || (pred_stride >= pred_pitch * (H - 1) + W && truth_stride >= truth_pitch * (H - 1) + W)),
+                "confusion_counts: pitches %lld / %lld or image strides %lld / %lld too small for %d x %d",
+                (long long)pred_pitch, (long long)truth_pitch, (long long)pred_stride, (long long)truth_stride, H, W);
+  B2U_CHECK_ARG(!tile_hist || (long long)H * W <= 0xffffffffll, "confusion_counts: %d x %d images overflow tile_hist", H, W);
+  // about eight blocks per SM over all images; rows per block a multiple of the 8 warps, and a block's counts stay below
+  // 2^31 so that its 32-bit shared counters cannot overflow
+  long long gx = std::max(1ll, ((long long)sm_count() * 8 + T - 1) / T);
+  long long rows = (H + gx - 1) / gx;
+  rows = std::min((rows + 7) / 8 * 8, std::max(1ll, ((1ll << 31) - 1) / W));
+  gx = (H + rows - 1) / rows;
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (C <= 4)
+    launch_k(confusion_counts_kernel<true>, dim3((unsigned)gx, T), dim3(256), 0, st, pred, (long long)pred_pitch,
+             (long long)pred_stride, truth, (long long)truth_pitch, (long long)truth_stride, H, W, C, (int)rows,
+             (unsigned long long*)joint, tile_hist, (unsigned long long*)skipped);
+  else
+    launch_k(confusion_counts_kernel<false>, dim3((unsigned)gx, T), dim3(256), 0, st, pred, (long long)pred_pitch,
+             (long long)pred_stride, truth, (long long)truth_pitch, (long long)truth_stride, H, W, C, (int)rows,
+             (unsigned long long*)joint, tile_hist, (unsigned long long*)skipped);
   B2U_LAUNCH_CHECK();
   return B2U_OK;
 }

@@ -33,6 +33,7 @@ import numpy as np
 import torch
 
 from . import _lib, ops
+from .assessment import ConfusionCounter, write_report
 from .engine import Trainer, one_cycle
 from .network import UNetB200, input_divisors
 from .predict_engine import TiledPredictor, gather_mask_strips
@@ -402,13 +403,15 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
     learn = predict_model if isinstance(predict_model, Learner) else load_learner(predict_model)
     if bool(regression) != learn.regression:
         raise ValueError(f"regression={regression} but the model was trained with regression={learn.regression}")
-    if validation_vision:
+    if validation_vision and regression:
         warnings.warn("validation_vision (confusion-matrix plots, predict.py:56-143) is outside the built path; skipped")
+    assess = bool(validation_vision) and not regression
     path = Path(predict_path)
     model_name = "model" if isinstance(predict_model, Learner) else os.path.basename(str(predict_model)).split(".")[0]
     tiles = sorted(path.glob("*.tif")) or sorted(path.glob("*.npy"))
     if not tiles:
         raise FileNotFoundError(f"no .tif / .npy tiles in {path}")
+    masks = {t: _mask_path(t) for t in tiles} if assess else {}
     rank, world = _rank(), _world()
     out_dir = path.parent if merge else path.parent / ("predicted_tiles_" + model_name)
     if rank == 0:
@@ -419,21 +422,32 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
     B, P = net.N, net.H
     dev, lib = net.device, net.lib
 
-    def batches(sel_tiles):
-        stage = None
+    def batches(sel_tiles, counted=None):
+        """(b0, tiles, georeferencing, staged tiles [B, n_in, P, P], staged labels [B, P, P], n_labels): with `counted`
+        (one flag per tile of `sel_tiles`) the labels of the flagged tiles of the batch fill the first n_labels slots"""
+        stage = ystage = None
         for b0 in range(0, len(sel_tiles), B):
             chunk = sel_tiles[b0:b0 + B]
             loaded = [_load_tile(t) for t in chunk]
             arr = np.stack([a for a, _ in loaded])
             if tuple(arr.shape[1:]) != (net.n_in, P, P):
                 raise ValueError(f"tiles must be [{net.n_in},{P},{P}], got {tuple(arr.shape[1:])}")
+            ys = [] if counted is None else [_load_labels(masks[t], net.n_out, P)
+                                             for t, k in zip(chunk, counted[b0:b0 + B]) if k]
             if stage is None or stage.dtype != torch.from_numpy(arr[:0]).dtype:
                 stage = torch.empty((B,) + arr.shape[1:], dtype=torch.from_numpy(arr[:0]).dtype).pin_memory()
-            torch.cuda.current_stream().synchronize()      # the previous batch's H2D copy has left the staging buffer
+            if counted is not None and ystage is None:
+                ystage = torch.empty((B, P, P), dtype=torch.uint8).pin_memory()
+            torch.cuda.current_stream().synchronize()      # the previous batch's H2D copies have left the staging buffers
             stage[:len(chunk)] = torch.from_numpy(arr)
             if len(chunk) < B:
                 stage[len(chunk):] = stage[:1]
-            yield b0, chunk, [g for _, g in loaded], stage
+            if ys:
+                ystage[:len(ys)] = torch.from_numpy(np.stack(ys))
+            yield b0, chunk, [g for _, g in loaded], stage, ystage, len(ys)
+
+    if assess:
+        y_dev = torch.empty((B, P, P), dtype=torch.uint8, device=dev)
 
     if merge:
         # ---- pass 1 over the headers: extent of the mosaic (predict.py:257-276)
@@ -461,11 +475,12 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
         y_len = round((gts[:, 3].min() + gts[ymin_r, 4] * gts[ymin_r, 5] - uly_full) / gts[0, 5])
         place = [placement_from_geotransform(g[0], P, g[2], g[3], P, g[5], ulx_full, uly_full) for g in gts]
         # owner-computes column strip of this rank (the whole mosaic on one GPU): every tile that intersects it
-        base_w, rem_w = divmod(x_len, world)
-        xb = rank * base_w + min(rank, rem_w)
-        xe = xb + base_w + (1 if rank < rem_w else 0)
-        mine = [i for i in range(len(tiles)) if place[i][0] < xe and place[i][0] + P > xb]
+        xb, xe, mine, own = _merge_strip(place, P, x_len, rank, world)
         SX = xe - xb
+        if assess:
+            counter = ConfusionCounter(net.n_out, dev, max(sum(_merge_strip(place, P, x_len, r, world)[3])
+                                                           for r in range(world)), rank, world)
+            amax_dev = torch.empty((B, P, P), dtype=torch.uint8, device=dev)
         acc = torch.zeros((net.n_out, y_len, SX), dtype=torch.float32, device=dev)
         cnt = torch.zeros((y_len, SX), dtype=torch.uint8, device=dev)
         accumulate = (lib.b2u_stitch_accumulate_raw if regression else
@@ -489,13 +504,25 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
         meta = torch.tensor(flat if flat else [0], dtype=torch.int32).to(dev)
         mbase = meta.data_ptr()
         s_ = ops.stream_ptr()
-        for (b0, chunk, _, x), (oy, ox, classes) in zip(batches([tiles[i] for i in mine]), plan):
+        for (b0, chunk, _, x, ys, ny), (oy, ox, classes) in zip(batches([tiles[i] for i in mine],
+                                                                         own if assess else None), plan):
             net.set_input(x.to(dev, non_blocking=True))
             net.forward()
             for osel, nsel in classes:
                 _lib.check(accumulate(net.logits.data_ptr(), net.logits.shape[-1], net.n_out, B, P, P, mbase + 4 * oy,
                                       mbase + 4 * ox, mbase + 4 * osel, nsel, acc.data_ptr(), cnt.data_ptr(), y_len, SX,
                                       0, xb, s_), "b2u_stitch_accumulate")
+            if ny:
+                # the per-tile argmax (what predict_tiles returns) of the tiles this rank owns, packed in batch order
+                k, ld = 0, net.logits.shape[-1]
+                for i0, i1 in _runs(own[b0:b0 + len(chunk)]):
+                    _lib.check(lib.b2u_softmax_nchw(net.logits.data_ptr() + 4 * i0 * P * P * ld, ld, net.n_out, i1 - i0,
+                                                    P, P, None, amax_dev.data_ptr() + k * P * P, s_), "b2u_softmax_nchw")
+                    k += i1 - i0
+                y_dev[:ny].copy_(ys[:ny], non_blocking=True)
+                counter.count(amax_dev[:ny], y_dev[:ny], per_tile=True)
+        if assess:
+            _write_validation(counter, world, rank, out_dir, AOI, year, model_name, class_zero)
         nodata = None
         if regression:
             outd = torch.empty((1, y_len, SX), dtype=torch.float32, device=dev)
@@ -536,12 +563,18 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
         return _store(out_dir / (name + ".tif"), out, geo, nodata, class_zero)
 
     outs = []
-    for b0, chunk, geos, x in batches(tiles[rank::world]):
+    sel = tiles[rank::world]
+    if assess:
+        counter = ConfusionCounter(net.n_out, dev, -(-len(tiles) // world), rank, world)
+    for b0, chunk, geos, x, ys, ny in batches(sel, [True] * len(sel) if assess else None):
         xd = x.to(dev, non_blocking=True)
         if regression:
             vals = pred.predict_tiles_raw(xd).cpu().numpy()
         else:
             probs, amax = pred.predict_tiles(xd)
+            if assess:                                          # the real tiles of a padded last batch
+                y_dev[:ny].copy_(ys[:ny], non_blocking=True)
+                counter.count(amax[:ny], y_dev[:ny], per_tile=True)
             probs, amax = probs.cpu().numpy(), amax.cpu().numpy()
         for i, t in enumerate(chunk):
             if regression:
@@ -555,11 +588,67 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
             if large_file and not regression and (all_classes or specific_class):   # predict.py:245-249 (sic: class 0 is falsy there)
                 arr = np.around(arr * ((128 / 4) - 1)).astype(np.int8)
             outs.append(_store(out_dir / t.name, arr, geos[i], None, class_zero))
+    if assess:
+        _write_validation(counter, world, rank, out_dir, AOI, year, model_name, class_zero)
     return outs
 
 
+def _mask_path(tile: Path) -> Path:
+    """`open_mask`'s rule (utils.py:51-55): the mask tile of an image tile is the file of the same name with `img_tiles`
+    replaced by `mask_tiles` in its path (a `.npy` tile has a `.npy` mask)"""
+    m = Path(str(tile).replace("img_tiles", "mask_tiles"))
+    if m == tile:
+        raise FileNotFoundError(f"{tile}: validation_vision needs the tiles in an img_tiles folder with a mask_tiles sibling")
+    if not m.exists():
+        raise FileNotFoundError(f"mask tile {m} of {tile} is missing")
+    return m
+
+
+def _load_labels(path: Path, n_classes: int, P: int) -> np.ndarray:
+    """band 1 of a mask tile as uint8 class ids below `n_classes` (the labels training reads, `_label_values`)"""
+    y = read_geotiff(path)[0] if path.suffix.lower() in (".tif", ".tiff") else np.load(path)
+    y = y[0] if y.ndim == 3 else y
+    if y.shape != (P, P):
+        raise ValueError(f"{path}: mask tile of shape {y.shape}, expected ({P}, {P})")
+    return _label_values(y, n_classes, False, path)
+
+
+def _merge_strip(place, P: int, x_len: int, rank: int, world: int):
+    """The owner-computes column strip [xb, xe) of `rank` in a mosaic `x_len` wide, the indices of the tiles at
+    `place` [(x, y, ...)] that intersect it (`mine`: the tiles the rank predicts) and, per tile of `mine`, whether the
+    rank owns it (its left edge column lies in the strip): every tile has exactly one owner, which assesses it."""
+    base_w, rem_w = divmod(x_len, world)
+    xb = rank * base_w + min(rank, rem_w)
+    xe = xb + base_w + (1 if rank < rem_w else 0)
+    mine = [i for i in range(len(place)) if place[i][0] < xe and place[i][0] + P > xb]
+    return xb, xe, mine, [xb <= place[i][0] < xe for i in mine]
+
+
+def _runs(flags: Sequence[bool]) -> List[Tuple[int, int]]:
+    """[i0, i1) ranges of consecutive True flags"""
+    out, i0 = [], None
+    for i, f in enumerate(list(flags) + [False]):
+        if f and i0 is None:
+            i0 = i
+        elif not f and i0 is not None:
+            out.append((i0, i))
+            i0 = None
+    return out
+
+
+def _write_validation(counter: ConfusionCounter, world: int, rank: int, out_dir: Path, AOI, year, model_name: str,
+                      class_zero: bool) -> None:
+    """the counts of all ranks summed; rank 0 writes `<AOI>_<year>_<model>_validation{.json,_confusion.csv,
+    _tile_confusion.csv}`"""
+    cm, skipped, hist = counter.read(all_reduce=world > 1)
+    if rank == 0:
+        name = "_".join([str(p_) for p_ in (AOI, year, model_name, "validation") if p_])
+        write_report(out_dir, name, cm, skipped, hist, class_zero)
+
+
 def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: float = 0.125, large_file: bool = False,
-                    class_zero: bool = False, rank: int = 0, world: int = 1, max_strip_columns: Optional[int] = None):
+                    class_zero: bool = False, rank: int = 0, world: int = 1, max_strip_columns: Optional[int] = None,
+                    mask_path=None):
     """Tile-free variant of the predict path: what `split_raster` (create_tiles_unet.py:252-431) + `save_predictions(merge=
     True)` produce together - the stitched argmax mask of a whole multi-band GeoTIFF (uint8 / uint16 / int16 bands) -
     without writing tiles to disk: the raster is windowed on the device with `compute_windows` offsets, predicted and
@@ -568,7 +657,13 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
     at most that many output columns - each strip reads only the file window of the tile columns it needs
     (`read_geotiff(window=)`), is predicted as an owner-computes strip and lands in its columns of the mask, so the
     result is bit-identical to the one-shot prediction.  With `world > 1` every rank writes the column strip it owns
-    (`<out>.part<rank>.tif`, georeferenced to its origin)."""
+    (`<out>.part<rank>.tif`, georeferenced to its origin).
+    `mask_path`: a reference mask on the raster's grid.  Each strip's stitched mask is then compared, on the device, with
+    the labels `prepare_raster` makes of the mask (class_zero shift, no-data of image or mask -> 0; a label >= the number
+    of classes raises ValueError) over the columns the strip owns, and the accuracy report of the rank's columns goes next
+    to the mask as `<out stem>_assessment{.json,_confusion.csv}` (`assessment.write_report`).  The written mask and the
+    return value do not change."""
+    from .create_tiles import check_same_grid, mask_labels, mask_tile_values
     learn = predict_model if isinstance(predict_model, Learner) else load_learner(predict_model)
     if learn.regression:
         raise ValueError("predict_geotiff writes class masks; use save_predictions(regression=True, merge=True) over tiles")
@@ -584,6 +679,11 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
     _, xb, xe = shard_windows_by_columns(windows, X, rank, world)
     n_strips = 1 if not max_strip_columns else max(1, -(-(xe - xb) // int(max_strip_columns)))
     mask = np.empty((Y, xe - xb), dtype=np.uint8)
+    counter = None
+    if mask_path is not None:
+        _, mY, mX, _, mgeo = geotiff_info(mask_path)
+        check_same_grid(geo, mgeo, (Y, X), (mY, mX))
+        counter = ConfusionCounter(net.n_out, net.device)
     for k in range(n_strips):
         # strip k of this rank's columns: the balanced partition of [xb, xe), then the tile columns intersecting it
         base, rem = divmod(xe - xb, n_strips)
@@ -596,11 +696,23 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
         dev_s = torch.from_numpy(np.ascontiguousarray(strip)).pin_memory().to(net.device, non_blocking=True)
         # the strip holds exactly the tile columns of [sb, se): a one-rank prediction of it reproduces those tiles
         m, _, _ = pred.predict_raster(dev_s, patch_overlap, 0, 1, large_file=large_file)
+        if counter is not None:
+            # the truth of the same window, laid out like `m` so that both rows sit at the same 16-byte offset
+            truth, _ = read_geotiff(mask_path, window=(xs0, 0, xs1 - xs0, Y))
+            truth, _ = mask_labels(strip, geo.nodata, truth, mgeo.nodata, class_zero)
+            truth = _label_values(mask_tile_values(truth[0]), net.n_out, False, mask_path)
+            truth_d = torch.from_numpy(np.ascontiguousarray(truth)).pin_memory().to(net.device, non_blocking=True)
+            counter.count(m[:, sb - xs0:se - xs0], truth_d[:, sb - xs0:se - xs0])
         mask[:, sb - xb:se - xb] = m[:, sb - xs0:se - xs0].cpu().numpy()
     out_path = Path(out_path) if out_path is not None else Path(raster_path).with_name(Path(raster_path).stem + "_prediction.tif")
     if world > 1:
         out_path = out_path.with_suffix(f".part{rank}.tif")
     write_geotiff(out_path, mask, geo.window(xb, 0), nodata=None, class_zero=class_zero)
+    if counter is not None:
+        cm, skipped, _ = counter.read()
+        write_report(Path(mask_path).parent, out_path.stem + "_assessment", cm, skipped, None, class_zero,
+                     extra={"raster": str(raster_path), "mask": str(mask_path), "prediction": str(out_path),
+                            "columns": [xb, xe]})
     return out_path
 
 
