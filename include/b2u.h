@@ -383,36 +383,23 @@ int b2u_adam_step(float* p, const float* g, float* m, float* v, int64_t n, const
 
 /* ---- prediction: softmax + overlap-tile accumulate, normalise + argmax (predict.py:284-334) ------------------- */
 /* logits fp32 [T][th][tw][ld]; tile t sits at (y0[t], x0[t]) of the full raster; acc fp32 [C][Y][X] and cnt uint8
- * [Y][X] cover the raster window starting at (y_off, x_off).  `sel` (nullable, n_sel entries) lists the tiles of this
- * launch; tiles within one launch must not overlap each other (the host colours the overlap graph), which makes the
- * sums independent of scheduling without atomics. */
+ * [Y][X] cover the raster window starting at (y_off, x_off).  The launch adds the first min(*n_sel_dev, max_sel)
+ * tiles listed in `sel` (0 < max_sel <= T); the count lives on the device, so the host can refill a batch's tile
+ * origins and class lists with one device copy instead of waiting for them.  Tiles within one launch must not overlap
+ * each other (the host colours the overlap graph), which makes the sums independent of scheduling without atomics.
+ * mode 0: softmax probabilities are added.  mode 1: the `large_file` merge (predict.py:217-219): every probability is
+ * quantised to np.around(p * 31) (int8 in the reference; the sums <= 4*31 are exact in the fp32 accumulator).
+ * mode 2: the regression merge (predict.py:196-198, 300-302): the raw network output is added, no softmax. */
 int b2u_stitch_accumulate(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                          const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel, float* acc,
-                          uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off, void* stream);
-/* mask[y][x] = argmax_c acc[c][y][x]/cnt (first max wins like np.argmax, unplaced pixels -> 0), uint8 */
-int b2u_stitch_finalize(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, uint8_t* mask,
-                        void* stream);
-/* `large_file` mode of the merge (predict.py:217-219, 318-323): every tile's probabilities are quantised to
- * np.around(p * 31) (int8 in the reference; the sums <= 4*31 are exact in the fp32 accumulator), the sums are
- * floor-divided by the count and arg-maxed.  Same arguments as the two entry points above. */
-int b2u_stitch_accumulate_q31(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                              const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel, float* acc,
-                              uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off, void* stream);
-int b2u_stitch_finalize_q31(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, uint8_t* mask,
-                            void* stream);
-/* the same accumulate with the selection count on the device (`*n_sel_dev` <= max_sel tiles of `sel` are processed), so
- * that a whole batch - crop, forward, accumulate of each colour class - replays as ONE captured CUDA graph while the
- * per-batch tile origins / class lists are swapped underneath it.  mode: 0 softmax, 1 `large_file` (x31), 2 raw. */
-int b2u_stitch_accumulate_dev(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                              const int32_t* y0, const int32_t* x0, const int32_t* sel, const int32_t* n_sel_dev,
-                              int32_t max_sel, int32_t mode, float* acc, uint8_t* cnt, int64_t Y, int64_t X,
-                              int64_t y_off, int64_t x_off, void* stream);
-/* regression merge (predict.py:196-198, 300-316): the raw network output is summed (no softmax) ... */
-int b2u_stitch_accumulate_raw(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                              const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel, float* acc,
-                              uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off, void* stream);
-/* ... and out[c][y][x] = acc/cnt where tiles were placed, `nodata` elsewhere (regression: -9999, predict.py:313-316;
- * also the averaged probabilities of the `all_classes` / `specific_class` merge, predict.py:326-337, nodata 0) */
+                          const int32_t* y0, const int32_t* x0, const int32_t* sel, const int32_t* n_sel_dev,
+                          int32_t max_sel, int32_t mode, float* acc, uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off,
+                          int64_t x_off, void* stream);
+/* mask[y][x] = argmax_c acc[c][y][x]/cnt (first max wins like np.argmax, unplaced pixels -> 0), uint8.  int_div != 0:
+ * the quotients are floored first, as the `large_file` merge floor-divides its int8 sums (predict.py:318-323). */
+int b2u_stitch_finalize(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, int32_t int_div,
+                        uint8_t* mask, void* stream);
+/* out[c][y][x] = acc/cnt where tiles were placed, `nodata` elsewhere (regression: -9999, predict.py:313-316; also the
+ * averaged probabilities of the `all_classes` / `specific_class` merge, predict.py:326-337, nodata 0) */
 int b2u_stitch_finalize_mean(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, float nodata,
                              float* out, void* stream);
 /* per-tile softmax probabilities (fp32 NCHW, what learn.predict returns, predict.py:193-203) and argmax */

@@ -1,6 +1,6 @@
 """The accuracy report of `validation_vision` / `predict_geotiff(mask_path=)` without a GPU: the metrics of
 `unet_b200.assessment` against scikit-learn, the report files, the per-tile majority rule, the label conversion shared
-with `prepare_raster`, the merge-mode tile ownership and the mask-tile lookup."""
+with `prepare_raster` and the mask-tile lookup."""
 import json
 import math
 import warnings
@@ -119,24 +119,6 @@ def test_mask_labels_reproduce_prepare_raster_on_windows(tmp_path, class_zero):
         lab, bad = mask_labels(img[:, :, x0:x0 + w], 0, msk[:, :, x0:x0 + w], 255, class_zero)
         assert np.array_equal(mask_tile_values(lab[0]), ref[:, x0:x0 + w]), (x0, w)
     assert ref[45, 65] == 0 and ref[6, 12] == 0
-
-
-@pytest.mark.parametrize("world", range(1, 9))
-def test_merge_tiles_have_exactly_one_owner(world):
-    from unet_b200.reference_api import _merge_strip
-    rng = np.random.default_rng(world)
-    P = 16
-    for _ in range(5):
-        n = int(rng.integers(1, 60))
-        place = [(int(rng.integers(0, 200)), int(rng.integers(0, 50)), P, P) for _ in range(n)]
-        x_len = max(x for x, *_ in place) + P
-        owners = [[] for _ in range(n)]
-        for r in range(world):
-            xb, xe, mine, own = _merge_strip(place, P, x_len, r, world)
-            for i, o in zip(mine, own):
-                if o:
-                    owners[i].append(r)
-        assert all(len(o) == 1 for o in owners)
 
 
 def test_missing_mask_tile_raises(tmp_path):

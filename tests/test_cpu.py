@@ -73,6 +73,26 @@ def test_coverage_counts_and_colour_classes():
             assert xs[0][0] == 0 and xs[-1][1] == w and all(xs[i][1] == xs[i + 1][0] for i in range(world - 1))
 
 
+@pytest.mark.parametrize("world", range(1, 9))
+def test_column_owned_gives_every_tile_one_owner(world):
+    """tiling.column_owned over the strips of shard_windows_by_columns (the merge of save_predictions): every tile of
+    randomly placed mosaics is owned by exactly one rank, which counts it in a validation_vision assessment."""
+    from unet_b200.tiling import column_owned, shard_windows_by_columns
+    rng = np.random.default_rng(world)
+    P = 16
+    for _ in range(5):
+        n = int(rng.integers(1, 60))
+        place = [(int(rng.integers(0, 200)), int(rng.integers(0, 50)), P, P) for _ in range(n)]
+        x_len = max(x for x, *_ in place) + P
+        owners = [[] for _ in range(n)]
+        for r in range(world):
+            mine, xb, xe = shard_windows_by_columns(place, x_len, r, world)
+            for i, o in zip(mine, column_owned(place, mine, xb, xe)):
+                if o:
+                    owners[i].append(r)
+        assert all(len(o) == 1 for o in owners)
+
+
 # ------------------------------------------------------------------------------------------------ stitch oracle
 def test_stitch_oracle_matches_golden():
     from oracle import stitch

@@ -393,9 +393,10 @@ def test_dice_counts(C):
     assert abs(sum(dice) / len(dice) - dice_multi(pred, labels.long(), C)) <= 1e-12
 
 
-def test_regression_stitch():
-    """regression merge (predict.py:300-316): raw predictions summed, divided by the count, -9999 where no tile was
-    placed - against the numpy restatement of the reference's merge."""
+def test_regression_stitch_mode2():
+    """regression merge (predict.py:300-316) through `b2u_stitch_accumulate` mode 2 with the tile count on the device:
+    raw predictions summed, divided by the count, -9999 where no tile was placed - against the numpy restatement of
+    the reference's merge."""
     from oracle.stitch import merge_pixel_windows_regression
     L, _lib = lib()
     T, P_, ld, Y, X = 6, 16, 8, 40, 52
@@ -409,8 +410,9 @@ def test_regression_stitch():
     cnt = torch.zeros((Y, X), dtype=torch.uint8, device="cuda")
     for cls in colour_classes(wins):
         sel = torch.tensor(cls, dtype=torch.int32, device="cuda")
-        _lib.check(L.b2u_stitch_accumulate_raw(p(z), ld, 1, T, P_, P_, p(y0), p(x0), p(sel), len(cls), p(acc), p(cnt),
-                                               Y, X, 0, 0, S()))
+        n_sel = torch.tensor([len(cls)], dtype=torch.int32, device="cuda")
+        _lib.check(L.b2u_stitch_accumulate(p(z), ld, 1, T, P_, P_, p(y0), p(x0), p(sel), p(n_sel), len(cls), 2, p(acc),
+                                           p(cnt), Y, X, 0, 0, S()))
     out = torch.zeros((1, Y, X), device="cuda")
     _lib.check(L.b2u_stitch_finalize_mean(p(acc), p(cnt), 1, Y, X, -9999.0, p(out), S()))
     torch.cuda.synchronize()
@@ -451,8 +453,9 @@ def test_stage_weights(Cout, Cin, ks):
 
 
 @pytest.mark.parametrize("H,W,P,ov,Cc", [(300, 420, 64, 0.125, 2), (257, 511, 128, 0.5, 3)])
-def test_stitch_against_numpy_merge(H, W, P, ov, Cc):
-    """softmax + overlap accumulate + normalise + argmax vs the numpy restatement of predict.py:284-337."""
+def test_stitch_mode0_against_numpy_merge(H, W, P, ov, Cc):
+    """softmax + overlap accumulate (`b2u_stitch_accumulate` mode 0, tile count on the device) + normalise + argmax vs
+    the numpy restatement of predict.py:284-337."""
     from oracle.stitch import merge_pixel_windows, softmax_probs
     from unet_b200.tiling import colour_classes, compute_windows
     L, _lib = lib()
@@ -469,9 +472,10 @@ def test_stitch_against_numpy_merge(H, W, P, ov, Cc):
     x0 = torch.tensor([w[0] for w in wins], dtype=torch.int32, device="cuda")
     for cls in colour_classes(wins):
         sel = torch.tensor(cls, dtype=torch.int32, device="cuda")
-        _lib.check(L.b2u_stitch_accumulate(p(logits), 8, Cc, T, P, P, p(y0), p(x0), p(sel), len(cls), p(acc), p(cnt),
-                                           H, W, 0, 0, S()))
-    _lib.check(L.b2u_stitch_finalize(p(acc), p(cnt), Cc, H, W, p(mask), S()))
+        n_sel = torch.tensor([len(cls)], dtype=torch.int32, device="cuda")
+        _lib.check(L.b2u_stitch_accumulate(p(logits), 8, Cc, T, P, P, p(y0), p(x0), p(sel), p(n_sel), len(cls), 0,
+                                           p(acc), p(cnt), H, W, 0, 0, S()))
+    _lib.check(L.b2u_stitch_finalize(p(acc), p(cnt), Cc, H, W, 0, p(mask), S()))
     torch.cuda.synchronize()
     # coverage counts are integers: exact;  the class mask agrees except where two class means tie within fp32 rounding
     cov = np.zeros((H, W), np.int64)

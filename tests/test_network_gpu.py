@@ -301,15 +301,16 @@ def test_eval_forward_and_tile_prediction():
 def test_predict_raster_matches_reference_merge():
     """Tiled predict-and-stitch of a small raster: GPU mask vs the numpy merge (predict.py:284-337 restated) fed with
     the oracle's per-tile softmax probabilities; also checks that a 2-way column sharding reproduces the 1-GPU mask
-    bit-exactly (owner-computes strips)."""
+    bit-exactly (owner-computes strips).  At overlap 0.75 a tile overlaps three neighbours per axis: batches then need
+    more than 2 x 2 colour classes."""
     import numpy as np
     from oracle.stitch import merge_pixel_windows
     from oracle.unet_oracle import make_oracle
     from unet_b200.network import UNetB200
     from unet_b200.predict_engine import TiledPredictor
-    from unet_b200.tiling import compute_windows
+    from unet_b200.tiling import colour_classes, compute_windows
     torch.backends.cudnn.allow_tf32 = False
-    P, ov, H, W = 64, 0.125, 200, 264
+    P, H, W = 64, 200, 264
     oracle = make_oracle("xresnet18", 4, 2).cuda().eval()
     net = UNetB200("xresnet18", 4, 2, (P, P), 8, training=False)
     net.load_state_dict(oracle.state_dict())
@@ -318,28 +319,31 @@ def test_predict_raster_matches_reference_merge():
     raster = (torch.nn.functional.interpolate(low[None], size=(H, W), mode="bilinear")[0] * 255).round().to(torch.uint8)
     raster = raster.cuda().contiguous()
     pred = TiledPredictor(net)
-    mask, xb, xe = pred.predict_raster(raster, ov)
-    torch.cuda.synchronize()
-    wins = compute_windows(H, W, P, ov)
-    probs = []
-    with torch.no_grad():
-        for (x, y, w, h) in wins:
-            t = raster[:, y:y + h, x:x + w][None].float() / 255.0
-            probs.append(oracle(t).softmax(1)[0].cpu().numpy())
-    ref = merge_pixel_windows(probs, wins, H, W)
-    agree = (mask.cpu().numpy() == ref).mean()
-    assert agree >= 0.995, agree      # random-init logits are near-ties almost everywhere; see test docstring above
-    # sharded == single GPU, bit-exact
-    parts = []
-    for r in range(2):
-        m, b, e = pred.predict_raster(raster, ov, rank=r, world=2)
-        parts.append(m)
-    torch.cuda.synchronize()
-    assert torch.equal(torch.cat(parts, dim=1), mask)
-    # 2 x 2 ownership grid (what 8 GPUs use as 4 x 2): every cell equals the same window of the 1-GPU mask
-    for r in range(4):
-        m, (xb, xe, yb, ye) = pred.predict_raster(raster, ov, rank=r, world=4, grid=(2, 2))
-        assert torch.equal(m, mask[yb:ye, xb:xe])
+    for ov in (0.125, 0.75):
+        mask, xb, xe = pred.predict_raster(raster, ov)
+        torch.cuda.synchronize()
+        wins = compute_windows(H, W, P, ov)
+        if ov > 0.5:
+            assert max(len(colour_classes(wins[b:b + 8])) for b in range(0, len(wins), 8)) > 4
+        probs = []
+        with torch.no_grad():
+            for (x, y, w, h) in wins:
+                t = raster[:, y:y + h, x:x + w][None].float() / 255.0
+                probs.append(oracle(t).softmax(1)[0].cpu().numpy())
+        ref = merge_pixel_windows(probs, wins, H, W)
+        agree = (mask.cpu().numpy() == ref).mean()
+        assert agree >= 0.995, (ov, agree)  # random-init logits are near-ties almost everywhere; see test docstring above
+        # sharded == single GPU, bit-exact
+        parts = []
+        for r in range(2):
+            m, b, e = pred.predict_raster(raster, ov, rank=r, world=2)
+            parts.append(m)
+        torch.cuda.synchronize()
+        assert torch.equal(torch.cat(parts, dim=1), mask)
+        # 2 x 2 ownership grid (what 8 GPUs use as 4 x 2): every cell equals the same window of the 1-GPU mask
+        for r in range(4):
+            m, (xb, xe, yb, ye) = pred.predict_raster(raster, ov, rank=r, world=4, grid=(2, 2))
+            assert torch.equal(m, mask[yb:ye, xb:xe])
 
 
 def test_against_committed_golden_fixture():

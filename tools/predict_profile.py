@@ -35,7 +35,7 @@ timed("forward (eager)", lambda: net.forward(s))
 acc = torch.zeros((2, side, side), device="cuda"); cnt = torch.zeros((side, side), dtype=torch.uint8, device="cuda")
 sel = torch.arange(B, dtype=torch.int32, device="cuda"); nsel = torch.tensor([B // 4], dtype=torch.int32, device="cuda")
 yy = (torch.arange(B, dtype=torch.int32, device="cuda") // 8) * 256; xx = (torch.arange(B, dtype=torch.int32, device="cuda") % 8) * 256
-timed("stitch_accumulate x4 classes", lambda: [_lib.check(lib.b2u_stitch_accumulate_dev(net.logits.data_ptr(), net.logits.shape[-1], 2, B, 256, 256, yy.data_ptr(), xx.data_ptr(), sel.data_ptr(), nsel.data_ptr(), B, 0, acc.data_ptr(), cnt.data_ptr(), side, side, 0, 0, s)) for _ in range(4)])
+timed("stitch_accumulate x4 classes", lambda: [_lib.check(lib.b2u_stitch_accumulate(net.logits.data_ptr(), net.logits.shape[-1], 2, B, 256, 256, yy.data_ptr(), xx.data_ptr(), sel.data_ptr(), nsel.data_ptr(), B, 0, acc.data_ptr(), cnt.data_ptr(), side, side, 0, 0, s)) for _ in range(4)])
 mask = torch.empty((side, side), dtype=torch.uint8, device="cuda")
-timed("stitch_finalize", lambda: _lib.check(lib.b2u_stitch_finalize(acc.data_ptr(), cnt.data_ptr(), 2, side, side, mask.data_ptr(), s)))
+timed("stitch_finalize", lambda: _lib.check(lib.b2u_stitch_finalize(acc.data_ptr(), cnt.data_ptr(), 2, side, side, 0, mask.data_ptr(), s)))
 timed("zero acc+cnt", lambda: (acc.zero_(), cnt.zero_()))

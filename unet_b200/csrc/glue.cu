@@ -1114,27 +1114,26 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 // ------------------------------------------------------------------------------------------------ stitching
 // softmax of tile logits added into the raster accumulators; one launch handles tiles that do not overlap each other.
 template <int MAXC>
-__global__ void stitch_accumulate_kernel(const float* __restrict__ logits, int ld, int C, int T, int th, int tw,
+__global__ void stitch_accumulate_kernel(const float* __restrict__ logits, int ld, int C, int th, int tw,
                                          const int* __restrict__ ty0, const int* __restrict__ tx0,
-                                         const int* __restrict__ sel, int n_sel, float* __restrict__ acc,
-                                         uint8_t* __restrict__ cnt, long long Y, long long X, long long y_off,
-                                         long long x_off, float quant, int raw, const int* __restrict__ n_sel_dev) {
+                                         const int* __restrict__ sel, const int* __restrict__ n_sel_dev, int max_sel,
+                                         int mode, float* __restrict__ acc, uint8_t* __restrict__ cnt, long long Y,
+                                         long long X, long long y_off, long long x_off) {
   pdl_enter();
   const long long per_tile = (long long)th * tw;
-  // n_sel_dev: the number of selected tiles lives on the device (launches captured in a CUDA graph: the host value
-  // n_sel is then only the upper bound the grid was sized for)
-  const int nt = sel ? (n_sel_dev ? min(*n_sel_dev, n_sel) : n_sel) : T;
+  // the number of selected tiles lives on the device; max_sel is the upper bound the grid was sized for
+  const int nt = min(*n_sel_dev, max_sel);
   const long long total = (long long)nt * per_tile;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int k = (int)(i / per_tile);
-    const int t = sel ? sel[k] : k;
+    const int t = sel[k];
     const long long r = i - (long long)k * per_tile;
     const int yy = (int)(r / tw), xx = (int)(r - (long long)yy * tw);
     const long long gy = (long long)ty0[t] + yy - y_off, gx = (long long)tx0[t] + xx - x_off;
     if (gy < 0 || gy >= Y || gx < 0 || gx >= X) continue;
     const float* z = logits + ((long long)t * per_tile + r) * ld;
     const long long o = gy * X + gx;
-    if (raw) {
+    if (mode == 2) {
       // regression merge (predict.py:196-198, 300-302): the network output itself is summed, no softmax
       for (int c = 0; c < C; ++c) acc[(long long)c * Y * X + o] += z[c];
       cnt[o] += 1;
@@ -1157,9 +1156,9 @@ __global__ void stitch_accumulate_kernel(const float* __restrict__ logits, int l
 #pragma unroll
     for (int c = 0; c < MAXC; ++c)
       if (c < C) {
-        // quant > 0: the reference's `large_file` mode (predict.py:217-219): prob * 31 -> np.around (half to even) -> int8
+        // mode 1: the reference's `large_file` mode (predict.py:217-219): prob * 31 -> np.around (half to even) -> int8
         const float pr = e[c] * inv;
-        acc[(long long)c * Y * X + o] += quant > 0.f ? rintf(pr * quant) : pr;
+        acc[(long long)c * Y * X + o] += mode == 1 ? rintf(pr * 31.f) : pr;
       }
     cnt[o] += 1;
   }
@@ -1738,47 +1737,22 @@ extern "C" int b2u_adam_step(float* p, const float* g, float* m, float* v, int64
   return B2U_OK;
 }
 
-static int stitch_accumulate_impl(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                                  const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel, float* acc,
-                                  uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off, float quant,
-                                  int raw, void* stream, const int32_t* n_sel_dev = nullptr) {
-  B2U_CHECK_ARG(logits && y0 && x0 && acc && cnt && C >= 1 && C <= 32 && C <= ld, "stitch_accumulate: bad argument");
-  const int nt = sel ? n_sel : T;
-  if (nt <= 0) return B2U_OK;
-  const long long items = (long long)nt * th * tw;
+extern "C" int b2u_stitch_accumulate(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
+                                     const int32_t* y0, const int32_t* x0, const int32_t* sel, const int32_t* n_sel_dev,
+                                     int32_t max_sel, int32_t mode, float* acc, uint8_t* cnt, int64_t Y, int64_t X,
+                                     int64_t y_off, int64_t x_off, void* stream) {
+  B2U_CHECK_ARG(logits && y0 && x0 && sel && n_sel_dev && acc && cnt && C >= 1 && C <= 32 && C <= ld && max_sel > 0 &&
+                max_sel <= T && mode >= 0 && mode <= 2, "stitch_accumulate: bad argument");
+  const long long items = (long long)max_sel * th * tw;
   cudaStream_t st = (cudaStream_t)stream;
   if (C <= 8)
-    launch_k(stitch_accumulate_kernel<8>, dim3(grid_for(items, 256)), dim3(256), 0, st, logits, ld, C, T, th, tw, y0, x0,
-             sel, n_sel, acc, cnt, Y, X, y_off, x_off, quant, raw, n_sel_dev);
+    launch_k(stitch_accumulate_kernel<8>, dim3(grid_for(items, 256)), dim3(256), 0, st, logits, ld, C, th, tw, y0, x0,
+             sel, n_sel_dev, max_sel, mode, acc, cnt, Y, X, y_off, x_off);
   else
-    launch_k(stitch_accumulate_kernel<32>, dim3(grid_for(items, 256)), dim3(256), 0, st, logits, ld, C, T, th, tw, y0, x0,
-             sel, n_sel, acc, cnt, Y, X, y_off, x_off, quant, raw, n_sel_dev);
+    launch_k(stitch_accumulate_kernel<32>, dim3(grid_for(items, 256)), dim3(256), 0, st, logits, ld, C, th, tw, y0, x0,
+             sel, n_sel_dev, max_sel, mode, acc, cnt, Y, X, y_off, x_off);
   B2U_LAUNCH_CHECK();
   return B2U_OK;
-}
-
-extern "C" int b2u_stitch_accumulate(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                                     const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel,
-                                     float* acc, uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off,
-                                     void* stream) {
-  return stitch_accumulate_impl(logits, ld, C, T, th, tw, y0, x0, sel, n_sel, acc, cnt, Y, X, y_off, x_off, 0.f, 0, stream);
-}
-
-extern "C" int b2u_stitch_accumulate_dev(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                                         const int32_t* y0, const int32_t* x0, const int32_t* sel,
-                                         const int32_t* n_sel_dev, int32_t max_sel, int32_t mode, float* acc,
-                                         uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off,
-                                         void* stream) {
-  B2U_CHECK_ARG(sel && n_sel_dev && max_sel > 0 && mode >= 0 && mode <= 2, "stitch_accumulate_dev: bad argument");
-  return stitch_accumulate_impl(logits, ld, C, T, th, tw, y0, x0, sel, max_sel, acc, cnt, Y, X, y_off, x_off,
-                                mode == 1 ? 31.f : 0.f, mode == 2 ? 1 : 0, stream, n_sel_dev);
-}
-
-extern "C" int b2u_stitch_accumulate_raw(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                                         const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel,
-                                         float* acc, uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off,
-                                         void* stream) {
-  return stitch_accumulate_impl(logits, ld, C, T, th, tw, y0, x0, sel, n_sel, acc, cnt, Y, X, y_off, x_off, 0.f, 1, stream);
 }
 
 extern "C" int b2u_stitch_finalize_mean(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X,
@@ -1790,25 +1764,11 @@ extern "C" int b2u_stitch_finalize_mean(const float* acc, const uint8_t* cnt, in
   return B2U_OK;
 }
 
-extern "C" int b2u_stitch_accumulate_q31(const float* logits, int32_t ld, int32_t C, int32_t T, int32_t th, int32_t tw,
-                                         const int32_t* y0, const int32_t* x0, const int32_t* sel, int32_t n_sel,
-                                         float* acc, uint8_t* cnt, int64_t Y, int64_t X, int64_t y_off, int64_t x_off,
-                                         void* stream) {
-  return stitch_accumulate_impl(logits, ld, C, T, th, tw, y0, x0, sel, n_sel, acc, cnt, Y, X, y_off, x_off, 31.f, 0, stream);
-}
-
-extern "C" int b2u_stitch_finalize(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, uint8_t* mask,
-                                   void* stream) {
+extern "C" int b2u_stitch_finalize(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, int32_t int_div,
+                                   uint8_t* mask, void* stream) {
   B2U_CHECK_ARG(acc && cnt && mask && C >= 1, "stitch_finalize: bad argument");
-  launch_k(stitch_finalize_kernel, dim3(grid_for(Y * X, 256)), dim3(256), 0, (cudaStream_t)stream, acc, cnt, C, Y * X, mask, 0);
-  B2U_LAUNCH_CHECK();
-  return B2U_OK;
-}
-
-extern "C" int b2u_stitch_finalize_q31(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X,
-                                       uint8_t* mask, void* stream) {
-  B2U_CHECK_ARG(acc && cnt && mask && C >= 1, "stitch_finalize_q31: bad argument");
-  launch_k(stitch_finalize_kernel, dim3(grid_for(Y * X, 256)), dim3(256), 0, (cudaStream_t)stream, acc, cnt, C, Y * X, mask, 1);
+  launch_k(stitch_finalize_kernel, dim3(grid_for(Y * X, 256)), dim3(256), 0, (cudaStream_t)stream, acc, cnt, C, Y * X, mask,
+           int_div);
   B2U_LAUNCH_CHECK();
   return B2U_OK;
 }

@@ -7,13 +7,13 @@ never leave HBM between the network and the stitch.
 """
 from __future__ import annotations
 
-from typing import List, Optional, Sequence, Tuple
+from typing import Optional, Sequence, Tuple
 
 import torch
 
 from . import _lib, ops
 from .network import UNetB200, input_contract
-from .tiling import Window, _split, colour_classes, compute_windows, shard_grid, shard_windows_2d, shard_windows_by_columns
+from .tiling import colour_classes, compute_windows, shard_windows_2d, shard_windows_by_columns, split_range
 
 
 def gather_mask_strips(strip: torch.Tensor, width: int, rank: int, world: int, dst: int = 0) -> Optional[torch.Tensor]:
@@ -24,8 +24,7 @@ def gather_mask_strips(strip: torch.Tensor, width: int, rank: int, world: int, d
     if world == 1:
         return strip
     Y = strip.shape[0]
-    base, rem = divmod(width, world)
-    widest = base + (1 if rem else 0)
+    widest = split_range(width, world, 0)[1]          # the first part is the widest
     # all_gather of column-major strips: [widest, Y] rows are contiguous columns of the mask
     buf = torch.zeros((widest, Y), dtype=strip.dtype, device=strip.device)
     buf[:strip.shape[1]] = strip.t()
@@ -35,8 +34,8 @@ def gather_mask_strips(strip: torch.Tensor, width: int, rank: int, world: int, d
         return None
     cols = []
     for r in range(world):
-        w_r = base + (1 if r < rem else 0)
-        cols.append(parts[r][:w_r])
+        xb, xe = split_range(width, world, r)
+        cols.append(parts[r][:xe - xb])
     return torch.cat(cols, 0).t().contiguous()
 
 
@@ -48,8 +47,7 @@ def gather_mask_cells(cell: torch.Tensor, height: int, width: int, grid: Tuple[i
     if world == 1:
         return cell
     gx, gy = grid
-    hmax = max(_split(height, gy, k)[1] - _split(height, gy, k)[0] for k in range(gy))
-    wmax = max(_split(width, gx, k)[1] - _split(width, gx, k)[0] for k in range(gx))
+    hmax, wmax = split_range(height, gy, 0)[1], split_range(width, gx, 0)[1]     # the first parts are the largest
     buf = torch.zeros((hmax, wmax), dtype=cell.dtype, device=cell.device)
     buf[:cell.shape[0], :cell.shape[1]] = cell
     parts = [torch.empty_like(buf) for _ in range(world)]
@@ -58,10 +56,81 @@ def gather_mask_cells(cell: torch.Tensor, height: int, width: int, grid: Tuple[i
         return None
     full = torch.empty((height, width), dtype=cell.dtype, device=cell.device)
     for r in range(world):
-        xb, xe = _split(width, gx, r % gx)
-        yb, ye = _split(height, gy, r // gx)
+        xb, xe = split_range(width, gx, r % gx)
+        yb, ye = split_range(height, gy, r // gx)
         full[yb:ye, xb:xe] = parts[r][:ye - yb, :xe - xb]
     return full
+
+
+class StitchPlan:
+    """The overlap stitching of one job's predicted tiles into the output rectangle `region` = (yb, ye, xb, xe) of the
+    raster: per batch of tiles the network has just run, one `b2u_stitch_accumulate` launch per colour class adds the
+    tiles into `acc` (fp32 [n_out, ye-yb, xe-xb]) and `cnt` (uint8 [ye-yb, xe-xb]); `mask` / `mean` finalize them.
+    mode 0: softmax probabilities, 1: the reference's int8 `large_file` merge (x31, floor division), 2: the raw
+    network output (regression).  `origins[i][:2]` is the (x, y) of tile i of the raster; `batches[b]` lists the tiles
+    of batch b in batch order (at most net.N).
+    Per-batch metadata block (int32): y0[B] x0[B], then one (count, sel[B]) slot per colour class, as many slots as the
+    batch with the most classes needs (tiles overlapping beyond their direct neighbours need more than 2 x 2).  The
+    blocks of the whole job go to the device in ONE copy: a small pageable host-to-device copy per batch would block
+    the host behind the previous batch's kernels every time (measured on the 20000 x 20000 raster: 10.08k -> 10.46k
+    tiles/s); `load` refills the current block device-to-device in front of the batch."""
+
+    def __init__(self, net: UNetB200, origins: Sequence[Sequence[int]], batches: Sequence[Sequence[int]],
+                 region: Tuple[int, int, int, int], mode: int):
+        B, P = net.N, net.H
+        self.net, self.mode = net, mode
+        self.yb, ye, self.xb, xe = region
+        self.SY, self.SX = ye - self.yb, xe - self.xb
+        classes = [colour_classes([(origins[i][0], origins[i][1], P, P) for i in idx]) for idx in batches]
+        self.n_classes = max((len(c) for c in classes), default=0)
+        blk = 2 * B + self.n_classes * (1 + B)
+        host = torch.zeros((max(1, len(batches)), blk), dtype=torch.int32)
+        for row, idx, cls_b in zip(host, batches, classes):
+            pad = list(idx) + [idx[0]] * (B - len(idx))      # padded tiles are never selected for stitching
+            row[:B] = torch.tensor([origins[i][1] for i in pad], dtype=torch.int32)
+            row[B:2 * B] = torch.tensor([origins[i][0] for i in pad], dtype=torch.int32)
+            for k, cls in enumerate(cls_b):
+                o = 2 * B + k * (1 + B)
+                row[o] = len(cls)
+                row[o + 1:o + 1 + len(cls)] = torch.tensor(cls, dtype=torch.int32)
+        self.meta = host.to(net.device)
+        self.cur = torch.zeros(blk, dtype=torch.int32, device=net.device)
+        self.acc = torch.zeros((net.n_out, self.SY, self.SX), dtype=torch.float32, device=net.device)
+        self.cnt = torch.zeros((self.SY, self.SX), dtype=torch.uint8, device=net.device)
+
+    def load(self, b: int) -> Tuple[int, int]:
+        """makes batch b's block current (a device copy on the current stream, which the plan's launches must use too);
+        returns the device pointers of its tile rows y0[B] and x0[B]"""
+        self.cur.copy_(self.meta[b], non_blocking=True)
+        cb = self.cur.data_ptr()
+        return cb, cb + 4 * self.net.N
+
+    def accumulate(self, stream: int) -> None:
+        """adds the current batch's tiles, as the network left them in its logits, into the accumulators"""
+        net, B, P = self.net, self.net.N, self.net.H
+        cb = self.cur.data_ptr()
+        for k in range(self.n_classes):
+            o = cb + 4 * (2 * B + k * (1 + B))
+            _lib.check(net.lib.b2u_stitch_accumulate(net.logits.data_ptr(), net.logits.shape[-1], net.n_out, B, P, P, cb,
+                                                     cb + 4 * B, o + 4, o, B, self.mode, self.acc.data_ptr(),
+                                                     self.cnt.data_ptr(), self.SY, self.SX, self.yb, self.xb, stream),
+                       "b2u_stitch_accumulate")
+
+    def mask(self, stream: int) -> torch.Tensor:
+        """the stitched argmax, uint8 [SY, SX] (unplaced pixels 0)"""
+        out = torch.empty((self.SY, self.SX), dtype=torch.uint8, device=self.acc.device)
+        _lib.check(self.net.lib.b2u_stitch_finalize(self.acc.data_ptr(), self.cnt.data_ptr(), self.net.n_out, self.SY,
+                                                    self.SX, int(self.mode == 1), out.data_ptr(), stream),
+                   "b2u_stitch_finalize")
+        return out
+
+    def mean(self, nodata: float, stream: int) -> torch.Tensor:
+        """the overlap average, fp32 [n_out, SY, SX], `nodata` where no tile was placed"""
+        out = torch.empty_like(self.acc)
+        _lib.check(self.net.lib.b2u_stitch_finalize_mean(self.acc.data_ptr(), self.cnt.data_ptr(), self.net.n_out,
+                                                         self.SY, self.SX, float(nodata), out.data_ptr(), stream),
+                   "b2u_stitch_finalize_mean")
+        return out
 
 
 class TiledPredictor:
@@ -70,8 +139,6 @@ class TiledPredictor:
         self.net, self.lib, self.dev = net, net.lib, net.device
         self.B, self.P = net.N, net.H
         assert net.H == net.W
-
-    MAX_CLASSES = 4       # tiles on a regular grid overlap their direct neighbours only: 2 x 2 colour classes
 
     def predict_raster(self, raster: torch.Tensor, patch_overlap: float, rank: int = 0, world: int = 1,
                        return_probs: bool = False, large_file: bool = False, grid: Optional[Tuple[int, int]] = None):
@@ -82,10 +149,10 @@ class TiledPredictor:
         the return value is (mask [y_end-y_begin, x_end-x_begin], (x_begin, x_end, y_begin, y_end)).  `large_file`: the
         reference's int8 merge (predict.py:217-219, 318-323).  `return_probs` also returns the accumulators.
         One batch = crop -> forward -> one accumulate per colour class, every launch reading the batch's tile origins /
-        class lists from a fixed device block that is refilled (device-to-device) in front of it - no host round trip, no
-        per-batch host-to-device copy.  (Replaying the batch as a captured CUDA graph was measured and dropped: with
+        class lists from the `StitchPlan`'s device block, refilled (device-to-device) in front of it - no host round trip,
+        no per-batch host-to-device copy.  (Replaying the batch as a captured CUDA graph was measured and dropped: with
         programmatic dependent launch the eager launches already overlap, 5.86 vs 6.07 ms per batch of 64 tiles.)"""
-        net, lib, dev, P, B = self.net, self.lib, self.dev, self.P, self.B
+        net, lib, P, B = self.net, self.lib, self.P, self.B
         assert raster.is_cuda and raster.dim() == 3 and raster.is_contiguous()
         r_dt, r_div, r_div2 = input_contract(raster.dtype, net.input_div)
         Cc, Y, X = raster.shape
@@ -96,59 +163,24 @@ class TiledPredictor:
             yb, ye = 0, Y
         else:
             idx, (xb, xe, yb, ye) = shard_windows_2d(windows, X, Y, rank, world, grid)
-        SX, SY = xe - xb, ye - yb
-        acc = torch.zeros((net.n_out, SY, SX), dtype=torch.float32, device=dev)
-        cnt = torch.zeros((SY, SX), dtype=torch.uint8, device=dev)
-        mask = torch.empty((SY, SX), dtype=torch.uint8, device=dev)
-        ld = net.logits.shape[-1]
         self.tiles_run = len(idx)
-        # Per-batch metadata block (int32): y0[B] x0[B] then MAX_CLASSES x (count, sel[B]).  The blocks of the whole job go
-        # to the device in ONE copy: a small pageable host-to-device copy per batch would block the host behind the
-        # previous batch's kernels every time (measured on the 20000 x 20000 raster: 10.08k -> 10.46k tiles/s)
-        MC = self.MAX_CLASSES
-        blk = 2 * B + MC * (1 + B)
-        n_batches = (len(idx) + B - 1) // B
-        host = torch.zeros((max(1, n_batches), blk), dtype=torch.int32)
-        for b in range(n_batches):
-            wins = [windows[i] for i in idx[b * B:(b + 1) * B]]
-            pad = wins + [wins[0]] * (B - len(wins))      # padded tiles are never selected for stitching
-            row = host[b]
-            row[:B] = torch.tensor([w[1] for w in pad], dtype=torch.int32)
-            row[B:2 * B] = torch.tensor([w[0] for w in pad], dtype=torch.int32)
-            classes = colour_classes(wins)
-            assert len(classes) <= MC, "tiles overlap more than their direct neighbours"
-            for k, cls in enumerate(classes):
-                o = 2 * B + k * (1 + B)
-                row[o] = len(cls)
-                row[o + 1:o + 1 + len(cls)] = torch.tensor(cls, dtype=torch.int32)
-        meta = host.to(dev)
-        cur = torch.zeros(blk, dtype=torch.int32, device=dev)
-        self._keep = (meta, cur)
-        cb = cur.data_ptr()
-        mode = 1 if large_file else 0
-
-        def one_batch(s):
-            _lib.check(lib.b2u_crop_tiles(raster.data_ptr(), r_dt, r_div, r_div2, Cc, Y, X, cb, cb + 4 * B, B, P,
+        batches = [idx[b0:b0 + B] for b0 in range(0, len(idx), B)]
+        plan = StitchPlan(net, windows, batches, (yb, ye, xb, xe), 1 if large_file else 0)
+        self._keep = plan           # its device blocks are read by launches still in flight when this returns
+        s = ops.stream_ptr()
+        for b in range(len(batches)):
+            y0, x0 = plan.load(b)
+            _lib.check(lib.b2u_crop_tiles(raster.data_ptr(), r_dt, r_div, r_div2, Cc, Y, X, y0, x0, B, P,
                                           net.x_in.t.data_ptr(), net.x_in.ld, s), "b2u_crop_tiles")
             net.forward(s)
-            for k in range(MC):
-                o = cb + 4 * (2 * B + k * (1 + B))
-                _lib.check(lib.b2u_stitch_accumulate_dev(net.logits.data_ptr(), ld, net.n_out, B, P, P, cb, cb + 4 * B,
-                                                         o + 4, o, B, mode, acc.data_ptr(), cnt.data_ptr(), SY, SX, yb, xb,
-                                                         s), "b2u_stitch_accumulate_dev")
-
-        s = ops.stream_ptr()
-        for b in range(n_batches):
-            cur.copy_(meta[b], non_blocking=True)
-            one_batch(s)
-        finalize = lib.b2u_stitch_finalize_q31 if large_file else lib.b2u_stitch_finalize
-        _lib.check(finalize(acc.data_ptr(), cnt.data_ptr(), net.n_out, SY, SX, mask.data_ptr(), s), "b2u_stitch_finalize")
-        self.last_stitch_profile = {"batches": n_batches, "tiles_run": len(idx),
-                                    "launches_per_batch": 1 + net.launches_fwd + MC + 1}
+            plan.accumulate(s)
+        mask = plan.mask(s)
+        self.last_stitch_profile = {"batches": len(batches), "tiles_run": len(idx),
+                                    "launches_per_batch": 1 + net.launches_fwd + plan.n_classes + 1}
         if grid is not None:
-            return (mask, (xb, xe, yb, ye), acc, cnt) if return_probs else (mask, (xb, xe, yb, ye))
+            return (mask, (xb, xe, yb, ye), plan.acc, plan.cnt) if return_probs else (mask, (xb, xe, yb, ye))
         if return_probs:
-            return mask, xb, xe, acc, cnt
+            return mask, xb, xe, plan.acc, plan.cnt
         return mask, xb, xe
 
     def _forward_tiles(self, tiles: torch.Tensor) -> int:

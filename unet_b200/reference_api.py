@@ -36,10 +36,10 @@ from . import _lib, ops
 from .assessment import ConfusionCounter, write_report
 from .engine import Trainer, one_cycle
 from .network import UNetB200, input_divisors
-from .predict_engine import TiledPredictor, gather_mask_strips
+from .predict_engine import StitchPlan, TiledPredictor, gather_mask_strips
 from .losses import LossSpec, dice_blocks_per_sample, launch_loss, parse_loss_func, warn_dice_weights
 from .geotiff import GeoInfo, geotiff_info, open_mask, open_tile, read_geotiff, write_geotiff
-from .tiling import colour_classes, compute_windows, placement_from_geotransform, shard_windows_by_columns
+from .tiling import column_owned, compute_windows, placement_from_geotransform, shard_windows_by_columns, split_range
 
 ARCHITECTURES = ("xresnet18", "xresnet34", "xresnet50", "xresnet101")   # params_and_main.py:12,99
 
@@ -473,45 +473,24 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
         xmax_r, ymin_r = int(np.argmax(gts[:, 0])), int(np.argmin(gts[:, 3]))
         x_len = round((gts[:, 0].max() + gts[xmax_r, 1] * gts[xmax_r, 2] - ulx_full) / gts[0, 2])
         y_len = round((gts[:, 3].min() + gts[ymin_r, 4] * gts[ymin_r, 5] - uly_full) / gts[0, 5])
-        place = [placement_from_geotransform(g[0], P, g[2], g[3], P, g[5], ulx_full, uly_full) for g in gts]
-        # owner-computes column strip of this rank (the whole mosaic on one GPU): every tile that intersects it
-        xb, xe, mine, own = _merge_strip(place, P, x_len, rank, world)
-        SX = xe - xb
+        wins = [(x0, y0, P, P) for x0, y0, _, _ in
+                (placement_from_geotransform(g[0], P, g[2], g[3], P, g[5], ulx_full, uly_full) for g in gts)]
+        # owner-computes column strip of this rank (the whole mosaic on one GPU): every tile that intersects it; the
+        # rank owning a tile's left edge assesses it
+        mine, xb, xe = shard_windows_by_columns(wins, x_len, rank, world)
+        own = column_owned(wins, mine, xb, xe)
         if assess:
-            counter = ConfusionCounter(net.n_out, dev, max(sum(_merge_strip(place, P, x_len, r, world)[3])
-                                                           for r in range(world)), rank, world)
+            n_own = max(sum(column_owned(wins, *shard_windows_by_columns(wins, x_len, r, world))) for r in range(world))
+            counter = ConfusionCounter(net.n_out, dev, n_own, rank, world)
             amax_dev = torch.empty((B, P, P), dtype=torch.uint8, device=dev)
-        acc = torch.zeros((net.n_out, y_len, SX), dtype=torch.float32, device=dev)
-        cnt = torch.zeros((y_len, SX), dtype=torch.uint8, device=dev)
-        accumulate = (lib.b2u_stitch_accumulate_raw if regression else
-                      lib.b2u_stitch_accumulate_q31 if large_file else lib.b2u_stitch_accumulate)
-        # tile origins and the colour classes of every batch go to the device in one copy (no per-batch pageable
-        # uploads, no per-batch synchronisation beyond the reuse of the pinned staging buffer)
-        flat: List[int] = []
-        plan = []
-        for b0 in range(0, len(mine), B):
-            idx = mine[b0:b0 + B]
-            wins = [(place[i][0], place[i][1], P, P) for i in idx]
-            oy = len(flat)
-            flat += [w_[1] for w_ in wins] + [0] * (B - len(idx))
-            ox = len(flat)
-            flat += [w_[0] for w_ in wins] + [0] * (B - len(idx))
-            classes = []
-            for cls in colour_classes(wins):
-                classes.append((len(flat), len(cls)))
-                flat += cls
-            plan.append((oy, ox, classes))
-        meta = torch.tensor(flat if flat else [0], dtype=torch.int32).to(dev)
-        mbase = meta.data_ptr()
+        plan = StitchPlan(net, wins, [mine[b0:b0 + B] for b0 in range(0, len(mine), B)], (0, y_len, xb, xe),
+                          2 if regression else 1 if large_file else 0)
         s_ = ops.stream_ptr()
-        for (b0, chunk, _, x, ys, ny), (oy, ox, classes) in zip(batches([tiles[i] for i in mine],
-                                                                         own if assess else None), plan):
+        for b, (b0, chunk, _, x, ys, ny) in enumerate(batches([tiles[i] for i in mine], own if assess else None)):
+            plan.load(b)
             net.set_input(x.to(dev, non_blocking=True))
             net.forward()
-            for osel, nsel in classes:
-                _lib.check(accumulate(net.logits.data_ptr(), net.logits.shape[-1], net.n_out, B, P, P, mbase + 4 * oy,
-                                      mbase + 4 * ox, mbase + 4 * osel, nsel, acc.data_ptr(), cnt.data_ptr(), y_len, SX,
-                                      0, xb, s_), "b2u_stitch_accumulate")
+            plan.accumulate(s_)
             if ny:
                 # the per-tile argmax (what predict_tiles returns) of the tiles this rank owns, packed in batch order
                 k, ld = 0, net.logits.shape[-1]
@@ -525,31 +504,21 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
             _write_validation(counter, world, rank, out_dir, AOI, year, model_name, class_zero)
         nodata = None
         if regression:
-            outd = torch.empty((1, y_len, SX), dtype=torch.float32, device=dev)
-            _lib.check(lib.b2u_stitch_finalize_mean(acc.data_ptr(), cnt.data_ptr(), 1, y_len, SX, -9999.0,
-                                                    outd.data_ptr(), s_), "b2u_stitch_finalize_mean")
-            strip, nodata = outd[0], -9999                                                     # predict.py:313-316
+            strip, nodata = plan.mean(-9999, s_)[0], -9999                                   # predict.py:313-316
         elif all_classes or specific_class is not None:
             if large_file:
                 # int8 sums floor-divided by the count (predict.py:318-323): the reference's own host arithmetic
-                m = acc.cpu().numpy().astype(np.int8)
-                c8 = cnt.cpu().numpy().astype(np.int8)
+                m = plan.acc.cpu().numpy().astype(np.int8)
+                c8 = plan.cnt.cpu().numpy().astype(np.int8)
                 mk = np.broadcast_to(c8 > 0, m.shape)
                 m[mk] //= np.broadcast_to(c8, m.shape)[mk]
                 strip = torch.from_numpy(m).to(dev)
             else:
-                outd = torch.empty_like(acc)
-                _lib.check(lib.b2u_stitch_finalize_mean(acc.data_ptr(), cnt.data_ptr(), net.n_out, y_len, SX, 0.0,
-                                                        outd.data_ptr(), s_), "b2u_stitch_finalize_mean")
-                strip = outd
+                strip = plan.mean(0, s_)
             if not all_classes:
                 strip = strip[specific_class]
         else:
-            mask = torch.empty((y_len, SX), dtype=torch.uint8, device=dev)
-            finalize = lib.b2u_stitch_finalize_q31 if large_file else lib.b2u_stitch_finalize
-            _lib.check(finalize(acc.data_ptr(), cnt.data_ptr(), net.n_out, y_len, SX, mask.data_ptr(), s_),
-                       "b2u_stitch_finalize")
-            strip = mask
+            strip = plan.mask(s_)
         full = _gather_strips(strip.contiguous(), x_len, rank, world) if world > 1 else strip
         if rank != 0:
             return None
@@ -611,17 +580,6 @@ def _load_labels(path: Path, n_classes: int, P: int) -> np.ndarray:
     if y.shape != (P, P):
         raise ValueError(f"{path}: mask tile of shape {y.shape}, expected ({P}, {P})")
     return _label_values(y, n_classes, False, path)
-
-
-def _merge_strip(place, P: int, x_len: int, rank: int, world: int):
-    """The owner-computes column strip [xb, xe) of `rank` in a mosaic `x_len` wide, the indices of the tiles at
-    `place` [(x, y, ...)] that intersect it (`mine`: the tiles the rank predicts) and, per tile of `mine`, whether the
-    rank owns it (its left edge column lies in the strip): every tile has exactly one owner, which assesses it."""
-    base_w, rem_w = divmod(x_len, world)
-    xb = rank * base_w + min(rank, rem_w)
-    xe = xb + base_w + (1 if rank < rem_w else 0)
-    mine = [i for i in range(len(place)) if place[i][0] < xe and place[i][0] + P > xb]
-    return xb, xe, mine, [xb <= place[i][0] < xe for i in mine]
 
 
 def _runs(flags: Sequence[bool]) -> List[Tuple[int, int]]:
@@ -686,9 +644,7 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
         counter = ConfusionCounter(net.n_out, net.device)
     for k in range(n_strips):
         # strip k of this rank's columns: the balanced partition of [xb, xe), then the tile columns intersecting it
-        base, rem = divmod(xe - xb, n_strips)
-        sb = xb + k * base + min(k, rem)
-        se = sb + base + (1 if k < rem else 0)
+        sb, se = (xb + v for v in split_range(xe - xb, n_strips, k))
         idx = [i for i, (x, y, w, h) in enumerate(windows) if x < se and x + w > sb]
         xs0 = min(windows[i][0] for i in idx)
         xs1 = max(windows[i][0] + windows[i][2] for i in idx)

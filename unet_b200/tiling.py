@@ -84,21 +84,27 @@ def colour_classes(windows: Sequence[Window]) -> List[List[int]]:
     return [c for c in classes if c]
 
 
+def split_range(n: int, parts: int, k: int) -> Tuple[int, int]:
+    """[begin, end) of part k of the balanced partition of range(n) into `parts` contiguous parts: the first n % parts
+    parts take one more.  Every sharding of the output and every gather of the shards uses this one partition."""
+    base, rem = divmod(n, parts)
+    b = k * base + min(k, rem)
+    return b, b + base + (1 if k < rem else 0)
+
+
 def shard_windows_by_columns(windows: Sequence[Window], width: int, rank: int, world: int):
     """Owner-computes sharding for multi-GPU prediction (SURVEY 8(e)): rank r owns output columns [X_r, X_{r+1}) and
     runs every tile that intersects them, so sum / count / argmax of its strip are local and bit-identical to a
     single-GPU run.  Returns (tile indices, x_begin, x_end)."""
-    base, rem = divmod(width, world)
-    xb = rank * base + min(rank, rem)
-    xe = xb + base + (1 if rank < rem else 0)
+    xb, xe = split_range(width, world, rank)
     idx = [i for i, (x, y, w, h) in enumerate(windows) if x < xe and x + w > xb]
     return idx, xb, xe
 
 
-def _split(n: int, parts: int, k: int) -> Tuple[int, int]:
-    base, rem = divmod(n, parts)
-    b = k * base + min(k, rem)
-    return b, b + base + (1 if k < rem else 0)
+def column_owned(windows: Sequence[Window], idx: Sequence[int], xb: int, xe: int) -> List[bool]:
+    """Per tile of `idx`: whether its left edge column lies in [xb, xe).  Over the strips of `shard_windows_by_columns`
+    every tile has exactly one owner, so work done once per tile (counting it in an assessment) is done by one rank."""
+    return [xb <= windows[i][0] < xe for i in idx]
 
 
 def shard_grid(windows: Sequence[Window], width: int, height: int, world: int) -> Tuple[int, int]:
@@ -113,8 +119,8 @@ def shard_grid(windows: Sequence[Window], width: int, height: int, world: int) -
         gy = world // gx
         worst = 0
         for r in range(world):
-            xb, xe = _split(width, gx, r % gx)
-            yb, ye = _split(height, gy, r // gx)
+            xb, xe = split_range(width, gx, r % gx)
+            yb, ye = split_range(height, gy, r // gx)
             worst = max(worst, sum(1 for (x, y, w, h) in windows if x < xe and x + w > xb and y < ye and y + h > yb))
         key = (worst, gy)              # ties: fewer row cuts (strips keep whole raster rows contiguous)
         if best is None or key < best[0]:
@@ -128,7 +134,7 @@ def shard_windows_2d(windows: Sequence[Window], width: int, height: int, rank: i
     tile that intersects it - sums, counts and argmax of the cell are local, exactly as with column strips.
     Returns (tile indices, (x_begin, x_end, y_begin, y_end))."""
     gx, gy = grid or shard_grid(windows, width, height, world)
-    xb, xe = _split(width, gx, rank % gx)
-    yb, ye = _split(height, gy, rank // gx)
+    xb, xe = split_range(width, gx, rank % gx)
+    yb, ye = split_range(height, gy, rank // gx)
     idx = [i for i, (x, y, w, h) in enumerate(windows) if x < xe and x + w > xb and y < ye and y + h > yb]
     return idx, (xb, xe, yb, ye)
