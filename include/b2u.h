@@ -416,6 +416,21 @@ int b2u_softmax_nchw(const float* logits, int32_t ld, int32_t C, int64_t tiles, 
 int b2u_confusion_counts(const uint8_t* pred, int64_t pred_pitch, int64_t pred_stride, const uint8_t* truth,
                          int64_t truth_pitch, int64_t truth_stride, int32_t T, int32_t H, int32_t W, int32_t C,
                          uint64_t* joint, uint32_t* tile_hist, uint64_t* skipped, void* stream);
+/* ---- assessment of regression maps: error statistics of fp32 predictions against fp32 truth ------------------------
+ * Same layout as b2u_confusion_counts, in floats: pixel (t, y, x) of a map is at base + t * stride + y * pitch + x
+ * (4-byte aligned; rows are read with 16-byte loads where both maps allow).  A pixel is skipped (skipped += 1, uint64)
+ * when either value is not finite, the prediction equals pred_nodata or the truth equals truth_nodata (NaN: no nodata
+ * value).  Over the counted pixels, with e = p - t, a record of 15 doubles holds
+ *   {n, mean t, mean p, M2 t, M2 p, C tp, sum |e|, sum e, sum e^2, min t, max t, min p, max p, min e, max e}
+ * (M2 = sum of squared deviations from the mean, C = sum of the products of the deviations).  `totals` (double [15]) and
+ * `tile_rec` (nullable, double [T][15], one record per image) are merged with the call's records by Chan et al.'s pairwise
+ * update, so they accumulate over calls; a zero-filled record is empty.  scratch: `scratch_records` >= T records of 15
+ * doubles (more records allow more blocks per image); ticket: one zero-initialised uint32 that the call leaves zero.
+ * Every merge happens in a fixed order, without float atomics: the records are the same bits on every run. */
+int b2u_regression_assess(const float* pred, int64_t pred_pitch, int64_t pred_stride, const float* truth,
+                          int64_t truth_pitch, int64_t truth_stride, int32_t T, int32_t H, int32_t W, float pred_nodata,
+                          float truth_nodata, double* totals, double* tile_rec, uint64_t* skipped, double* scratch,
+                          int64_t scratch_records, uint32_t* ticket, void* stream);
 
 /* ---- SelfAttention (fastai layers.SelfAttention on UnetBlock.conv2 when self_attention=True, train.py:142) --------
  * The 1x1 query / key / value convolutions run through b2u_conv_*, the two batched attention products are plain

@@ -1359,6 +1359,191 @@ __global__ void __launch_bounds__(256) confusion_counts_kernel(const uint8_t* __
   if (threadIdx.x == 0 && sskip) atomicAdd(skipped, (unsigned long long)sskip);
 }
 
+// Error statistics of a prediction map against a truth map (b2u.h b2u_regression_assess).  The record is
+// {n, mean t, mean p, M2 t, M2 p, co-moment, sum |e|, sum e, sum e^2, min t, max t, min p, max p, min e, max e}.
+constexpr int REG_K = 15;
+struct RegMoments {
+  double v[REG_K];
+};
+
+// Chan et al.'s pairwise update of (n, means, M2, co-moment); the sums add, the extremes combine.  An empty side
+// (n == 0) leaves the other unchanged, so a zero-filled record is the empty record.
+__device__ __forceinline__ void reg_merge(RegMoments& a, const RegMoments& b) {
+  if (b.v[0] == 0.0) return;
+  if (a.v[0] == 0.0) { a = b; return; }
+  const double n = a.v[0] + b.v[0], f = b.v[0] / n, w = a.v[0] * f;
+  const double dt = b.v[1] - a.v[1], dp = b.v[2] - a.v[2];
+  a.v[0] = n;
+  a.v[1] += dt * f;
+  a.v[2] += dp * f;
+  a.v[3] += b.v[3] + dt * dt * w;
+  a.v[4] += b.v[4] + dp * dp * w;
+  a.v[5] += b.v[5] + dt * dp * w;
+#pragma unroll
+  for (int k = 6; k < 9; ++k) a.v[k] += b.v[k];
+#pragma unroll
+  for (int k = 9; k < REG_K; k += 2) { a.v[k] = fmin(a.v[k], b.v[k]); a.v[k + 1] = fmax(a.v[k + 1], b.v[k + 1]); }
+}
+
+__device__ __forceinline__ void reg_load(RegMoments& m, const double* p) {
+#pragma unroll
+  for (int k = 0; k < REG_K; ++k) m.v[k] = __ldcg(p + k);
+}
+
+__device__ __forceinline__ void reg_store(double* p, const RegMoments& m) {
+#pragma unroll
+  for (int k = 0; k < REG_K; ++k) p[k] = m.v[k];
+}
+
+// lane 0 receives the merge of the warp's records, always in the same tree order
+__device__ __forceinline__ void reg_warp_merge(RegMoments& m) {
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    RegMoments other;
+#pragma unroll
+    for (int k = 0; k < REG_K; ++k) other.v[k] = __shfl_down_sync(0xffffffffu, m.v[k], o);
+    if ((threadIdx.x & (2 * o - 1)) == 0) reg_merge(m, other);
+  }
+}
+
+// one thread's pixels as plain sums, shifted by its first counted pixel so that offset data (1000 +- 0.01) keeps its
+// variance; min / max of t and p in fp32 (exact)
+struct RegThread {
+  float pnd, tnd;
+  float kt = 0.f, kp = 0.f;
+  unsigned n = 0, skip = 0;
+  double st = 0, sp = 0, stt = 0, spp = 0, stp = 0, sa = 0, se = 0, see = 0;
+  float mint = INFINITY, maxt = -INFINITY, minp = INFINITY, maxp = -INFINITY;
+  double mine = INFINITY, maxe = -INFINITY;
+
+  __device__ __forceinline__ void px(float p, float t) {
+    // a NaN nodata compares unequal to everything: "no nodata value"
+    if (!isfinite(p) || !isfinite(t) || p == pnd || t == tnd) { ++skip; return; }
+    if (n == 0) { kt = t; kp = p; }
+    ++n;
+    const double dt = (double)t - kt, dp = (double)p - kp, e = (double)p - (double)t;
+    st += dt; sp += dp; stt += dt * dt; spp += dp * dp; stp += dt * dp;
+    sa += fabs(e); se += e; see += e * e;
+    mint = fminf(mint, t); maxt = fmaxf(maxt, t); minp = fminf(minp, p); maxp = fmaxf(maxp, p);
+    mine = fmin(mine, e); maxe = fmax(maxe, e);
+  }
+  __device__ __forceinline__ void px4(float4 p, float4 t) { px(p.x, t.x); px(p.y, t.y); px(p.z, t.z); px(p.w, t.w); }
+
+  __device__ __forceinline__ RegMoments moments() const {
+    RegMoments m;
+    if (n == 0) {
+#pragma unroll
+      for (int k = 0; k < REG_K; ++k) m.v[k] = 0.0;
+      return m;
+    }
+    const double c = n, mt = st / c, mp = sp / c;
+    m.v[0] = c; m.v[1] = kt + mt; m.v[2] = kp + mp;
+    m.v[3] = fmax(0.0, stt - st * mt); m.v[4] = fmax(0.0, spp - sp * mp); m.v[5] = stp - st * mp;
+    m.v[6] = sa; m.v[7] = se; m.v[8] = see;
+    m.v[9] = mint; m.v[10] = maxt; m.v[11] = minp; m.v[12] = maxp; m.v[13] = mine; m.v[14] = maxe;
+    return m;
+  }
+};
+
+// Grid (row blocks, T images), 256 threads, a warp per row as in confusion_counts_kernel.  Each block leaves its merged
+// record in partial[t * gx + bx]; the last block to finish (ticket) folds them: a warp per image over its gx blocks,
+// then warp 0 over the images, every merge in a fixed order, so the records are the same bits on every run.
+__global__ void __launch_bounds__(256) regression_assess_kernel(
+    const float* __restrict__ pred, long long pp, long long ps, const float* __restrict__ truth, long long tp,
+    long long ts, int T, int H, int W, int rows, float pnd, float tnd, double* __restrict__ totals,
+    double* __restrict__ tile_rec, unsigned long long* __restrict__ skipped, double* __restrict__ partial,
+    unsigned* __restrict__ ticket) {
+  __shared__ double sw[8][REG_K];
+  __shared__ unsigned sskip;
+  __shared__ bool last;
+  pdl_enter();
+  if (threadIdx.x == 0) sskip = 0u;
+  RegThread c;
+  c.pnd = pnd; c.tnd = tnd;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  const int t = blockIdx.y, gx = gridDim.x;
+  const int y1 = min(H, (blockIdx.x + 1) * rows);
+  for (int y = blockIdx.x * rows + warp; y < y1; y += nw) {
+    const float* p = pred + t * ps + y * pp;
+    const float* q = truth + t * ts + y * tp;
+    // 16-byte loads from the first 16-byte boundary of the row when both rows sit at the same offset from it
+    int head = (int)(((16 - (reinterpret_cast<uintptr_t>(p) & 15)) & 15) >> 2);
+    if ((reinterpret_cast<uintptr_t>(p) ^ reinterpret_cast<uintptr_t>(q)) & 15) head = W;
+    head = min(head, W);
+    const int nv = (W - head) >> 2;
+    for (int x = lane; x < head; x += 32) c.px(__ldg(p + x), __ldg(q + x));
+    const float4* pv = reinterpret_cast<const float4*>(p + head);
+    const float4* qv = reinterpret_cast<const float4*>(q + head);
+    int v = lane;
+    for (; v + 96 < nv; v += 128) {     // four chunk pairs in flight per lane
+      float4 a[4], b[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) { a[u] = __ldg(pv + v + 32 * u); b[u] = __ldg(qv + v + 32 * u); }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) c.px4(a[u], b[u]);
+    }
+    for (; v < nv; v += 32) c.px4(__ldg(pv + v), __ldg(qv + v));
+    for (int x = head + 4 * nv + lane; x < W; x += 32) c.px(__ldg(p + x), __ldg(q + x));
+  }
+  RegMoments m = c.moments();
+  reg_warp_merge(m);
+  const unsigned sk = __reduce_add_sync(0xffffffffu, c.skip);
+  __syncthreads();                                    // sskip is initialised
+  if (lane == 0) {
+#pragma unroll
+    for (int k = 0; k < REG_K; ++k) sw[warp][k] = m.v[k];
+    if (sk) atomicAdd(&sskip, sk);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    RegMoments b = m;
+    for (int i = 1; i < nw; ++i) {
+      RegMoments o;
+#pragma unroll
+      for (int k = 0; k < REG_K; ++k) o.v[k] = sw[i][k];
+      reg_merge(b, o);
+    }
+    reg_store(partial + ((long long)t * gx + blockIdx.x) * REG_K, b);
+    if (sskip) atomicAdd(skipped, (unsigned long long)sskip);
+    __threadfence();
+    last = atomicAdd(ticket, 1u) == (unsigned)(gx * T) - 1u;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  // per image: lanes fold the image's blocks lane, lane + 32, ... in order, then the warp tree
+  for (int i = warp; i < T; i += nw) {
+    RegMoments r, o;
+#pragma unroll
+    for (int k = 0; k < REG_K; ++k) r.v[k] = 0.0;
+    for (int b = lane; b < gx; b += 32) { reg_load(o, partial + ((long long)i * gx + b) * REG_K); reg_merge(r, o); }
+    reg_warp_merge(r);
+    __syncwarp();
+    if (lane == 0) {
+      reg_store(partial + (long long)i * gx * REG_K, r);
+      if (tile_rec) {
+        reg_load(o, tile_rec + (long long)i * REG_K);
+        reg_merge(o, r);
+        reg_store(tile_rec + (long long)i * REG_K, o);
+      }
+    }
+  }
+  __syncthreads();
+  if (warp == 0) {
+    RegMoments r, o;
+#pragma unroll
+    for (int k = 0; k < REG_K; ++k) r.v[k] = 0.0;
+    for (int i = lane; i < T; i += 32) { reg_load(o, partial + (long long)i * gx * REG_K); reg_merge(r, o); }
+    reg_warp_merge(r);
+    if (lane == 0) {
+      reg_load(o, totals);
+      reg_merge(o, r);
+      reg_store(totals, o);
+      *ticket = 0u;
+    }
+  }
+}
+
 }  // namespace b2u
 
 using namespace b2u;
@@ -1812,6 +1997,33 @@ extern "C" int b2u_confusion_counts(const uint8_t* pred, int64_t pred_pitch, int
     launch_k(confusion_counts_kernel<false>, dim3((unsigned)gx, T), dim3(256), 0, st, pred, (long long)pred_pitch,
              (long long)pred_stride, truth, (long long)truth_pitch, (long long)truth_stride, H, W, C, (int)rows,
              (unsigned long long*)joint, tile_hist, (unsigned long long*)skipped);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_regression_assess(const float* pred, int64_t pred_pitch, int64_t pred_stride, const float* truth,
+                                     int64_t truth_pitch, int64_t truth_stride, int32_t T, int32_t H, int32_t W,
+                                     float pred_nodata, float truth_nodata, double* totals, double* tile_rec,
+                                     uint64_t* skipped, double* scratch, int64_t scratch_records, uint32_t* ticket,
+                                     void* stream) {
+  B2U_CHECK_ARG(pred && truth && totals && skipped && scratch && ticket, "regression_assess: null argument");
+  B2U_CHECK_ARG(((reinterpret_cast<uintptr_t>(pred) | reinterpret_cast<uintptr_t>(truth)) & 3) == 0,
+                "regression_assess: fp32 maps must be 4-byte aligned");
+  B2U_CHECK_ARG(T >= 1 && T <= 65535 && H >= 1 && W >= 1 && scratch_records >= T,
+                "regression_assess: T=%d H=%d W=%d (scratch for %lld records) out of range", T, H, W,
+                (long long)scratch_records);
+  B2U_CHECK_ARG(pred_pitch >= W && truth_pitch >= W &&
+                (T == 1 || (pred_stride >= pred_pitch * (H - 1) + W && truth_stride >= truth_pitch * (H - 1) + W)),
+                "regression_assess: pitches %lld / %lld or image strides %lld / %lld too small for %d x %d",
+                (long long)pred_pitch, (long long)truth_pitch, (long long)pred_stride, (long long)truth_stride, H, W);
+  // about eight blocks per SM over all images, as many as the scratch holds; rows per block a multiple of the 8 warps
+  long long gx = std::max(1ll, std::min(((long long)sm_count() * 8 + T - 1) / T, (long long)scratch_records / T));
+  long long rows = (H + gx - 1) / gx;
+  rows = (rows + 7) / 8 * 8;
+  gx = (H + rows - 1) / rows;
+  launch_k(regression_assess_kernel, dim3((unsigned)gx, T), dim3(256), 0, (cudaStream_t)stream, pred,
+           (long long)pred_pitch, (long long)pred_stride, truth, (long long)truth_pitch, (long long)truth_stride, T, H, W,
+           (int)rows, pred_nodata, truth_nodata, totals, tile_rec, (unsigned long long*)skipped, scratch, ticket);
   B2U_LAUNCH_CHECK();
   return B2U_OK;
 }

@@ -144,9 +144,10 @@ class TiledPredictor:
                        return_probs: bool = False, large_file: bool = False, grid: Optional[Tuple[int, int]] = None):
         """raster: uint8 / uint16 / int16 [C, Y, X] on the device (raw band values, scaled by the plan's input contract).
         Returns (mask uint8 [Y, x_end-x_begin], x_begin, x_end) for the
-        column strip this rank owns (the whole raster when world == 1).  With `grid=(gx, gy)` the rank owns cell
-        (rank % gx, rank // gx) of a gx x gy grid instead (`tiling.shard_windows_2d`; fewer duplicated tiles at 8 ranks) and
-        the return value is (mask [y_end-y_begin, x_end-x_begin], (x_begin, x_end, y_begin, y_end)).  `large_file`: the
+        column strip this rank owns (the whole raster when world == 1).  A regression net (`net.regression`) returns the
+        overlap mean of its output in place of the mask: fp32, -9999 where no tile was placed (predict.py:307-316).
+        With `grid=(gx, gy)` the rank owns cell (rank % gx, rank // gx) of a gx x gy grid instead
+        (`tiling.shard_windows_2d`; fewer duplicated tiles at 8 ranks) and the return value is (mask [y_end-y_begin, x_end-x_begin], (x_begin, x_end, y_begin, y_end)).  `large_file`: the
         reference's int8 merge (predict.py:217-219, 318-323).  `return_probs` also returns the accumulators.
         One batch = crop -> forward -> one accumulate per colour class, every launch reading the batch's tile origins /
         class lists from the `StitchPlan`'s device block, refilled (device-to-device) in front of it - no host round trip,
@@ -165,7 +166,7 @@ class TiledPredictor:
             idx, (xb, xe, yb, ye) = shard_windows_2d(windows, X, Y, rank, world, grid)
         self.tiles_run = len(idx)
         batches = [idx[b0:b0 + B] for b0 in range(0, len(idx), B)]
-        plan = StitchPlan(net, windows, batches, (yb, ye, xb, xe), 1 if large_file else 0)
+        plan = StitchPlan(net, windows, batches, (yb, ye, xb, xe), 2 if net.regression else 1 if large_file else 0)
         self._keep = plan           # its device blocks are read by launches still in flight when this returns
         s = ops.stream_ptr()
         for b in range(len(batches)):
@@ -174,7 +175,7 @@ class TiledPredictor:
                                           net.x_in.t.data_ptr(), net.x_in.ld, s), "b2u_crop_tiles")
             net.forward(s)
             plan.accumulate(s)
-        mask = plan.mask(s)
+        mask = plan.mean(-9999, s)[0] if net.regression else plan.mask(s)
         self.last_stitch_profile = {"batches": len(batches), "tiles_run": len(idx),
                                     "launches_per_batch": 1 + net.launches_fwd + plan.n_classes + 1}
         if grid is not None:

@@ -33,7 +33,7 @@ import numpy as np
 import torch
 
 from . import _lib, ops
-from .assessment import ConfusionCounter, write_report
+from .assessment import ConfusionCounter, RegressionCounter, write_regression_report, write_report
 from .engine import Trainer, one_cycle
 from .network import UNetB200, input_divisors
 from .predict_engine import StitchPlan, TiledPredictor, gather_mask_strips
@@ -399,13 +399,15 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
     (`all_classes` / `specific_class` write the averaged probabilities instead; `large_file` uses the int8 x31 /
     floor-division merge; `regression` the mean prediction with nodata -9999, predict.py:307-316).
     Under `torch.distributed` the tiles are sharded over the ranks: per-tile outputs round-robin, the merge as
-    owner-computes column strips of the mosaic gathered on rank 0 (no other collective).  Returns the output path(s)."""
+    owner-computes column strips of the mosaic gathered on rank 0 (no other collective).  Returns the output path(s).
+    `validation_vision`: every tile's prediction is compared on the device with its mask tile (`_mask_path`), and rank 0
+    writes `<AOI>_<year>_<model>_validation*` next to the outputs: the confusion report (`assessment.write_report`), or
+    for `regression` the error statistics against the float32 mask values, the mask tile's no-data skipped
+    (`assessment.write_regression_report`)."""
     learn = predict_model if isinstance(predict_model, Learner) else load_learner(predict_model)
     if bool(regression) != learn.regression:
         raise ValueError(f"regression={regression} but the model was trained with regression={learn.regression}")
-    if validation_vision and regression:
-        warnings.warn("validation_vision (confusion-matrix plots, predict.py:56-143) is outside the built path; skipped")
-    assess = bool(validation_vision) and not regression
+    assess = bool(validation_vision)
     path = Path(predict_path)
     model_name = "model" if isinstance(predict_model, Learner) else os.path.basename(str(predict_model)).split(".")[0]
     tiles = sorted(path.glob("*.tif")) or sorted(path.glob("*.npy"))
@@ -432,12 +434,12 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
             arr = np.stack([a for a, _ in loaded])
             if tuple(arr.shape[1:]) != (net.n_in, P, P):
                 raise ValueError(f"tiles must be [{net.n_in},{P},{P}], got {tuple(arr.shape[1:])}")
-            ys = [] if counted is None else [_load_labels(masks[t], net.n_out, P)
+            ys = [] if counted is None else [_load_labels(masks[t], net.n_out, P, regression)
                                              for t, k in zip(chunk, counted[b0:b0 + B]) if k]
             if stage is None or stage.dtype != torch.from_numpy(arr[:0]).dtype:
                 stage = torch.empty((B,) + arr.shape[1:], dtype=torch.from_numpy(arr[:0]).dtype).pin_memory()
             if counted is not None and ystage is None:
-                ystage = torch.empty((B, P, P), dtype=torch.uint8).pin_memory()
+                ystage = torch.empty((B, P, P), dtype=ydtype).pin_memory()
             torch.cuda.current_stream().synchronize()      # the previous batch's H2D copies have left the staging buffers
             stage[:len(chunk)] = torch.from_numpy(arr)
             if len(chunk) < B:
@@ -446,8 +448,9 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
                 ystage[:len(ys)] = torch.from_numpy(np.stack(ys))
             yield b0, chunk, [g for _, g in loaded], stage, ystage, len(ys)
 
+    ydtype = torch.float32 if regression else torch.uint8
     if assess:
-        y_dev = torch.empty((B, P, P), dtype=torch.uint8, device=dev)
+        y_dev = torch.empty((B, P, P), dtype=ydtype, device=dev)
 
     if merge:
         # ---- pass 1 over the headers: extent of the mosaic (predict.py:257-276)
@@ -480,9 +483,17 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
         mine, xb, xe = shard_windows_by_columns(wins, x_len, rank, world)
         own = column_owned(wins, mine, xb, xe)
         if assess:
-            n_own = max(sum(column_owned(wins, *shard_windows_by_columns(wins, x_len, r, world))) for r in range(world))
-            counter = ConfusionCounter(net.n_out, dev, n_own, rank, world)
-            amax_dev = torch.empty((B, P, P), dtype=torch.uint8, device=dev)
+            # the tiles each rank owns, in its batch order
+            owned = []
+            for r in range(world):
+                mine_r, xb_r, xe_r = shard_windows_by_columns(wins, x_len, r, world)
+                owned.append([tiles[i].name for i, o in zip(mine_r, column_owned(wins, mine_r, xb_r, xe_r)) if o])
+            n_own = max(len(o) for o in owned)
+            if regression:
+                counter = RegressionCounter(dev, n_own, rank, world)
+            else:
+                counter = ConfusionCounter(net.n_out, dev, n_own, rank, world)
+                amax_dev = torch.empty((B, P, P), dtype=torch.uint8, device=dev)
         plan = StitchPlan(net, wins, [mine[b0:b0 + B] for b0 in range(0, len(mine), B)], (0, y_len, xb, xe),
                           2 if regression else 1 if large_file else 0)
         s_ = ops.stream_ptr()
@@ -491,7 +502,15 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
             net.set_input(x.to(dev, non_blocking=True))
             net.forward()
             plan.accumulate(s_)
-            if ny:
+            if ny and regression:
+                # the per-tile raw prediction (what predict_tiles_raw returns) of each tile this rank owns
+                vals = net.logits_nchw()[:, 0]
+                y_dev[:ny].copy_(ys[:ny], non_blocking=True)
+                k = 0
+                for i0, i1 in _runs(own[b0:b0 + len(chunk)]):
+                    counter.count(vals[i0:i1], y_dev[k:k + i1 - i0], per_tile=True)
+                    k += i1 - i0
+            elif ny:
                 # the per-tile argmax (what predict_tiles returns) of the tiles this rank owns, packed in batch order
                 k, ld = 0, net.logits.shape[-1]
                 for i0, i1 in _runs(own[b0:b0 + len(chunk)]):
@@ -500,7 +519,9 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
                     k += i1 - i0
                 y_dev[:ny].copy_(ys[:ny], non_blocking=True)
                 counter.count(amax_dev[:ny], y_dev[:ny], per_tile=True)
-        if assess:
+        if assess and regression:
+            _write_regression_validation(counter, owned, world, rank, out_dir, AOI, year, model_name)
+        elif assess:
             _write_validation(counter, world, rank, out_dir, AOI, year, model_name, class_zero)
         nodata = None
         if regression:
@@ -533,12 +554,18 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
 
     outs = []
     sel = tiles[rank::world]
-    if assess:
+    if assess and regression:
+        counter = RegressionCounter(dev, -(-len(tiles) // world), rank, world)
+    elif assess:
         counter = ConfusionCounter(net.n_out, dev, -(-len(tiles) // world), rank, world)
     for b0, chunk, geos, x, ys, ny in batches(sel, [True] * len(sel) if assess else None):
         xd = x.to(dev, non_blocking=True)
         if regression:
-            vals = pred.predict_tiles_raw(xd).cpu().numpy()
+            vals = pred.predict_tiles_raw(xd)
+            if assess:                                          # the real tiles of a padded last batch
+                y_dev[:ny].copy_(ys[:ny], non_blocking=True)
+                counter.count(vals[:ny, 0], y_dev[:ny], per_tile=True)
+            vals = vals.cpu().numpy()
         else:
             probs, amax = pred.predict_tiles(xd)
             if assess:                                          # the real tiles of a padded last batch
@@ -557,7 +584,10 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
             if large_file and not regression and (all_classes or specific_class):   # predict.py:245-249 (sic: class 0 is falsy there)
                 arr = np.around(arr * ((128 / 4) - 1)).astype(np.int8)
             outs.append(_store(out_dir / t.name, arr, geos[i], None, class_zero))
-    if assess:
+    if assess and regression:
+        _write_regression_validation(counter, [[t.name for t in tiles[r::world]] for r in range(world)], world, rank,
+                                     out_dir, AOI, year, model_name)
+    elif assess:
         _write_validation(counter, world, rank, out_dir, AOI, year, model_name, class_zero)
     return outs
 
@@ -573,13 +603,24 @@ def _mask_path(tile: Path) -> Path:
     return m
 
 
-def _load_labels(path: Path, n_classes: int, P: int) -> np.ndarray:
-    """band 1 of a mask tile as uint8 class ids below `n_classes` (the labels training reads, `_label_values`)"""
-    y = read_geotiff(path)[0] if path.suffix.lower() in (".tif", ".tiff") else np.load(path)
+def _load_labels(path: Path, n_classes: int, P: int, regression: bool = False) -> np.ndarray:
+    """band 1 of a mask tile as uint8 class ids below `n_classes` (the labels training reads, `_label_values`); for the
+    regression variant the float32 targets, NaN (skipped by the assessment) where the tile declares its no-data value"""
+    nodata = None
+    if path.suffix.lower() in (".tif", ".tiff"):
+        y, geo = read_geotiff(path)
+        nodata = geo.nodata
+    else:
+        y = np.load(path)
     y = y[0] if y.ndim == 3 else y
     if y.shape != (P, P):
         raise ValueError(f"{path}: mask tile of shape {y.shape}, expected ({P}, {P})")
-    return _label_values(y, n_classes, False, path)
+    if not regression:
+        return _label_values(y, n_classes, False, path)
+    t = _label_values(y, n_classes, True, path)
+    if nodata is not None:
+        t[y == nodata] = np.nan
+    return t
 
 
 def _runs(flags: Sequence[bool]) -> List[Tuple[int, int]]:
@@ -604,6 +645,17 @@ def _write_validation(counter: ConfusionCounter, world: int, rank: int, out_dir:
         write_report(out_dir, name, cm, skipped, hist, class_zero)
 
 
+def _write_regression_validation(counter: RegressionCounter, names: Sequence[Sequence[str]], world: int, rank: int,
+                                 out_dir: Path, AOI, year, model_name: str) -> None:
+    """the moments of all ranks merged in rank order (`names[r]`: the tiles rank r counted, in its slot order); rank 0
+    writes `<AOI>_<year>_<model>_validation{.json,_tile_metrics.csv}` with the tile rows sorted by name"""
+    totals, skipped, recs = counter.read(all_reduce=world > 1)
+    if rank == 0:
+        rows = sorted(((n, recs[r][j]) for r in range(world) for j, n in enumerate(names[r])), key=lambda e: e[0])
+        name = "_".join([str(p_) for p_ in (AOI, year, model_name, "validation") if p_])
+        write_regression_report(out_dir, name, totals, skipped, [m for _, m in rows], [n for n, _ in rows])
+
+
 def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: float = 0.125, large_file: bool = False,
                     class_zero: bool = False, rank: int = 0, world: int = 1, max_strip_columns: Optional[int] = None,
                     mask_path=None):
@@ -620,11 +672,15 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
     the labels `prepare_raster` makes of the mask (class_zero shift, no-data of image or mask -> 0; a label >= the number
     of classes raises ValueError) over the columns the strip owns, and the accuracy report of the rank's columns goes next
     to the mask as `<out stem>_assessment{.json,_confusion.csv}` (`assessment.write_report`).  The written mask and the
-    return value do not change."""
+    return value do not change.
+    A regression model (`enable_regression`) writes what `save_predictions(regression=True, merge=True)` writes: the
+    overlap mean of its output as a Float32 GeoTIFF with nodata -9999 (`large_file` has no effect).  With `mask_path`
+    its error statistics against the mask values (the same window read, grid check and class_zero shift) go to
+    `<out stem>_assessment.json` (`assessment.write_regression_report`); pixels that are no-data in the image or the
+    mask are skipped and counted, not zeroed."""
     from .create_tiles import check_same_grid, mask_labels, mask_tile_values
     learn = predict_model if isinstance(predict_model, Learner) else load_learner(predict_model)
-    if learn.regression:
-        raise ValueError("predict_geotiff writes class masks; use save_predictions(regression=True, merge=True) over tiles")
+    regression = learn.regression
     net = learn._eval_net()
     bands, Y, X, dt, geo = geotiff_info(raster_path)
     if dt not in _NP_OK:
@@ -636,12 +692,12 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
     windows = compute_windows(Y, X, P, patch_overlap)
     _, xb, xe = shard_windows_by_columns(windows, X, rank, world)
     n_strips = 1 if not max_strip_columns else max(1, -(-(xe - xb) // int(max_strip_columns)))
-    mask = np.empty((Y, xe - xb), dtype=np.uint8)
+    mask = np.empty((Y, xe - xb), dtype=np.float32 if regression else np.uint8)
     counter = None
     if mask_path is not None:
         _, mY, mX, _, mgeo = geotiff_info(mask_path)
         check_same_grid(geo, mgeo, (Y, X), (mY, mX))
-        counter = ConfusionCounter(net.n_out, net.device)
+        counter = RegressionCounter(net.device, pred_nodata=-9999) if regression else ConfusionCounter(net.n_out, net.device)
     for k in range(n_strips):
         # strip k of this rank's columns: the balanced partition of [xb, xe), then the tile columns intersecting it
         sb, se = (xb + v for v in split_range(xe - xb, n_strips, k))
@@ -655,20 +711,25 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
         if counter is not None:
             # the truth of the same window, laid out like `m` so that both rows sit at the same 16-byte offset
             truth, _ = read_geotiff(mask_path, window=(xs0, 0, xs1 - xs0, Y))
-            truth, _ = mask_labels(strip, geo.nodata, truth, mgeo.nodata, class_zero)
-            truth = _label_values(mask_tile_values(truth[0]), net.n_out, False, mask_path)
+            truth, bad = mask_labels(strip, geo.nodata, truth, mgeo.nodata, class_zero)
+            truth = _label_values(mask_tile_values(truth[0]), net.n_out, regression, mask_path)
+            if regression:
+                truth[bad] = np.nan                 # 0 is a real value of a continuous target: skip, do not zero
             truth_d = torch.from_numpy(np.ascontiguousarray(truth)).pin_memory().to(net.device, non_blocking=True)
             counter.count(m[:, sb - xs0:se - xs0], truth_d[:, sb - xs0:se - xs0])
         mask[:, sb - xb:se - xb] = m[:, sb - xs0:se - xs0].cpu().numpy()
     out_path = Path(out_path) if out_path is not None else Path(raster_path).with_name(Path(raster_path).stem + "_prediction.tif")
     if world > 1:
         out_path = out_path.with_suffix(f".part{rank}.tif")
-    write_geotiff(out_path, mask, geo.window(xb, 0), nodata=None, class_zero=class_zero)
+    write_geotiff(out_path, mask, geo.window(xb, 0), nodata=-9999 if regression else None, class_zero=class_zero)
     if counter is not None:
-        cm, skipped, _ = counter.read()
-        write_report(Path(mask_path).parent, out_path.stem + "_assessment", cm, skipped, None, class_zero,
-                     extra={"raster": str(raster_path), "mask": str(mask_path), "prediction": str(out_path),
-                            "columns": [xb, xe]})
+        extra = {"raster": str(raster_path), "mask": str(mask_path), "prediction": str(out_path), "columns": [xb, xe]}
+        if regression:
+            totals, skipped, _ = counter.read()
+            write_regression_report(Path(mask_path).parent, out_path.stem + "_assessment", totals, skipped, extra=extra)
+        else:
+            cm, skipped, _ = counter.read()
+            write_report(Path(mask_path).parent, out_path.stem + "_assessment", cm, skipped, None, class_zero, extra=extra)
     return out_path
 
 
