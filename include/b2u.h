@@ -402,6 +402,14 @@ int b2u_stitch_finalize(const float* acc, const uint8_t* cnt, int32_t C, int64_t
  * averaged probabilities of the `all_classes` / `specific_class` merge, predict.py:326-337, nodata 0) */
 int b2u_stitch_finalize_mean(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, float nodata,
                              float* out, void* stream);
+/* The averaged class probabilities of the `all_classes` / `specific_class` merge (predict.py:226-254, 307-337) for
+ * classes [c0, c0 + nc) over columns [x0, x0 + w) of acc / cnt, written pixel-interleaved - the sample order of a
+ * striped GeoTIFF: out[y * pitch + (x - x0) * nc + k] for y < Y, pitch in elements (>= w * nc), 1 <= nc <= 32.
+ * mode 0 (sums of accumulate mode 0): fp32 acc / cnt, the same IEEE division as b2u_stitch_finalize_mean, 0 where
+ * cnt == 0.  mode 1 (sums of accumulate mode 1, `large_file`): int8, the reference's int8 arithmetic - the sum wraps
+ * modulo 256 and is floor-divided (toward -inf) by the count as int8 where that is > 0; 0 where cnt == 0. */
+int b2u_stitch_finalize_probs(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X, int32_t c0,
+                              int32_t nc, int64_t x0, int64_t w, int32_t mode, void* out, int64_t pitch, void* stream);
 /* per-tile softmax probabilities (fp32 NCHW, what learn.predict returns, predict.py:193-203) and argmax */
 int b2u_softmax_nchw(const float* logits, int32_t ld, int32_t C, int64_t tiles, int32_t H, int32_t W, float* probs,
                      uint8_t* argmax, void* stream);

@@ -172,6 +172,7 @@ def _declare(lib):
         "b2u_stitch_accumulate": [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, i32, i32, vp, u8p, i64, i64, i64, i64, vp],
         "b2u_stitch_finalize": [vp, u8p, i32, i64, i64, i32, u8p, vp],
         "b2u_stitch_finalize_mean": [vp, u8p, i32, i64, i64, f32, vp, vp],
+        "b2u_stitch_finalize_probs": [vp, u8p, i32, i64, i64, i32, i32, i64, i64, i32, vp, i64, vp],
         "b2u_softmax_nchw": [vp, i32, i32, i64, i32, i32, vp, u8p, vp],
         "b2u_confusion_counts": [u8p, i64, i64, u8p, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp],
         "b2u_regression_assess": [vp, i64, i64, vp, i64, i64, i32, i32, i32, f32, f32, vp, vp, vp, vp, i64, vp, vp],

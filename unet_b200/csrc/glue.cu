@@ -1183,15 +1183,99 @@ __global__ void stitch_finalize_kernel(const float* __restrict__ acc, const uint
   }
 }
 
-// averaged values of the merge: out[c][i] = acc[c][i] / cnt[i] where tiles were placed, else `nodata` (regression:
-// predict.py:307-316 with nodata -9999; averaged class probabilities of `all_classes` / `specific_class`: nodata 0)
-__global__ void stitch_finalize_mean_kernel(const float* __restrict__ acc, const uint8_t* __restrict__ cnt, int C,
-                                            long long YX, float nodata, float* __restrict__ out) {
+// one averaged value of the merge from a pixel's sum `a` and count `n`
+__device__ __forceinline__ float stitch_average(float a, int n, float nodata, float*) {
+  // the IEEE division of numpy's float32 `merged[counter > 0] /= counter` (predict.py:307-326): no fast-math here
+  return n > 0 ? a / (float)n : nodata;
+}
+__device__ __forceinline__ int8_t stitch_average(float a, int n, float, int8_t*) {
+  // the reference's int8 `large_file` arithmetic (predict.py:217-219, 318-323): the sums of x31 probabilities (exact
+  // integers in fp32) wrap modulo 256 like its int8 `+=`; its counter is int8 too, and `//=` floors where it is > 0.
+  // Counts of 128 or more are negative as int8 and leave the sum undivided, as the reference's masked `//=` does.
+  int s = n ? (int)a & 255 : 0;
+  s -= (s & 128) << 1;
+  const int d = n - ((n & 128) << 1);
+  if (d <= 0) return (int8_t)s;
+  int q = s / d;
+  if (q * d > s) --q;                           // C truncates toward zero, numpy floors
+  return (int8_t)q;
+}
+
+// Classes [c0, c0 + nc) of columns [x0, x0 + w) of the stitch accumulators (acc fp32 [C][Y][X], cnt uint8 [Y][X]),
+// averaged and written pixel-interleaved: out[y * pitch + (x - x0) * nc + k].  A block takes 256 * PPT pixels of one
+// row: every thread reads the count and the nc planes of its pixels (coalesced along x, PPT x UNROLL loads in flight),
+// the values are transposed through shared memory (one padding word per 32, conflict-free for any nc) and the block
+// stores the chunk's npx * nc consecutive outputs with consecutive threads - 16 bytes each where `vec` says the rows
+// are 16-byte aligned - so every warp fills whole sectors whatever nc is.
+template <typename T, int PPT, int UNROLL>
+__global__ void __launch_bounds__(256) stitch_finalize_probs_kernel(const float* __restrict__ acc,
+                                                                    const uint8_t* __restrict__ cnt, long long Y,
+                                                                    long long X, int c0, int nc, long long x0,
+                                                                    long long w, float nodata, T* __restrict__ out,
+                                                                    long long pitch, int vec) {
   pdl_enter();
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < YX; i += (long long)gridDim.x * blockDim.x) {
-    const int n = cnt[i];
-    for (int c = 0; c < C; ++c) out[(long long)c * YX + i] = n > 0 ? acc[(long long)c * YX + i] / (float)n : nodata;
+  extern __shared__ __align__(16) unsigned char stitch_smem[];
+  T* s = reinterpret_cast<T*>(stitch_smem);
+  constexpr int kPix = 256 * PPT, V = 16 / sizeof(T);
+  const long long YX = Y * X, per_row = (w + kPix - 1) / kPix, chunks = Y * per_row;
+  const float* a0 = acc + (long long)c0 * YX;
+  for (long long ch = blockIdx.x; ch < chunks; ch += gridDim.x) {
+    const long long y = ch / per_row, xs = (ch - y * per_row) * kPix;
+    const int npx = (int)min((long long)kPix, w - xs);
+    const long long base = y * X + x0 + xs;
+    int n[PPT];
+#pragma unroll
+    for (int p = 0; p < PPT; ++p) {
+      const int px = threadIdx.x + 256 * p;
+      n[p] = px < npx ? cnt[base + px] : 0;
+    }
+#pragma unroll UNROLL
+    for (int k = 0; k < nc; ++k) {
+      float v[PPT];
+#pragma unroll
+      for (int p = 0; p < PPT; ++p) {
+        const int px = threadIdx.x + 256 * p;
+        v[p] = px < npx ? a0[(long long)k * YX + base + px] : 0.f;
+      }
+#pragma unroll
+      for (int p = 0; p < PPT; ++p) {
+        const int j = (threadIdx.x + 256 * p) * nc + k;
+        if (threadIdx.x + 256 * p < npx) s[j + (j >> 5)] = stitch_average(v[p], n[p], nodata, (T*)nullptr);
+      }
+    }
+    __syncthreads();
+    T* o = out + y * pitch + xs * nc;
+    const int total = npx * nc, j0 = vec ? total / V * V : 0;
+    for (int q = threadIdx.x * V; q < j0; q += 256 * V) {
+      union { uint4 u; T e[V]; } r;
+#pragma unroll
+      for (int e = 0; e < V; ++e) r.e[e] = s[q + e + ((q + e) >> 5)];
+      *reinterpret_cast<uint4*>(o + q) = r.u;
+    }
+    for (int j = j0 + threadIdx.x; j < total; j += 256) o[j] = s[j + (j >> 5)];
+    __syncthreads();
   }
+}
+
+// enough pixels per thread that PPT x UNROLL loads are in flight for any nc; the staged chunk stays at 33 KB
+template <typename T>
+static void launch_stitch_finalize_probs(const float* acc, const uint8_t* cnt, long long Y, long long X, int c0, int nc,
+                                         long long x0, long long w, float nodata, T* out, long long pitch,
+                                         cudaStream_t st) {
+  const int ppt = nc <= 4 ? 8 : nc <= 8 ? 4 : 1;
+  const long long chunks = Y * ((w + 256 * ppt - 1) / (256 * ppt));
+  const size_t smem = (size_t)256 * ppt * nc / 32 * 33 * sizeof(T);
+  const dim3 grid(grid_for(chunks * 256, 256));
+  const int vec = (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (pitch * (long long)sizeof(T)) % 16 == 0;
+  if (ppt == 8)
+    launch_k(stitch_finalize_probs_kernel<T, 8, 1>, grid, dim3(256), smem, st, acc, cnt, Y, X, c0, nc, x0, w, nodata,
+             out, pitch, vec);
+  else if (ppt == 4)
+    launch_k(stitch_finalize_probs_kernel<T, 4, 2>, grid, dim3(256), smem, st, acc, cnt, Y, X, c0, nc, x0, w, nodata,
+             out, pitch, vec);
+  else
+    launch_k(stitch_finalize_probs_kernel<T, 1, 8>, grid, dim3(256), smem, st, acc, cnt, Y, X, c0, nc, x0, w, nodata,
+             out, pitch, vec);
 }
 
 // per-tile probabilities (fp32 NCHW) and argmax — what learn.predict hands back per tile
@@ -1943,8 +2027,31 @@ extern "C" int b2u_stitch_accumulate(const float* logits, int32_t ld, int32_t C,
 extern "C" int b2u_stitch_finalize_mean(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X,
                                         float nodata, float* out, void* stream) {
   B2U_CHECK_ARG(acc && cnt && out && C >= 1, "stitch_finalize_mean: bad argument");
-  launch_k(stitch_finalize_mean_kernel, dim3(grid_for(Y * X, 256)), dim3(256), 0, (cudaStream_t)stream, acc, cnt, C, (long long)(Y * X),
-           nodata, out);
+  // planar [C][Y][X]: class c is the one-class interleaved layout of plane c
+  for (int c = 0; c < C; ++c)
+    launch_stitch_finalize_probs<float>(acc, cnt, Y, X, c, 1, 0, X, nodata, out + (long long)c * Y * X, X,
+                                        (cudaStream_t)stream);
+  B2U_LAUNCH_CHECK();
+  return B2U_OK;
+}
+
+extern "C" int b2u_stitch_finalize_probs(const float* acc, const uint8_t* cnt, int32_t C, int64_t Y, int64_t X,
+                                         int32_t c0, int32_t nc, int64_t x0, int64_t w, int32_t mode, void* out,
+                                         int64_t pitch, void* stream) {
+  B2U_CHECK_ARG(acc && cnt && out, "stitch_finalize_probs: null argument");
+  B2U_CHECK_ARG(C >= 1 && Y >= 1 && X >= 1 && (mode == 0 || mode == 1),
+                "stitch_finalize_probs: C=%d Y=%lld X=%lld mode=%d out of range", C, (long long)Y, (long long)X, mode);
+  B2U_CHECK_ARG(c0 >= 0 && nc >= 1 && nc <= 32 && c0 + nc <= C,
+                "stitch_finalize_probs: classes [%d, %d + %d) outside [0, %d) or more than 32", c0, c0, nc, C);
+  B2U_CHECK_ARG(x0 >= 0 && w >= 1 && x0 + w <= X, "stitch_finalize_probs: columns [%lld, %lld + %lld) outside [0, %lld)",
+                (long long)x0, (long long)x0, (long long)w, (long long)X);
+  B2U_CHECK_ARG(pitch >= w * nc, "stitch_finalize_probs: pitch %lld < %lld columns x %d classes", (long long)pitch,
+                (long long)w, nc);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (mode == 0)
+    launch_stitch_finalize_probs<float>(acc, cnt, Y, X, c0, nc, x0, w, 0.f, (float*)out, pitch, st);
+  else
+    launch_stitch_finalize_probs<int8_t>(acc, cnt, Y, X, c0, nc, x0, w, 0.f, (int8_t*)out, pitch, st);
   B2U_LAUNCH_CHECK();
   return B2U_OK;
 }

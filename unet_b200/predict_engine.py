@@ -62,6 +62,20 @@ def gather_mask_cells(cell: torch.Tensor, height: int, width: int, grid: Tuple[i
     return full
 
 
+def finalize_probs(acc: torch.Tensor, cnt: torch.Tensor, c0: int, nc: int, x0: int, w: int, large_file: bool,
+                   stream: int) -> torch.Tensor:
+    """the averaged probabilities of classes [c0, c0 + nc) over columns [x0, x0 + w) of stitch accumulators (`acc` fp32
+    [C, SY, SX] and `cnt` uint8 [SY, SX] of a `StitchPlan` in mode 0, or mode 1 with `large_file`), as the device tensor
+    [SY, w, nc] the bands of a striped GeoTIFF are stored in: float32 acc / cnt, or with `large_file` the reference's
+    int8 merge (sums wrapped to int8, floor-divided by the count); 0 where no tile was placed"""
+    C, SY, SX = acc.shape
+    out = torch.empty((SY, w, nc), dtype=torch.int8 if large_file else torch.float32, device=acc.device)
+    _lib.check(_lib.load().b2u_stitch_finalize_probs(acc.data_ptr(), cnt.data_ptr(), C, SY, SX, c0, nc, x0, w,
+                                                     int(large_file), out.data_ptr(), w * nc, stream),
+               "b2u_stitch_finalize_probs")
+    return out
+
+
 class StitchPlan:
     """The overlap stitching of one job's predicted tiles into the output rectangle `region` = (yb, ye, xb, xe) of the
     raster: per batch of tiles the network has just run, one `b2u_stitch_accumulate` launch per colour class adds the

@@ -36,7 +36,7 @@ from . import _lib, ops
 from .assessment import ConfusionCounter, RegressionCounter, write_regression_report, write_report
 from .engine import Trainer, one_cycle
 from .network import UNetB200, input_divisors
-from .predict_engine import StitchPlan, TiledPredictor, gather_mask_strips
+from .predict_engine import StitchPlan, TiledPredictor, finalize_probs, gather_mask_strips
 from .losses import LossSpec, dice_blocks_per_sample, launch_loss, parse_loss_func, warn_dice_weights
 from .geotiff import GeoInfo, geotiff_info, open_mask, open_tile, read_geotiff, write_geotiff
 from .tiling import column_owned, compute_windows, placement_from_geotransform, shard_windows_by_columns, split_range
@@ -378,11 +378,12 @@ def _store(path: Path, arr: np.ndarray, geo: Optional[GeoInfo], nodata, class_ze
 
 
 def _gather_strips(strip: torch.Tensor, width: int, rank: int, world: int) -> Optional[torch.Tensor]:
-    """[Y, w] or [C, Y, w] column strips of every rank -> the full-width array on rank 0 (predict_engine.gather_mask_strips)."""
+    """[Y, w] or [Y, w, bands] column strips of every rank -> the full-width array on rank 0
+    (predict_engine.gather_mask_strips)."""
     if strip.dim() == 2:
         return gather_mask_strips(strip, width, rank, world)
-    parts = [gather_mask_strips(strip[c].contiguous(), width, rank, world) for c in range(strip.shape[0])]
-    return None if parts[0] is None else torch.stack(parts)
+    parts = [gather_mask_strips(strip[:, :, k].contiguous(), width, rank, world) for k in range(strip.shape[2])]
+    return None if parts[0] is None else torch.stack(parts, 2)
 
 
 def save_predictions(predict_model, predict_path, regression: bool = False, merge: bool = False,
@@ -527,23 +528,18 @@ def save_predictions(predict_model, predict_path, regression: bool = False, merg
         if regression:
             strip, nodata = plan.mean(-9999, s_)[0], -9999                                   # predict.py:313-316
         elif all_classes or specific_class is not None:
-            if large_file:
-                # int8 sums floor-divided by the count (predict.py:318-323): the reference's own host arithmetic
-                m = plan.acc.cpu().numpy().astype(np.int8)
-                c8 = plan.cnt.cpu().numpy().astype(np.int8)
-                mk = np.broadcast_to(c8 > 0, m.shape)
-                m[mk] //= np.broadcast_to(c8, m.shape)[mk]
-                strip = torch.from_numpy(m).to(dev)
-            else:
-                strip = plan.mean(0, s_)
-            if not all_classes:
-                strip = strip[specific_class]
+            # [y_len, xe - xb, bands], float32 or with `large_file` the int8 merge (predict.py:318-326)
+            c0, nc = (0, net.n_out) if all_classes else (range(net.n_out)[specific_class], 1)     # python indexing
+            strip = finalize_probs(plan.acc, plan.cnt, c0, nc, 0, plan.SX, large_file, s_)
         else:
             strip = plan.mask(s_)
-        full = _gather_strips(strip.contiguous(), x_len, rank, world) if world > 1 else strip
+        full = _gather_strips(strip, x_len, rank, world) if world > 1 else strip
         if rank != 0:
             return None
         out = full.cpu().numpy()
+        if out.ndim == 3:
+            # [bands, Y, X] (one band: [Y, X]) as a view: write_geotiff stores it without a transposing copy
+            out = np.moveaxis(out, 2, 0) if all_classes else out[:, :, 0]
         name = "_".join([p_ for p_ in (AOI, year, model_name, "prediction") if p_])
         geo = None
         if geos[0] is not None:
@@ -658,7 +654,7 @@ def _write_regression_validation(counter: RegressionCounter, names: Sequence[Seq
 
 def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: float = 0.125, large_file: bool = False,
                     class_zero: bool = False, rank: int = 0, world: int = 1, max_strip_columns: Optional[int] = None,
-                    mask_path=None):
+                    mask_path=None, all_classes: bool = False, specific_class: Optional[int] = None):
     """Tile-free variant of the predict path: what `split_raster` (create_tiles_unet.py:252-431) + `save_predictions(merge=
     True)` produce together - the stitched argmax mask of a whole multi-band GeoTIFF (uint8 / uint16 / int16 bands) -
     without writing tiles to disk: the raster is windowed on the device with `compute_windows` offsets, predicted and
@@ -677,11 +673,23 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
     overlap mean of its output as a Float32 GeoTIFF with nodata -9999 (`large_file` has no effect).  With `mask_path`
     its error statistics against the mask values (the same window read, grid check and class_zero shift) go to
     `<out stem>_assessment.json` (`assessment.write_regression_report`); pixels that are no-data in the image or the
-    mask are skipped and counted, not zeroed."""
+    mask are skipped and counted, not zeroed.
+    `all_classes` / `specific_class=k`: the averaged class probabilities instead of the mask, as `save_predictions(merge=
+    True)` writes them over the tiles of the same raster with the same flags - all `n_out` bands, or band k alone
+    (`all_classes` wins if both are given); Float32, or with `large_file` the reference's int8 x31 merge; no nodata tag;
+    `class_zero` applied by `write_geotiff` as for the mask.  Each strip's accumulators are finalized on the device
+    straight into the file's pixel-interleaved sample order.  With `mask_path` the assessment still counts the stitched
+    argmax of the same prediction pass.  The output is held in host memory until it is written: Y * X * bands * 4 bytes
+    for Float32 (1 byte per sample for int8), plus the strips `write_geotiff` builds while writing.  A `specific_class`
+    outside [0, n_out) raises ValueError before anything is predicted.  A regression model ignores both flags, as
+    `save_predictions` does."""
     from .create_tiles import check_same_grid, mask_labels, mask_tile_values
     learn = predict_model if isinstance(predict_model, Learner) else load_learner(predict_model)
     regression = learn.regression
     net = learn._eval_net()
+    probs = not regression and (all_classes or specific_class is not None)
+    if probs and not all_classes and not 0 <= specific_class < net.n_out:
+        raise ValueError(f"specific_class={specific_class} outside the model's {net.n_out} classes")
     bands, Y, X, dt, geo = geotiff_info(raster_path)
     if dt not in _NP_OK:
         raise ValueError(f"{raster_path}: {dt} rasters are not supported (uint8, uint16 or int16 band values)")
@@ -692,7 +700,11 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
     windows = compute_windows(Y, X, P, patch_overlap)
     _, xb, xe = shard_windows_by_columns(windows, X, rank, world)
     n_strips = 1 if not max_strip_columns else max(1, -(-(xe - xb) // int(max_strip_columns)))
-    mask = np.empty((Y, xe - xb), dtype=np.float32 if regression else np.uint8)
+    if probs:
+        c0, nc = (0, net.n_out) if all_classes else (specific_class, 1)
+        mask = np.empty((Y, xe - xb, nc), dtype=np.int8 if large_file else np.float32)
+    else:
+        mask = np.empty((Y, xe - xb), dtype=np.float32 if regression else np.uint8)
     counter = None
     if mask_path is not None:
         _, mY, mX, _, mgeo = geotiff_info(mask_path)
@@ -707,7 +719,7 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
         strip, _ = read_geotiff(raster_path, window=(xs0, 0, xs1 - xs0, Y))
         dev_s = torch.from_numpy(np.ascontiguousarray(strip)).pin_memory().to(net.device, non_blocking=True)
         # the strip holds exactly the tile columns of [sb, se): a one-rank prediction of it reproduces those tiles
-        m, _, _ = pred.predict_raster(dev_s, patch_overlap, 0, 1, large_file=large_file)
+        m, _, _, acc, cnt = pred.predict_raster(dev_s, patch_overlap, 0, 1, return_probs=True, large_file=large_file)
         if counter is not None:
             # the truth of the same window, laid out like `m` so that both rows sit at the same 16-byte offset
             truth, _ = read_geotiff(mask_path, window=(xs0, 0, xs1 - xs0, Y))
@@ -717,11 +729,17 @@ def predict_geotiff(predict_model, raster_path, out_path=None, patch_overlap: fl
                 truth[bad] = np.nan                 # 0 is a real value of a continuous target: skip, do not zero
             truth_d = torch.from_numpy(np.ascontiguousarray(truth)).pin_memory().to(net.device, non_blocking=True)
             counter.count(m[:, sb - xs0:se - xs0], truth_d[:, sb - xs0:se - xs0])
-        mask[:, sb - xb:se - xb] = m[:, sb - xs0:se - xs0].cpu().numpy()
+        if probs:
+            mask[:, sb - xb:se - xb] = finalize_probs(acc, cnt, c0, nc, sb - xs0, se - sb, large_file,
+                                                      ops.stream_ptr()).cpu().numpy()
+        else:
+            mask[:, sb - xb:se - xb] = m[:, sb - xs0:se - xs0].cpu().numpy()
     out_path = Path(out_path) if out_path is not None else Path(raster_path).with_name(Path(raster_path).stem + "_prediction.tif")
     if world > 1:
         out_path = out_path.with_suffix(f".part{rank}.tif")
-    write_geotiff(out_path, mask, geo.window(xb, 0), nodata=-9999 if regression else None, class_zero=class_zero)
+    # [Y, X, bands] as the [bands, Y, X] view whose transpose write_geotiff stores without a copy
+    write_geotiff(out_path, np.moveaxis(mask, 2, 0) if probs else mask, geo.window(xb, 0),
+                  nodata=-9999 if regression else None, class_zero=class_zero)
     if counter is not None:
         extra = {"raster": str(raster_path), "mask": str(mask_path), "prediction": str(out_path), "columns": [xb, xe]}
         if regression:
